@@ -4,6 +4,7 @@ its epilogue) + one GAE scan, at 262 144 envs per GPU (BASELINE configs[3] shard
 
     python bench.py --gpus N --steps K --warmup W                    # this repo's CUDA path (one process per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference torch path on the host CPU, same config
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR # also write the last timed rollout's outputs (.npy) to DIR
 
 Legs of the B200 arm (ONE JSON line, rank 0):
   value / roofline   the rollout with everything resident in HBM, replayed as one CUDA graph; the fused kernel's duration is read
@@ -29,6 +30,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -38,6 +40,27 @@ K0_BYTES = 144                         # SURVEY 8(d): actions 72 R + targets 72 
 POST_BYTES = 536 + 9                   # fused post-physics (prev_lin_vel buffer mode) + epilogue: value 4 R, shaped reward 4 W, done 1 W
 GAE_BYTES_PER_SAMPLE = 17
 POLICY_PARAMS = 124237                 # 54-400-200-100 ELU MLP + mu(18) + value(1) + sigma(18), cfg/train/bez_kickPPO.yaml:10-32
+DUMP_BYTES = 32 << 20                  # --dump-outputs writes at most this much (plus the .npy headers)
+
+
+def sample_envs(n, floats_per_env, seed=0):
+    """Sorted ids of a fixed, seeded sample of the n envs, as many as fit DUMP_BYTES at `floats_per_env` float32 values each."""
+    k = min(n, DUMP_BYTES // (4 * floats_per_env))
+    if k == n:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:k].sort().values
+
+
+def write_outputs(out_dir, arrays):
+    """name -> tensor as out_dir/<name>.npy: float64 stays float64, everything else becomes float32."""
+    import numpy as np
+    arrays = {k: (t.double() if t.dtype == torch.float64 else t.float()).cpu().numpy() for k, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"{total} bytes of outputs exceed the {DUMP_BYTES}-byte dump limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def parse():
@@ -58,7 +81,14 @@ def parse():
     p.add_argument("--no-learner", action="store_true")
     p.add_argument("--fusion", default="fused", choices=["fused", "split"])
     p.add_argument("--no-graph", action="store_true", help="time eager launches instead of a CUDA-graph replay of the step")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed rollout computed (rank 0, a fixed seeded sample of its envs) as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 def workload_config(args):
@@ -288,6 +318,18 @@ def rollout_leg(args, world, rank, dev):
     ms = start.elapsed_time(end)
     sampler.stop_flag = True
     sampler.join()
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        # the last timed rollout's results, taken before the passes below step the envs again: the PD targets of K0, what the
+        # post-physics step hands back, the dof rows its masked reset wrote, the epilogue's rollout storage, the GAE scan's output
+        idx = sample_envs(n, 18 + 54 + 4 + 36 + 2 * T + (2 * T + 1 if fused else 0))
+        per_env = {"pd_targets": env.targets, "obs": env._observations_out(), "rew": env.rew_buf, "reset": env.reset_buf,
+                   "time_outs": env.timeout_buf, "progress": env.progress_buf, "dof_state": env.dof_state.view(n, 36)}
+        per_step = {"advantages": advs.view(T, n), "returns": rets.view(T, n)}
+        if fused:
+            per_step.update(shaped_rewards=rewards.view(T, n), dones=dones)
+        outputs = {k: t[idx.to(t.device)].cpu() for k, t in per_env.items()}
+        outputs.update({k: t[:, idx.to(t.device)].cpu() for k, t in per_step.items()})
     post_graph_ms = post_eager_ms = eager_step_ms = in_region_ms = None
     if graph is not None and in_graph_events:
         try:
@@ -356,7 +398,7 @@ def rollout_leg(args, world, rank, dev):
            "ms_per_step_eager_with_events": eager_step_ms, "reset_rate_per_step": reset_rate,
            "parallelism": f"env-sharded x{world}, no data-path collective (the exchanges are in the learner leg)"}
     out = dict(value=value, ms_per_step=ms / args.steps, warmup=W, roofline=roofline, run=run, clocks=sampler.summary(),
-               gpu_launches=launches_per_step * args.steps)
+               gpu_launches=launches_per_step * args.steps, outputs=outputs)
     del env, sim, graph
     torch.cuda.empty_cache()
     return out
@@ -624,6 +666,8 @@ def run_b200(args):
                "data": "synthetic", "config": workload_config(args), "run": roll["run"], "clocks": roll["clocks"],
                "gpu_launches": roll["gpu_launches"], "roofline": roll["roofline"], "e2e": e2e, "learner": learner,
                "cpu_baseline": cpu_baseline, "gpu_torch_baseline": gpu_torch}
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, roll["outputs"])
         print(json.dumps(out))
     if world > 1:
         dist.barrier()

@@ -410,6 +410,33 @@ def test_bench_arms_share_one_workload_config(monkeypatch):
     assert bench.METRIC == "task+GAE env-steps/s" and bench.UNIT == "env-steps/s"
 
 
+def test_bench_dump_outputs_is_a_fixed_sample_within_the_size_limit(monkeypatch, tmp_path):
+    """``bench.py --dump-outputs DIR``: the env sample is the same on every run and fits the size limit; the files are float32
+    (float64 stays float64); an oversized dump is refused before anything is written; ``--steps`` below 1 is refused."""
+    import importlib
+    import sys
+    import numpy as np
+    bench = importlib.import_module("bench")
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "7", "--dump-outputs", str(tmp_path / "d")])
+    a = bench.parse()
+    assert a.steps == 7 and a.dump_outputs == str(tmp_path / "d")
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", *bad])
+        with pytest.raises(SystemExit):
+            bench.parse()
+    idx = bench.sample_envs(262144, 241)
+    assert torch.equal(idx, bench.sample_envs(262144, 241)) and bool((idx[1:] > idx[:-1]).all())
+    assert 0 < 4 * 241 * len(idx) <= bench.DUMP_BYTES and int(idx[-1]) < 262144
+    assert torch.equal(bench.sample_envs(100, 241), torch.arange(100))
+    bench.write_outputs(str(tmp_path / "d"), {"obs": torch.ones(3, 2), "reset": torch.ones(3, dtype=torch.long),
+                                              "stats": torch.ones(2, dtype=torch.float64)})
+    got = {p.stem: np.load(p) for p in (tmp_path / "d").iterdir()}
+    assert {k: v.dtype for k, v in got.items()} == {"obs": np.float32, "reset": np.float32, "stats": np.float64}
+    with pytest.raises(ValueError, match="dump limit"):
+        bench.write_outputs(str(tmp_path / "big"), {"x": torch.empty(bench.DUMP_BYTES // 4 + 1)})
+    assert not (tmp_path / "big").exists()
+
+
 def test_host_pack_pool_serves_several_issuing_threads():
     """The pool is process-wide: jobs issued and awaited from several Python threads at once (two envs stepping in two threads)
     all complete with the right bytes."""
