@@ -14,6 +14,7 @@ NUM_DOF = 18
 F_CLEATS = 1
 F_WRITE_CONTACT_FILTER = 2
 F_RESET_ROOT_STATES = 4
+F_OBS_STREAMED = 8
 
 PART_BOOKKEEP = 1
 PART_OBS = 2
@@ -105,6 +106,7 @@ SIGNATURES = {
     "bezk_reset_idx_task": (C.c_int, [C.c_int, _P, _I64, _P, _P, _U64, _U64, _P, _P, _P, _P, _P, _P, C.POINTER(BezkTaskCfg), _I64, _I64,
                                       _P]),
     "bezk_goal_uniforms": (C.c_int, [_U64, _U64, _P, _P]),
+    "bezk_l2_release": (C.c_int, [_P, _U64, _P]),
     "bezk_rms_moments_slabs": (C.c_int, [_P, _I64, _I64, _P, _P, _P, _I64, C.c_int32, _P]),
     "bezk_rms_normalize_slabs_batched": (C.c_int, [_P, _I64, _I64, _I64, _P, _P, _I64, C.c_float, _P, _I64, C.c_int32, C.c_int32, _P]),
     "bezk_rms_normalize_slabs": (C.c_int, [_P, _I64, _I64, _P, _P, C.c_float, C.c_int, _P, _I64, C.c_int32, _P]),

@@ -83,6 +83,7 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
         if (cfg->flags & BEZK_F_RESET_ROOT_STATES) REQUIRE(a.initial_root, "initial_root_states NULL");
     }
     bezk::fill_alignment(a, *cfg);
+    bezk::set_l2_policy(task, cfg->flags, a);
     if (bezk::persist_eligible(task, parts, a, *cfg))          // the persistent pipelined kernel (bezk_task_persist.cu)
         return cuda_rc(bezk::launch_task_persist(a, *cfg, (cudaStream_t)stream), where);
     return cuda_rc(bezk::launch_task(task, parts, a, *cfg, (cudaStream_t)stream), where);
@@ -335,6 +336,12 @@ int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_bod
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream) {
     REQUIRE(out2, "out2 NULL");
     return cuda_rc(bezk::launch_goal_uniforms(seed, step, out2, (cudaStream_t)stream), "bezk_goal_uniforms");
+}
+
+int bezk_l2_release(const void* ptr, uint64_t bytes, void* stream) {
+    if (bytes == 0) return 0;
+    REQUIRE(ptr, "ptr NULL");
+    return cuda_rc(bezk::launch_l2_release(ptr, bytes, (cudaStream_t)stream), "bezk_l2_release");
 }
 
 int bezk_philox_uniforms(uint64_t seed, uint64_t step, float* out, int64_t n, void* stream) {

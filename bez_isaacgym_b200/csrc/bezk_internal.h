@@ -48,7 +48,14 @@ struct TaskArgs {
     int rb_win;       // slice only 4 B aligned, but the 16-byte aligned window around it is readable: 3-4 vector loads
     int cf_vec2;      // both foot force rows of every env are 8 B aligned
     int smart_granule;  // per-lane 64 B / 128 B fill choice for the sparse gathers (env BEZK_SMART_GRANULE=0 disables)
+    // set_l2_policy: 1 = the step accesses the carried state (obs rows, reset / progress / timeout, rew, prev_lin_vel, goal,
+    // ball_init / goal_angle) with evict_last and the dense tiles and sparse gathers with evict_first (task_tile_l2_kernel)
+    int l2_resident;
 };
+// fills l2_resident (bezk_task.cu): after fill_alignment, before the launch
+void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a);
+// demote [ptr, ptr + bytes) to the normal L2 eviction priority (the 128-byte lines entirely inside the range)
+cudaError_t launch_l2_release(const void* ptr, uint64_t bytes, cudaStream_t st);
 struct PpoArgs {
     const float *actions, *mu, *logstd, *old_mu, *old_sigma, *values, *old_values, *returns, *old_neglogp, *advantages;
     float *grad_mu, *grad_values, *neglogp_out;

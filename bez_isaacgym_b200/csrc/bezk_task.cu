@@ -22,6 +22,7 @@
 #include "bezk_task_math.cuh"
 #include <math.h>
 #include <stdlib.h>
+#include <atomic>
 
 namespace bezk {
 
@@ -106,6 +107,10 @@ __device__ __forceinline__ Philox4 philox_goal(uint64_t seed, uint64_t step) {
                          (uint32_t)(seed >> 32));
 }
 
+// L2H: the hinted variant (task_tile_l2_kernel) -- the call with the cache policy; otherwise the plain call, so that the unhinted
+// kernel is the same code as without the hints (the policy descriptors cost ~9 % at 65 536 envs, where nothing is hinted)
+#define L2HINT(f, pol, ...) (L2H ? f(__VA_ARGS__, pol) : f(__VA_ARGS__))
+
 template <bool CLEATS>
 struct Gathered {
     // raw load results: NOTHING depends on them until consume(), so issuing gather_env() never stalls the warp
@@ -118,25 +123,9 @@ struct Gathered {
     long long reset_prev, progress;
 };
 
-__device__ __forceinline__ long long ld_i64(const int64_t* p) {
-    long long v;
-    asm volatile("ld.global.s64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ float2 ld_nc_v2(const void* p) {
-    float2 v;
-    asm volatile("ld.global.nc.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
-    return v;
-}
-__device__ __forceinline__ float ld_f32(const float* p) {
-    float v;
-    asm volatile("ld.global.f32 %0, [%1];" : "=f"(v) : "l"(p) : "memory");
-    return v;
-}
-
 // rb: this env's IMU-link slice (10 floats); cf_l / cf_r: its foot (first cleat) force rows.  The caller forms them as a
 // warp-uniform 64-bit base plus a 32-bit lane offset.
-template <bool OBS, bool BOOKREW, bool CLEATS, int TASK>
+template <bool OBS, bool BOOKREW, bool CLEATS, int TASK, bool L2H>
 __device__ __forceinline__ void gather_env(const TaskArgs& a, const BezkTaskCfg& cfg, int64_t e, bool valid, const float* rb,
                                            float* cf_l, float* cf_r, Gathered<CLEATS>& g) {
     constexpr int NFORCE = CLEATS ? 12 : 3;
@@ -152,6 +141,7 @@ __device__ __forceinline__ void gather_env(const TaskArgs& a, const BezkTaskCfg&
 #pragma unroll
     for (int k = 0; k < 6; ++k) g.win[k] = 0.0f;
     if (valid) {
+        const uint64_t ps = L2H ? policy_evict_first() : 0;     // the simulator's rows: read once per step
         if (a.rb_vec2) {
             // 40 bytes at an 8-byte aligned address: one 8 B + two 16 B loads, order chosen per lane by bit 3
             const char* p = reinterpret_cast<const char*>(rb);
@@ -163,9 +153,11 @@ __device__ __forceinline__ void gather_env(const TaskArgs& a, const BezkTaskCfg&
                                   (a.smart_granule && ((s128 & 63u) + 40u > 64u) && (s128 + 40u <= 128u));
             float2 a2; float4 b4, c4;
             if (one_line) {
-                a2 = ldg128B_nc_v2(p + (hi ? 0 : 32)); b4 = ldg128B_nc_v4(p + (hi ? 8 : 0)); c4 = ldg128B_nc_v4(p + (hi ? 24 : 16));
+                a2 = L2HINT(ldg128B_nc_v2, ps, p + (hi ? 0 : 32)); b4 = L2HINT(ldg128B_nc_v4, ps, p + (hi ? 8 : 0));
+                c4 = L2HINT(ldg128B_nc_v4, ps, p + (hi ? 24 : 16));
             } else {
-                a2 = ldg64B_nc_v2(p + (hi ? 0 : 32)); b4 = ldg64B_nc_v4(p + (hi ? 8 : 0)); c4 = ldg64B_nc_v4(p + (hi ? 24 : 16));
+                a2 = L2HINT(ldg64B_nc_v2, ps, p + (hi ? 0 : 32)); b4 = L2HINT(ldg64B_nc_v4, ps, p + (hi ? 8 : 0));
+                c4 = L2HINT(ldg64B_nc_v4, ps, p + (hi ? 24 : 16));
             }
             g.raw[0] = a2.x; g.raw[1] = a2.y; g.raw[2] = b4.x; g.raw[3] = b4.y; g.raw[4] = b4.z; g.raw[5] = b4.w;
             g.raw[6] = c4.x; g.raw[7] = c4.y; g.raw[8] = c4.z; g.raw[9] = c4.w;
@@ -174,15 +166,16 @@ __device__ __forceinline__ void gather_env(const TaskArgs& a, const BezkTaskCfg&
             // of the window around it instead of 10 scalar loads; consume() rotates by the start offset
             const char* p = reinterpret_cast<const char*>(rb);
             const uint32_t o = (uint32_t)(reinterpret_cast<uintptr_t>(p) & 15u);
-            const float4 c0 = ldg64B_nc_v4(p - o), c1 = ldg64B_nc_v4(p - o + 16), c2 = ldg64B_nc_v4(p - o + 32);
+            const float4 c0 = L2HINT(ldg64B_nc_v4, ps, p - o), c1 = L2HINT(ldg64B_nc_v4, ps, p - o + 16);
+            const float4 c2 = L2HINT(ldg64B_nc_v4, ps, p - o + 32);
             float4 c3 = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (o == 12u) c3 = ldg64B_nc_v4(p - o + 48);
+            if (o == 12u) c3 = L2HINT(ldg64B_nc_v4, ps, p - o + 48);
             g.raw[0] = c0.x; g.raw[1] = c0.y; g.raw[2] = c0.z; g.raw[3] = c0.w; g.raw[4] = c1.x; g.raw[5] = c1.y; g.raw[6] = c1.z;
             g.raw[7] = c1.w; g.raw[8] = c2.x; g.raw[9] = c2.y;
             g.win[0] = c2.z; g.win[1] = c2.w; g.win[2] = c3.x; g.win[3] = c3.y; g.win[4] = c3.z; g.win[5] = c3.w;
         } else {
 #pragma unroll
-            for (int k = 0; k < 10; ++k) g.raw[k] = ldg64B_nc(rb + k);
+            for (int k = 0; k < 10; ++k) g.raw[k] = L2HINT(ldg64B_nc, ps, rb + k);
         }
         if (OBS) {
             if (!CLEATS && a.cf_vec2) {
@@ -193,32 +186,34 @@ __device__ __forceinline__ void gather_env(const TaskArgs& a, const BezkTaskCfg&
                 const bool same_line = ((reinterpret_cast<uintptr_t>(cf_l) ^ (reinterpret_cast<uintptr_t>(cf_r) + 11u)) & ~(uintptr_t)127u) == 0;
                 const bool l_line = a.smart_granule == 2 || (a.smart_granule && (same_line || (((sl & 63u) + 12u > 64u) && (sl + 12u <= 128u))));
                 const bool r_line = a.smart_granule == 2 || (a.smart_granule && !same_line && (((sr & 63u) + 12u > 64u) && (sr + 12u <= 128u)));
-                const float2 l2 = l_line ? ldg128B_v2(cf_l) : ldg64B_v2(cf_l);
-                const float2 r2 = r_line ? ldg128B_v2(cf_r) : ldg64B_v2(cf_r);
-                g.fl[0] = l2.x; g.fl[1] = l2.y; g.fl[2] = ldg64B(cf_l + 2);
-                g.fr[0] = r2.x; g.fr[1] = r2.y; g.fr[2] = ldg64B(cf_r + 2);
+                const float2 l2 = l_line ? L2HINT(ldg128B_v2, ps, cf_l) : L2HINT(ldg64B_v2, ps, cf_l);
+                const float2 r2 = r_line ? L2HINT(ldg128B_v2, ps, cf_r) : L2HINT(ldg64B_v2, ps, cf_r);
+                g.fl[0] = l2.x; g.fl[1] = l2.y; g.fl[2] = L2HINT(ldg64B, ps, cf_l + 2);
+                g.fr[0] = r2.x; g.fr[1] = r2.y; g.fr[2] = L2HINT(ldg64B, ps, cf_r + 2);
             } else {
 #pragma unroll
-                for (int k = 0; k < NFORCE; ++k) { g.fl[k] = ldg64B(cf_l + k); g.fr[k] = ldg64B(cf_r + k); }
+                for (int k = 0; k < NFORCE; ++k) { g.fl[k] = L2HINT(ldg64B, ps, cf_l + k); g.fr[k] = L2HINT(ldg64B, ps, cf_r + k); }
             }
-            if (a.prev_lin_vel) {
+        }
+        // the carried per-env state: the same addresses every step
+        const uint64_t pk = L2H ? policy_evict_last() : 0;
+        if (OBS && a.prev_lin_vel) {
 #pragma unroll
-                for (int k = 0; k < 3; ++k) g.prev[k] = ld_f32(a.prev_lin_vel + e * 3 + k);
-            }
+            for (int k = 0; k < 3; ++k) g.prev[k] = L2HINT(ld_f32, pk, a.prev_lin_vel + e * 3 + k);
         }
         if (TASK == BEZK_TASK_KICK) {
-            const float2 g2 = ld_nc_v2(reinterpret_cast<const float2*>(a.goal) + e);
-            const float2 b2 = ld_nc_v2(reinterpret_cast<const float2*>(a.ball_init) + e);
+            const float2 g2 = L2HINT(ld_nc_v2, pk, reinterpret_cast<const float2*>(a.goal) + e);
+            const float2 b2 = L2HINT(ld_nc_v2, pk, reinterpret_cast<const float2*>(a.ball_init) + e);
             g.goal[0] = g2.x; g.goal[1] = g2.y; g.binit[0] = b2.x; g.binit[1] = b2.y;
         } else if (TASK == BEZK_TASK_WALK) {      // goal is rewritten by this kernel on reset: coherent load
-            const float2 g2 = ldg128B_v2(reinterpret_cast<const float2*>(a.goal) + e);
+            const float2 g2 = L2HINT(ldg128B_v2, pk, reinterpret_cast<const float2*>(a.goal) + e);
             g.goal[0] = g2.x; g.goal[1] = g2.y;
         } else {
-            g.gang = ld_f32(a.goal_angle + e);
+            g.gang = L2HINT(ld_f32, pk, a.goal_angle + e);
         }
         if (BOOKREW) {
-            g.reset_prev = ld_i64(a.reset_in + e);
-            g.progress = ld_i64(a.progress_in + e);
+            g.reset_prev = L2HINT(ld_i64, pk, a.reset_in + e);
+            g.progress = L2HINT(ld_i64, pk, a.progress_in + e);
             if (a.values) g.value = ld_f32(a.values + e * a.values_stride);
         }
     }
@@ -255,8 +250,8 @@ __device__ __forceinline__ void consume(const TaskArgs& a, const float* rb, Gath
 // ------------------------------------------------------------------------------------------------
 // The fused tile kernel.  PARTS: 1 bookkeeping+masked reset, 2 observations, 4 reward/termination.
 // ------------------------------------------------------------------------------------------------
-template <int PARTS, bool CLEATS, int TILE, int TASK>
-__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg) {
+template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H>
+__device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& cfg) {
     constexpr int ROOT_ROW = root_row(TASK);
     constexpr int OBS_ROW = obs_row(TASK);
     constexpr bool BOOK = (PARTS & BEZK_PART_BOOKKEEP) != 0;
@@ -302,15 +297,16 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
     float* cf_l = cf_env ? cf_env + a.cf_l_off : nullptr;
     float* cf_r = cf_env ? cf_env + a.cf_r_off : nullptr;
     Gathered<CLEATS> g;
-    gather_env<OBS, (BOOK || REW), CLEATS, TASK>(a, cfg, e, valid, rb, cf_l, cf_r, g);
+    gather_env<OBS, (BOOK || REW), CLEATS, TASK, L2H>(a, cfg, e, valid, rb, cf_l, cf_r, g);
 
 
     // ---- 2. dense tiles: TMA bulk copies (full sub-tiles) or cooperative coalesced loads (tail) ----
     if (full) {
         if (lane == 0) {
             mbar_arrive_expect_tx(s_bar, WT * (DOF_ROW + ROOT_ROW) * 4);
-            bulk_g2s(s_dof, a.dof_state + e0 * DOF_ROW, WT * DOF_ROW * 4, s_bar);
-            bulk_g2s(s_root, a.root_states + e0 * ROOT_ROW, WT * ROOT_ROW * 4, s_bar);
+            const uint64_t ps = L2H ? policy_evict_first() : 0;
+            L2HINT(bulk_g2s, ps, s_dof, a.dof_state + e0 * DOF_ROW, WT * DOF_ROW * 4, s_bar);
+            L2HINT(bulk_g2s, ps, s_root, a.root_states + e0 * ROOT_ROW, WT * ROOT_ROW * 4, s_bar);
         }
     } else {
         for (int i = lane; i < nv * DOF_ROW; i += WT) s_dof[i] = a.dof_state[e0 * DOF_ROW + i];
@@ -397,11 +393,14 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
                     else { const Philox4 x = philox_goal(a.seed, a.step); ux = u01(x.x); uy = u01(x.y); }
                     goal[0] = 4.0f * ux + -2.0f;                 // torch_rand_float(-2, 2): (hi - lo) * u + lo
                     goal[1] = 4.0f * uy + -2.0f;
-                    reinterpret_cast<float2*>(a.goal)[e] = make_float2(goal[0], goal[1]);
+                    L2HINT(st_v2, L2H ? policy_evict_last() : 0, reinterpret_cast<float2*>(a.goal) + e, make_float2(goal[0], goal[1]));
                 }
             }
-            a.timeout_buf[e] = timeout;
-            if (!REW) { a.progress_out[e] = progress; a.reset_out[e] = reset_cur; }
+            L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.timeout_buf + e, timeout);
+            if (!REW) {
+                L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress);
+                L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset_cur);
+            }
         }
     }
 
@@ -458,7 +457,7 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
         imu_term(q, v, w, pv, cfg, imu6, mo);
         if (a.prev_lin_vel) {
 #pragma unroll
-            for (int k = 0; k < 3; ++k) a.prev_lin_vel[e * 3 + k] = v[k];
+            for (int k = 0; k < 3; ++k) L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.prev_lin_vel + e * 3 + k, v[k]);
         }
         if (TASK == BEZK_TASK_ORIENT) {                                    // compute_off_angle, orient_env.py:720-733
             const float d = angle_to_goal(q, g.gang);
@@ -520,8 +519,9 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
             fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) {
-                bulk_s2g(a.obs + e0 * OBS_ROW, s_obs, WT * OBS_ROW * 4);
-                if (a.obs_clipped) bulk_s2g(a.obs_clipped + e0 * OBS_ROW, s_obs_clip, WT * OBS_ROW * 4);
+                const uint64_t po = L2H ? policy_keep(!(cfg.flags & BEZK_F_OBS_STREAMED)) : 0;
+                L2HINT(bulk_s2g, po, a.obs + e0 * OBS_ROW, s_obs, WT * OBS_ROW * 4);
+                if (a.obs_clipped) L2HINT(bulk_s2g, po, a.obs_clipped + e0 * OBS_ROW, s_obs_clip, WT * OBS_ROW * 4);
                 bulk_commit();
             }
         } else {
@@ -544,9 +544,9 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
             if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp);
             else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp);
         }
-        a.rew[e] = rew;
-        a.reset_out[e] = reset;
-        if (BOOK) { a.progress_out[e] = progress; rollout_epilogue(a, e, rew, reset, timeout, g.value); }
+        L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
+        L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
+        if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
     }
     if (REW && valid && TASK == BEZK_TASK_KICK) {
         RewardIn s;
@@ -566,12 +566,22 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
             Mth<false> mp;
             reward_term(s, cfg, progress, reset_cur, &rew, &reset, mp);
         }
-        a.rew[e] = rew;
-        a.reset_out[e] = reset;
-        if (BOOK) { a.progress_out[e] = progress; rollout_epilogue(a, e, rew, reset, timeout, g.value); }
+        L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
+        L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
+        if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
     }
 
     if (OBS && full && lane == 0) bulk_wait_read0();   // shared memory must outlive the bulk store's reads
+}
+
+template <int PARTS, bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg) {
+    task_tile<PARTS, CLEATS, TILE, TASK, false>(a, cfg);
+}
+// the same step with the L2 policy of set_l2_policy: carried state evict_last, simulator tensors evict_first
+template <int PARTS, bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_l2_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg) {
+    task_tile<PARTS, CLEATS, TILE, TASK, true>(a, cfg);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -628,12 +638,12 @@ static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>
 template <int PARTS, bool CLEATS, int TILE, int TASK>
 static cudaError_t launch_parts3(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st) {
     const size_t smem = (size_t)(smem_in_floats(TILE, TASK) + (a.obs_clipped ? smem_obs_floats(TILE, TASK) : 0)) * sizeof(float);
-    static SmemOptIn opt_in;               // per instantiation, per device
-    if (cudaError_t err = opt_in.ensure(task_tile_kernel<PARTS, CLEATS, TILE, TASK>,
-                                        (smem_in_floats(TILE, TASK) + smem_obs_floats(TILE, TASK)) * sizeof(float)))
+    static SmemOptIn opt_in, opt_in_l2;    // per instantiation, per device
+    const auto kernel = a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
+    if (cudaError_t err = (a.l2_resident ? opt_in_l2 : opt_in).ensure(kernel, (smem_in_floats(TILE, TASK) + smem_obs_floats(TILE, TASK)) * sizeof(float)))
         return err;
     const int64_t tiles = (a.n + TILE - 1) / TILE;
-    return launch_ex(task_tile_kernel<PARTS, CLEATS, TILE, TASK>, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg);
+    return launch_ex(kernel, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg);
 }
 
 template <int PARTS, int TASK>
@@ -698,6 +708,78 @@ void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg) {
     a.smart_granule = smart_granule;
     a.cf_vec2 = a.net_contact != nullptr && aligned8(a.net_contact) && (a.cf_stride % 2 == 0) && (a.cf_l_off % 2 == 0) &&
                 (a.cf_r_off % 2 == 0);
+}
+
+// L2 residency of the carried per-env state.  Between two steps the fused kernel streams ~650 B/env of simulator tensors through
+// L2 (dense tiles, 64-byte gathers) next to K0 and the rollout slots; at normal priority that evicts the ~270 B/env the step
+// re-reads or overwrites at the SAME address every step (obs rows, bookkeeping, prev_lin_vel, goal / ball_init), so each step paid
+// HBM for that state twice (write-back, re-fetch).  When the carried state of all n envs fits BEZK_L2_BUDGET_PCT of the device's
+// L2 and the step's streamed + carried bytes do not (below that L2 keeps both anyway, and the hints only cost K0 and GAE their hits),
+// the carried state is accessed with evict_last and the streams with evict_first; otherwise nothing is hinted.  Measured on B200
+// (profiles/r03_l2_resident.md): a partial set -- envs [0, k) resident at 1 048 576 envs -- and the hints at 65 536 envs were
+// both slower than no hints.  Launches whose carried buffers are not all device memory (host pipelines) are not hinted.
+#ifndef BEZK_L2_BUDGET_PCT
+#define BEZK_L2_BUDGET_PCT 75
+#endif
+static int64_t l2_bytes_of_device() {
+    static std::atomic<int64_t> bytes[64];          // per device, 0 = not read yet
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
+    int64_t b = bytes[dev].load(std::memory_order_relaxed);
+    if (b == 0) {
+        int v = 0;
+        if (cudaDeviceGetAttribute(&v, cudaDevAttrL2CacheSize, dev) != cudaSuccess) return 0;
+        b = v;
+        bytes[dev].store(b, std::memory_order_relaxed);
+    }
+    return b;
+}
+static bool on_device(const void* p) {
+    if (p == nullptr) return true;
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { (void)cudaGetLastError(); return false; }
+    return at.type == cudaMemoryTypeDevice;
+}
+void set_l2_policy(int task, uint32_t flags, TaskArgs& a) {
+    a.l2_resident = 0;
+    if (!l2_resident_enabled()) return;
+    const void* carried[] = {a.obs, a.obs_clipped, a.reset_out, a.progress_out, a.timeout_buf, a.rew, a.prev_lin_vel, a.goal,
+                             a.ball_init, a.goal_angle};
+    int64_t per_env = 0;
+    for (const void* p : carried)
+        if (!on_device(p)) return;
+    const bool obs_kept = !(flags & BEZK_F_OBS_STREAMED);
+    if (a.obs && obs_kept) per_env += obs_row(task) * 4;
+    if (a.obs_clipped && obs_kept) per_env += obs_row(task) * 4;
+    if (a.reset_out) per_env += 8;
+    if (a.progress_out) per_env += 8;
+    if (a.timeout_buf) per_env += 8;
+    if (a.rew) per_env += 4;
+    if (a.prev_lin_vel) per_env += 12;
+    if (a.goal) per_env += 8;
+    if (a.ball_init && task == BEZK_TASK_KICK) per_env += 8;
+    if (a.goal_angle && task == BEZK_TASK_ORIENT) per_env += 4;
+    const int64_t l2 = l2_bytes_of_device();
+    // per env and step the simulator tensors cost the two dense rows and at least three 64-byte granules (IMU slice, two feet)
+    const int64_t streamed = (DOF_ROW + root_row(task)) * 4 + 3 * 64;
+    if (per_env == 0 || a.n * per_env > l2 * BEZK_L2_BUDGET_PCT / 100 || a.n * (per_env + streamed) <= l2) return;
+    a.l2_resident = 1;
+}
+
+// applypriority works on one 128-byte line: only the lines entirely inside the range are touched
+__global__ void __launch_bounds__(256) l2_release_kernel(const char* base, int64_t lines) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < lines; i += (int64_t)gridDim.x * blockDim.x)
+        asm volatile("applypriority.global.L2::evict_normal [%0], 128;" ::"l"(base + i * 128) : "memory");
+}
+cudaError_t launch_l2_release(const void* ptr, uint64_t bytes, cudaStream_t st) {
+    const uintptr_t lo = (reinterpret_cast<uintptr_t>(ptr) + 127) & ~(uintptr_t)127;
+    const uintptr_t hi = (reinterpret_cast<uintptr_t>(ptr) + bytes) & ~(uintptr_t)127;
+    if (hi <= lo) return cudaSuccess;
+    const int64_t lines = (int64_t)((hi - lo) / 128);
+    int64_t blocks = (lines + 255) / 256;
+    if (blocks > 148LL * 16) blocks = 148LL * 16;
+    l2_release_kernel<<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const char*>(lo), lines);
+    return cudaGetLastError();
 }
 
 // Host pipeline: the sparse Isaac Gym rows leave PINNED HOST memory through the copy engines -- strided cudaMemcpy2DAsync

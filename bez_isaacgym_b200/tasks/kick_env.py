@@ -24,6 +24,7 @@ aliases ``obs_buf`` when ``clip_obs`` is infinite (the reference's clamp is then
 """
 import ctypes as C
 import math
+import weakref
 
 import numpy as np
 import torch
@@ -37,6 +38,13 @@ _P = C.c_void_p
 
 def _ptr(t):
     return _P(t.data_ptr()) if t is not None else None
+
+
+def _l2_release(lib, tensors):
+    if torch.cuda.is_current_stream_capturing():   # collected while another graph is being captured: not into that graph
+        return
+    for t in tensors:
+        lib.bezk_l2_release(t.data_ptr(), t.numel() * t.element_size(), torch.cuda.current_stream(t.device).cuda_stream)
 
 
 class KickEnv(VecTask):
@@ -204,6 +212,11 @@ class KickEnv(VecTask):
         self._rollout = None                # (BezkRolloutCfg, values, shaped_rewards, dones_u8) set by set_rollout_targets
         self._d_values = None               # staged_ce host pipeline: device image of host-resident critic values
         self._lib = _lib.load()
+        # the step keeps these in L2 with evict_last (bezk.h, bezk_l2_release): demoted again when the env goes away
+        carried = [self.obs_buf, self.obs_clipped_buf, self.reset_buf, self.progress_buf, self.timeout_buf, self.rew_buf,
+                   self._prev_buf, self.goal, self.ball_init, self.goal_angle]
+        self._l2_finalizer = weakref.finalize(self, _l2_release, self._lib, [t for t in carried if t is not None and t.is_cuda])
+        self._l2_finalizer.atexit = False   # at interpreter exit the CUDA context goes away with the process
         if self.host_staged:
             pin = dict(pin_memory=True)
             self._h_obs = torch.empty(n, self._obs_width, **pin); self._h_rew = torch.empty(n, **pin)
@@ -731,6 +744,10 @@ class KickEnv(VecTask):
                                   self.progress_buf, None, self._kcfg, None, self.rew_buf, goal_angle=self.goal_angle,
                                   parts=_lib.PART_REWARD)
 
+    def close(self):
+        """Give back the L2 priority the step gave this env's carried buffers (also done when the env is collected)."""
+        self._l2_finalizer()
+
     def reset_idx(self, env_ids):
         """kick_env.py:779-850 for an explicit id list (the per-step path uses the masked reset inside the fused
         kernel instead, which needs no ``nonzero()``)."""
@@ -766,6 +783,7 @@ class KickEnv(VecTask):
                 or tensor.device != self.compute_device:
             raise ValueError(f"obs target must be a contiguous float32 ({self.num_envs}, {self._obs_width}) tensor on "
                              f"{self.compute_device}")
+        self._kcfg.flags |= _lib.F_OBS_STREAMED      # a rollout slot is written once per rollout: not worth keeping in L2
         if self.obs_clipped_buf is not None:
             # finite clip_obs: what step() returns -- and what rl_games stores -- is the CLIPPED row (vec_task.py:343); the
             # raw obs_buf stays private

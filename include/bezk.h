@@ -35,6 +35,8 @@ extern "C" {
 #define BEZK_F_RESET_ROOT_STATES   4u  /* masked reset also copies initial_root_states rows into
                                           root_states (what the simulator's indexed setters do,
                                           tasks/kick_env.py:831-837); off when a real simulator owns that */
+#define BEZK_F_OBS_STREAMED        8u  /* obs / obs_clipped point at a different buffer every step (e.g. the next slot of a
+                                          rollout buffer): their rows are not kept resident in L2 (bezk_l2_release) */
 
 /* Constants of one BezKick instance.  Passed BY VALUE into the kernels (constant bank).
  * ref: tasks/kick_env.py:46-238 (constructor), cfg/task/bez_kick.yaml. */
@@ -373,6 +375,14 @@ int bezk_reset_idx_task(int task, const int64_t* env_ids, int64_t k, const float
                         const BezkTaskCfg* cfg, int64_t env_base, int64_t n, void* stream);
 /* The (2,) uniforms the Philox path uses for the goal draw of (seed, step). */
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream);
+/* The device-memory post-physics entries (bezk_post_physics, _task, _rollout, bezk_compute_*) access the state an env carries
+ * from step to step -- obs (and obs_clipped) rows, reset / progress / time-out flags, rew, prev_lin_vel, goal, ball_init /
+ * goal_angle -- with the L2 eviction priority evict_last when that state of all n envs fits 75 % of the device's L2 and one
+ * step streams more than L2 holds (per-instruction cache hints; no set-aside, no access-policy window, no device limit).  Lines so marked keep that priority while
+ * they stay in L2, also after the buffers are freed: an owner that drops those buffers calls bezk_l2_release on each of them
+ * first (stream-ordered; the 128-byte lines entirely inside [ptr, ptr + bytes) go back to the normal priority).  Env
+ * BEZK_L2_RESIDENT=0 (read once per process) turns the hints off. */
+int bezk_l2_release(const void* ptr, uint64_t bytes, void* stream);
 
 /* ---------------------------------------------------------------- rollout storage (SURVEY 8f rows 1-2) ----- */
 
