@@ -62,7 +62,8 @@ static void set_rollout(bezk::TaskArgs& a, const BezkRolloutCfg* rollout, const 
     }
 }
 
-static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK) {
+static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK,
+                    bezk::EpArgs* ep = nullptr) {
     if (int rc = check_cfg(cfg)) return rc;
     REQUIRE(a.n >= 0, "n < 0");
     if (a.n == 0) return 0;
@@ -83,7 +84,11 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
         if (cfg->flags & BEZK_F_RESET_ROOT_STATES) REQUIRE(a.initial_root, "initial_root_states NULL");
     }
     bezk::fill_alignment(a, *cfg);
-    bezk::set_l2_policy(task, cfg->flags, a);
+    bezk::set_l2_policy(task, cfg->flags, a, ep);
+    if (ep) {                              // the one-shot kernel with the episode accumulators (the persistent one has none)
+        ep->w = (a.n + 31) / 32;
+        return cuda_rc(bezk::launch_task_ep(task, a, *cfg, *ep, (cudaStream_t)stream), where);
+    }
     if (bezk::persist_eligible(task, parts, a, *cfg))          // the persistent pipelined kernel (bezk_task_persist.cu)
         return cuda_rc(bezk::launch_task_persist(a, *cfg, (cudaStream_t)stream), where);
     return cuda_rc(bezk::launch_task(task, parts, a, *cfg, (cudaStream_t)stream), where);
@@ -310,17 +315,21 @@ int bezk_post_physics_task(int task, float* dof_state, const float* rigid_body, 
     return run_task(parts, a, cfg, stream, "bezk_post_physics_task", task);
 }
 
-int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
-                              float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
-                              const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
-                              uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf,
-                              const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, const BezkRolloutCfg* rollout,
-                              const float* values, float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
-                              void* stream) {
+int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                 float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                 const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
+                                 uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf,
+                                 const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, const BezkRolloutCfg* rollout,
+                                 const float* values, float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                 float* ep_return, float* ep_length, double* ep_partials, void* stream) {
     REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
     REQUIRE(env_base >= 0, "env_base < 0");
     REQUIRE(!shaped_rewards || rollout, "shaped_rewards requested without a BezkRolloutCfg");
     REQUIRE(!(shaped_rewards && rollout && rollout->value_bootstrap) || values, "value_bootstrap needs values");
+    const int armed = (ep_return != nullptr) + (ep_length != nullptr) + (ep_partials != nullptr);
+    REQUIRE(armed == 0 || armed == 3, "ep_return, ep_length and ep_partials must be all NULL or all non-NULL");
+    if (armed && !(ALIGNED(ep_return, 4) && ALIGNED(ep_length, 4) && ALIGNED(ep_partials, 8)))
+        return fail(BEZK_E_ALIGN, "ep_return / ep_length must be 4-byte and ep_partials 8-byte aligned");
     bezk::TaskArgs a;
     memset(&a, 0, sizeof(a));
     a.dof_state = dof_state; a.rigid_body = rigid_body; a.root_states = root_states; a.net_contact = net_contact;
@@ -330,7 +339,34 @@ int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_bod
     a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
     a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
     set_rollout(a, rollout, values, shaped_rewards, dones_u8);
-    return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream, "bezk_post_physics_rollout", task);
+    bezk::EpArgs ep = {ep_return, ep_length, ep_partials, 0};
+    return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream,
+                    armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout", task, armed ? &ep : nullptr);
+}
+
+int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                              float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                              const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
+                              uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf,
+                              const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, const BezkRolloutCfg* rollout,
+                              const float* values, float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                              void* stream) {
+    return bezk_post_physics_rollout_ep(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
+                                        initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf,
+                                        randomize_buf, cfg, obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n,
+                                        nullptr, nullptr, nullptr, stream);
+}
+
+int bezk_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2, int64_t* size2,
+                              void* stream) {
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    REQUIRE(games_to_track > 0, "games_to_track must be positive");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(partials && mean2 && size2, "partials / mean2 / size2 NULL");
+    if (!ALIGNED(partials, 8) || !ALIGNED(mean2, 4) || !ALIGNED(size2, 8))
+        return fail(BEZK_E_ALIGN, "partials / size2 must be 8-byte and mean2 4-byte aligned");
+    return cuda_rc(bezk::launch_episode_meter_update(partials, steps, n, games_to_track, mean2, size2, (cudaStream_t)stream),
+                   "bezk_episode_meter_update");
 }
 
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream) {

@@ -52,8 +52,17 @@ struct TaskArgs {
     // ball_init / goal_angle) with evict_last and the dense tiles and sparse gathers with evict_first (task_tile_l2_kernel)
     int l2_resident;
 };
-// fills l2_resident (bezk_task.cu): after fill_alignment, before the launch
-void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a);
+// Episode accumulators of the fused step (bezk_post_physics_rollout_ep; rl_games play_steps' current_rewards / current_lengths and
+// the done-env sums its game_rewards / game_lengths meters are fed with).  A separate kernel parameter of task_tile_ep_kernel /
+// task_tile_ep_l2_kernel, not TaskArgs fields: a longer TaskArgs would move the BezkTaskCfg parameter of every other kernel.
+struct EpArgs {
+    float* ret;                  // (n,) carried episode return: ret + rew, times (1 - done)
+    float* len;                  // (n,) carried episode length: len + 1, times (1 - done)
+    double* partials;            // (3, W), W = ceil(n / 32): per warp of 32 envs [count of done envs, sum of their return, sum of their length]
+    int64_t w;                   // W
+};
+// fills l2_resident (bezk_task.cu): after fill_alignment, before the launch; ep: the armed episode accumulators or nullptr
+void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a, const EpArgs* ep = nullptr);
 // demote [ptr, ptr + bytes) to the normal L2 eviction priority (the 128-byte lines entirely inside the range)
 cudaError_t launch_l2_release(const void* ptr, uint64_t bytes, cudaStream_t st);
 struct PpoArgs {
@@ -69,6 +78,11 @@ struct PpoArgs {
     int use_tma;
 };
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st);
+// the whole step (parts = 7) with the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel)
+cudaError_t launch_task_ep(int task, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st);
+// folds `steps` x (3, ceil(n / 32)) partials of launch_task_ep into the two AverageMeters (bezk_rollout.cu)
+cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
+                                        int64_t* size2, cudaStream_t st);
 cudaError_t launch_goal_uniforms(uint64_t seed, uint64_t step, float* out2, cudaStream_t st);
 void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg);
 bool persist_eligible(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg);

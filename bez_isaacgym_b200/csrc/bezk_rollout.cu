@@ -513,4 +513,118 @@ cudaError_t launch_selftest_fastmath(uint64_t pairs, uint64_t seed, unsigned lon
     return cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------
+// Episode meters: rl_games' game_rewards / game_lengths (torch_ext.AverageMeter, games_to_track) fed by the per-step partials of
+// the fused step with episode accumulators ((T, 3, W): per warp of 32 envs the count of done envs, the sum of their returns and
+// of their lengths).  One launch, no host round trip: CTA t reduces step t's 3 x W partials in a fixed order (the same bits every
+// run), and the last CTA to finish (ticket) runs the AverageMeter recurrence over the steps in order in one warp:
+//   new_mean = sum / count (fp64, rounded to fp32); size = min(count, max_size); old_size = min(max_size - size, current_size)
+//   current_size = old_size + size; mean = (mean * old_size + new_mean * size) / current_size    (fp32, rl_games' order)
+// No CTA-wide barrier: the warps of a CTA meet through a ticket as well.
+// ------------------------------------------------------------------------------------------------
+constexpr int EPM_THREADS = 256;
+constexpr int EPM_WARPS = EPM_THREADS / 32;
+
+struct EpmScratch {
+    double* warp_sums;     // (steps, EPM_WARPS, 3)
+    double* step_sums;     // (steps, 3)
+    unsigned* tickets;     // (steps + 1,) zeroed: per step (its warps), then the steps
+};
+
+__global__ void __launch_bounds__(EPM_THREADS) episode_meter_kernel(const double* __restrict__ partials, int steps, int64_t w,
+                                                                    int64_t max_size, EpmScratch sc, float* mean2, int64_t* size2) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int step = blockIdx.x;
+    pdl_launch_dependents();
+    pdl_wait();
+    const double* p = partials + (int64_t)step * 3 * w;
+    double acc[3] = {0.0, 0.0, 0.0};
+    for (int64_t i = threadIdx.x; i < w; i += EPM_THREADS) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) acc[k] += p[k * w + i];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) acc[k] += __shfl_down_sync(0xffffffffu, acc[k], o);
+    }
+    const unsigned full = 0xffffffffu;
+    int last = 0;
+    if (lane == 0) {
+        double* ws = sc.warp_sums + ((int64_t)step * EPM_WARPS + warp) * 3;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) ws[k] = acc[k];
+        __threadfence();
+        last = atomicAdd(&sc.tickets[step], 1u) == EPM_WARPS - 1;
+    }
+    if (!__shfl_sync(full, last, 0)) return;
+    // the last warp of this CTA: the step's sums, warp by warp in order
+    __threadfence();
+    if (lane == 0) {
+        const double* wsum = sc.warp_sums + (int64_t)step * EPM_WARPS * 3;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            double v = 0.0;
+#pragma unroll
+            for (int j = 0; j < EPM_WARPS; ++j) v += __ldcg(wsum + j * 3 + k);
+            sc.step_sums[step * 3 + k] = v;
+        }
+        __threadfence();
+        last = atomicAdd(&sc.tickets[steps], 1u) == (unsigned)steps - 1;
+    }
+    if (!__shfl_sync(full, last, 0)) return;
+    // the last step to finish: the recurrence, step by step in order.  Lane j of the warp loads step t0 + j's sums, so the
+    // loads of 32 steps are in flight together; every lane then runs the same recurrence on the shuffled values.
+    __threadfence();
+    float mean[2] = {mean2[0], mean2[1]};
+    int64_t cur[2] = {size2[0], size2[1]};     // 0: game_rewards (returns), 1: game_lengths
+    for (int t0 = 0; t0 < steps; t0 += 32) {
+        double c = 0.0, s[2] = {0.0, 0.0};
+        if (t0 + lane < steps) {
+            c = __ldcg(sc.step_sums + 3 * (t0 + lane));
+            s[0] = __ldcg(sc.step_sums + 3 * (t0 + lane) + 1);
+            s[1] = __ldcg(sc.step_sums + 3 * (t0 + lane) + 2);
+        }
+        const int m = steps - t0 < 32 ? steps - t0 : 32;
+        for (int j = 0; j < m; ++j) {
+            const double cnt = __shfl_sync(full, c, j);
+            const double sum[2] = {__shfl_sync(full, s[0], j), __shfl_sync(full, s[1], j)};
+            if (!(cnt > 0.0)) continue;           // AverageMeter.update: size == 0 -> no-op
+            const int64_t size = (int64_t)cnt < max_size ? (int64_t)cnt : max_size;
+#pragma unroll
+            for (int k = 0; k < 2; ++k) {
+                const float new_mean = (float)(sum[k] / cnt);
+                const int64_t old_size = (max_size - size) < cur[k] ? (max_size - size) : cur[k];
+                const int64_t size_sum = old_size + size;
+                cur[k] = size_sum;
+                mean[k] = (mean[k] * (float)old_size + new_mean * (float)size) / (float)size_sum;
+            }
+        }
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) { mean2[k] = mean[k]; size2[k] = cur[k]; }
+    }
+}
+
+cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
+                                        int64_t* size2, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    // the sums and tickets live for this launch only: stream-ordered scratch (capturable in a CUDA graph, no host synchronisation)
+    const size_t nd = (size_t)steps * (EPM_WARPS + 1) * 3, bytes = nd * sizeof(double) + (size_t)(steps + 1) * sizeof(unsigned);
+    void* buf = nullptr;
+    cudaError_t e = cudaMallocAsync(&buf, bytes, st);
+    if (e != cudaSuccess) return e;
+    EpmScratch sc;
+    sc.warp_sums = static_cast<double*>(buf);
+    sc.step_sums = sc.warp_sums + (size_t)steps * EPM_WARPS * 3;
+    sc.tickets = reinterpret_cast<unsigned*>(sc.warp_sums + nd);
+    e = cudaMemsetAsync(sc.tickets, 0, (size_t)(steps + 1) * sizeof(unsigned), st);
+    if (e == cudaSuccess)
+        e = launch_ex(episode_meter_kernel, dim3((unsigned)steps), dim3(EPM_THREADS), 0, st, partials, steps, (n + 31) / 32,
+                      games_to_track, sc, mean2, size2);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
 }  // namespace bezk

@@ -250,8 +250,25 @@ __device__ __forceinline__ void consume(const TaskArgs& a, const float* rb, Gath
 // ------------------------------------------------------------------------------------------------
 // The fused tile kernel.  PARTS: 1 bookkeeping+masked reset, 2 observations, 4 reward/termination.
 // ------------------------------------------------------------------------------------------------
-template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H>
-__device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& cfg) {
+// rl_games' episode bookkeeping of one env in the reward epilogue (episode_step), its carried values stored like the bookkeeping
+template <bool L2H>
+__device__ __forceinline__ void episode_epilogue(const EpArgs& ep, int64_t e, float rew, int64_t reset, float ret, float len, bool& done,
+                                                 float& r, float& l) {
+    float ret_out, len_out;
+    episode_step(ret, len, rew, reset, r, l, ret_out, len_out);
+    const uint64_t pk = L2H ? policy_evict_last() : 0;
+    L2HINT(st_f32, pk, ep.ret + e, ret_out);
+    L2HINT(st_f32, pk, ep.len + e, len_out);
+    done = reset != 0;
+}
+
+// Ep: empty, or one EpArgs -- then EP is on and the episode accumulators ride along (task_tile_ep_kernel / task_tile_ep_l2_kernel;
+// whole step only).  A parameter pack rather than an always-present argument: the kernels without accumulators make exactly the
+// call they made before the accumulators existed (an unused EpArgs argument alone changes their register allocation).
+template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H, typename... Ep>
+__device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& cfg, const Ep&... eps) {
+    constexpr bool EP = sizeof...(Ep) == 1;
+    static_assert(!EP || PARTS == 7, "the episode accumulators ride in the whole step");
     constexpr int ROOT_ROW = root_row(TASK);
     constexpr int OBS_ROW = obs_row(TASK);
     constexpr bool BOOK = (PARTS & BEZK_PART_BOOKKEEP) != 0;
@@ -298,6 +315,17 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     float* cf_r = cf_env ? cf_env + a.cf_r_off : nullptr;
     Gathered<CLEATS> g;
     gather_env<OBS, (BOOK || REW), CLEATS, TASK, L2H>(a, cfg, e, valid, rb, cf_l, cf_r, g);
+    float ep_ret = 0.0f, ep_len = 0.0f;    // carried like the bookkeeping: the same addresses every step
+    if constexpr (EP) {
+        const EpArgs& ep = (eps, ...);
+        if (valid) {
+            const uint64_t pk = L2H ? policy_evict_last() : 0;
+            ep_ret = L2HINT(ld_f32, pk, ep.ret + e);
+            ep_len = L2HINT(ld_f32, pk, ep.len + e);
+        }
+    }
+    bool ep_done = false;                  // this env's episode ended in this step, with return ep_r and length ep_l
+    float ep_r = 0.0f, ep_l = 0.0f;
 
 
     // ---- 2. dense tiles: TMA bulk copies (full sub-tiles) or cooperative coalesced loads (tail) ----
@@ -547,6 +575,7 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
         L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
         if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
+        if constexpr (EP) episode_epilogue<L2H>((eps, ...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
     }
     if (REW && valid && TASK == BEZK_TASK_KICK) {
         RewardIn s;
@@ -569,6 +598,27 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
         L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
         if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
+        if constexpr (EP) episode_epilogue<L2H>((eps, ...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
+    }
+
+    // ---- 9. this warp's slot of the per-step episode statistics: [count of done envs, sum of their returns, sum of their
+    // lengths] at (k, env / 32).  Fixed-order shuffle tree, one store per value, every step (zeros included): nothing needs
+    // zeroing, no atomics, and the sums are the same bits from run to run ----
+    if constexpr (EP) if (nv > 0) {
+        const EpArgs& ep = (eps, ...);
+        const unsigned done_mask = __ballot_sync(0xffffffffu, ep_done);
+        double sr = ep_done ? (double)ep_r : 0.0, sl = ep_done ? (double)ep_l : 0.0;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            sr += __shfl_down_sync(0xffffffffu, sr, o);
+            sl += __shfl_down_sync(0xffffffffu, sl, o);
+        }
+        if (lane == 0) {
+            const int64_t slot = e0 / WT;
+            ep.partials[slot] = (double)__popc(done_mask);
+            ep.partials[ep.w + slot] = sr;
+            ep.partials[2 * ep.w + slot] = sl;
+        }
     }
 
     if (OBS && full && lane == 0) bulk_wait_read0();   // shared memory must outlive the bulk store's reads
@@ -582,6 +632,17 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_k
 template <int PARTS, bool CLEATS, int TILE, int TASK>
 __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_l2_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg) {
     task_tile<PARTS, CLEATS, TILE, TASK, true>(a, cfg);
+}
+// the whole step with the episode accumulators (bezk_post_physics_rollout_ep), plain and with the L2 policy
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_ep_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg,
+                                                                                         const EpArgs ep) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, ep);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_ep_l2_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg,
+                                                                                            const EpArgs ep) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -644,6 +705,31 @@ static cudaError_t launch_parts3(const TaskArgs& a, const BezkTaskCfg& cfg, cuda
         return err;
     const int64_t tiles = (a.n + TILE - 1) / TILE;
     return launch_ex(kernel, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg);
+}
+
+template <bool CLEATS, int TILE, int TASK>
+static cudaError_t launch_ep3(const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st) {
+    const size_t smem = (size_t)(smem_in_floats(TILE, TASK) + (a.obs_clipped ? smem_obs_floats(TILE, TASK) : 0)) * sizeof(float);
+    static SmemOptIn opt_in, opt_in_l2;
+    const auto kernel = a.l2_resident ? task_tile_ep_l2_kernel<CLEATS, TILE, TASK> : task_tile_ep_kernel<CLEATS, TILE, TASK>;
+    if (cudaError_t err = (a.l2_resident ? opt_in_l2 : opt_in).ensure(kernel, (smem_in_floats(TILE, TASK) + smem_obs_floats(TILE, TASK)) * sizeof(float)))
+        return err;
+    const int64_t tiles = (a.n + TILE - 1) / TILE;
+    return launch_ex(kernel, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg, ep);
+}
+
+template <int TASK>
+static cudaError_t launch_ep(const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st) {
+    return (cfg.flags & BEZK_F_CLEATS) ? launch_ep3<true, BEZK_TILE, TASK>(a, cfg, ep, st) : launch_ep3<false, BEZK_TILE, TASK>(a, cfg, ep, st);
+}
+
+cudaError_t launch_task_ep(int task, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st) {
+    switch (task) {
+        case BEZK_TASK_KICK: return launch_ep<BEZK_TASK_KICK>(a, cfg, ep, st);
+        case BEZK_TASK_WALK: return launch_ep<BEZK_TASK_WALK>(a, cfg, ep, st);
+        case BEZK_TASK_ORIENT: return launch_ep<BEZK_TASK_ORIENT>(a, cfg, ep, st);
+        default: return cudaErrorInvalidValue;
+    }
 }
 
 template <int PARTS, int TASK>
@@ -740,12 +826,12 @@ static bool on_device(const void* p) {
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { (void)cudaGetLastError(); return false; }
     return at.type == cudaMemoryTypeDevice;
 }
-void set_l2_policy(int task, uint32_t flags, TaskArgs& a) {
+void set_l2_policy(int task, uint32_t flags, TaskArgs& a, const EpArgs* ep) {
     a.l2_resident = 0;
     if (!l2_resident_enabled()) return;
     const void* carried[] = {a.obs, a.obs_clipped, a.reset_out, a.progress_out, a.timeout_buf, a.rew, a.prev_lin_vel, a.goal,
-                             a.ball_init, a.goal_angle};
-    int64_t per_env = 0;
+                             a.ball_init, a.goal_angle, ep ? ep->ret : nullptr, ep ? ep->len : nullptr};
+    int64_t per_env = ep ? 8 : 0;          // the two episode accumulators, when armed
     for (const void* p : carried)
         if (!on_device(p)) return;
     const bool obs_kept = !(flags & BEZK_F_OBS_STREAMED);

@@ -245,6 +245,19 @@ __device__ __forceinline__ void rollout_epilogue(const TaskArgs& a, int64_t e, f
     if (a.dones_u8) a.dones_u8[e] = (uint8_t)(reset != 0);
 }
 
+// rl_games play_steps episode bookkeeping of one env (a2c_common.py; `rewards` is the unshaped rew_buf, `dones` the reset mask):
+//   current_rewards += rewards; current_lengths += 1; ...; current_* = current_* * not_dones
+// r / l are what a done env hands to the game_rewards / game_lengths meters; the carried values are written back as MULTIPLIES by
+// (1 - done), so a NaN / inf return stays NaN in the accumulator after the env is done, as in rl_games.
+__device__ __forceinline__ void episode_step(float ret, float len, float rew, int64_t reset, float& r, float& l, float& ret_out,
+                                             float& len_out) {
+    r = ret + rew;
+    l = len + 1.0f;
+    const float not_done = 1.0f - (reset != 0 ? 1.0f : 0.0f);
+    ret_out = r * not_done;
+    len_out = l * not_done;
+}
+
 // reset_idx DOF part, kick_env.py:786-791
 __device__ __forceinline__ void reset_dof_row(const float (&u)[36], const BezkTaskCfg& c, float (&row)[36]) {
 #pragma unroll

@@ -15,11 +15,14 @@ SUM-all-reduced (exact merge) and the gradients averaged on one flat bucket.  ``
 ``epoch``, ``frame``, ``last_mean_rewards``), with the network's parameters under the ``a2c_network.*`` names of the reference's
 shipped checkpoint (``results/Bez_Kick/Normal/Bez_Kick_33.pth``), so that checkpoint loads.
 """
+import os
+
 import torch
 from torch import nn
 
 from .. import dist as bdist
 from . import a2c_common, experience, losses
+from .episode_meter import EpisodeMeter
 from .policy_head import policy_head as _policy_head
 from .running_mean_std import RunningMeanStd
 
@@ -64,6 +67,11 @@ DEFAULT_CONFIG = dict(gamma=0.99, tau=0.95, learning_rate=3e-4, lr_schedule="ada
                       clip_value=True, entropy_coef=0.0, bounds_loss_coef=0.001, normalize_input=True, normalize_value=True,
                       normalize_advantage=True, value_bootstrap=True, reward_shaper=dict(scale_value=0.01), mixed_precision=True,
                       bound_form="v1.1.3", cuda_graph=False)
+#: rl_games A2CBase's training-loop settings (RECALLED defaults of v1.1.3): meters of the last ``games_to_track`` episodes, best
+#: checkpoint ``<name>.pth`` once ``epoch >= save_best_after``, a ``last_`` checkpoint every ``save_frequency`` epochs (0: never),
+#: stop when the best mean return exceeds ``score_to_win`` or after ``max_epochs`` epochs
+TRAIN_DEFAULTS = dict(games_to_track=100, save_best_after=100, save_frequency=0, score_to_win=1e9, max_epochs=int(1e6),
+                      name="Bez_Kick")
 
 
 class A2CAgent:
@@ -74,7 +82,7 @@ class A2CAgent:
         ``global_advantage_stats``) the advantage moments all use the same group, so a rank-0 checkpoint carries the
         statistics of every shard.  Pass ``env.env_base`` = the rank's shard offset (``cfg['env']['envBase']``) so that the
         reset / exploration noise is keyed by global env ids."""
-        cfg = dict(DEFAULT_CONFIG)
+        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS)
         cfg.update(config or {})
         process_group = bdist.resolve_group(process_group)
         self.config, self.env, self.group = cfg, env, process_group
@@ -120,6 +128,12 @@ class A2CAgent:
         self._head_step = 0
         self._seed = seed
         self.last_mean_rewards = -100500.0
+        # rl_games play_steps' episode statistics, carried by the step kernel: current_rewards / current_lengths per env, the
+        # per-step done-env partials (count, return sum, length sum per 32 envs) and the game_rewards / game_lengths meters
+        self.current_rewards = torch.zeros(N, **f32)
+        self.current_lengths = torch.zeros(N, **f32)
+        self._ep_partials = torch.zeros(T, 3, (N + 31) // 32, dtype=torch.float64, device=self.device)
+        self.game_rewards, self.game_lengths = EpisodeMeter.pair(int(cfg["games_to_track"]), self.device)
         self.obs = env.reset()["obs"].clone()
         self.dones = torch.zeros(N, dtype=torch.uint8, device=self.device)
         self.dataset = None
@@ -163,12 +177,14 @@ class A2CAgent:
                 env.set_rollout_targets(values=res["values"], shaped_rewards=self.mb_rewards[t],
                                         dones_u8=buf.slot("dones", t + 1) if t + 1 < T else self.dones, gamma=self.gamma,
                                         scale_value=shaper.get("scale_value", 1.0), shift_value=shaper.get("shift_value", 0.0),
-                                        value_bootstrap=self.config["value_bootstrap"])
+                                        value_bootstrap=self.config["value_bootstrap"], episode_returns=self.current_rewards,
+                                        episode_lengths=self.current_lengths, episode_partials=self._ep_partials[t])
                 if head_targets:
                     env.step_precomputed_targets(res["env_actions"])
                 else:
                     env.step(res["env_actions"])
             env.set_rollout_targets()
+            self.game_rewards.update(self._ep_partials, self.num_actors)      # both meters, the T steps in order
             _, last_v = self._forward(self._norm_obs(self.obs))
             last_values = self.value_mean_std(last_v, unnorm=True) if self.config["normalize_value"] else last_v
             a2c_common.discount_values(self.dones, last_values, buf.tensor_dict["dones"], buf.tensor_dict["values"], self.mb_rewards,
@@ -296,6 +312,50 @@ class A2CAgent:
         last = self._learn_graphed() if self.config["cuda_graph"] else self._learn_eager()
         self.epoch_num += 1
         return dict(a_loss=last["a_loss"], c_loss=last["c_loss"], kl=last["kl"], lr=self.last_lr)
+
+    def train(self, directory):
+        """rl_games ``A2CBase.train`` (RECALLED): ``train_epoch`` until a stop rule fires.  After each epoch with finished games
+        (``game_rewards.current_size > 0``), rank 0 saves ``<directory>/<name>.pth`` when the mean return beats
+        ``last_mean_rewards`` and ``epoch >= save_best_after`` (then stops if it exceeds ``score_to_win``), and
+        ``last_<name>_ep_<epoch>.pth`` every ``save_frequency`` epochs; the loop stops after ``max_epochs`` epochs.  The meters
+        are per rank, as in rl_games.  Deviation: rank 0 broadcasts its stop decision every epoch, so every rank leaves on the
+        same epoch (in rl_games the other ranks would wait in the next epoch's collectives).  Returns ``(last_mean_rewards,
+        epoch)`` and a per-epoch history (mean return / length or None before the first finished game, losses, lr)."""
+        cfg = self.config
+        rank0 = not bdist.is_distributed(self.group) or torch.distributed.get_rank() == 0
+        if rank0:
+            os.makedirs(directory, exist_ok=True)
+        history = []
+        while True:
+            info = self.train_epoch()
+            epoch = self.epoch_num
+            row = dict(epoch=epoch, mean_reward=None, mean_length=None, a_loss=float(info["a_loss"]), c_loss=float(info["c_loss"]),
+                       kl=float(info["kl"]), lr=float(info["lr"]))
+            should_exit = False
+            if rank0:
+                if self.game_rewards.current_size > 0:
+                    mean_rewards = float(self.game_rewards.get_mean()[0])
+                    row["mean_reward"], row["mean_length"] = mean_rewards, float(self.game_lengths.get_mean()[0])
+                    if cfg["save_frequency"] > 0 and epoch % cfg["save_frequency"] == 0 and mean_rewards <= self.last_mean_rewards:
+                        self.save(os.path.join(directory, f"last_{cfg['name']}_ep_{epoch}"))
+                    if mean_rewards > self.last_mean_rewards and epoch >= cfg["save_best_after"]:
+                        self.last_mean_rewards = mean_rewards
+                        self.save(os.path.join(directory, cfg["name"]))
+                        if self.last_mean_rewards > cfg["score_to_win"]:
+                            should_exit = True
+                if epoch >= cfg["max_epochs"]:
+                    should_exit = True
+            history.append(row)
+            if bdist.is_distributed(self.group):
+                flag = torch.tensor([1.0 if should_exit else 0.0], device=self.device)
+                torch.distributed.broadcast(flag, src=0, group=self.group)
+                should_exit = bool(flag.item())
+            if should_exit:
+                return (self.last_mean_rewards, epoch), history
+
+    def save(self, path):
+        """rl_games ``torch_ext.save_checkpoint``: ``torch.save(get_full_state_weights(), path + '.pth')``."""
+        torch.save(self.get_full_state_weights(), path + ".pth")
 
     # ------------------------------------------------------------------ checkpoints (rl_games keys)
     def get_full_state_weights(self):

@@ -210,6 +210,7 @@ class KickEnv(VecTask):
         self._rng_step = 0
         self._ce_copy_out = False
         self._rollout = None                # (BezkRolloutCfg, values, shaped_rewards, dones_u8) set by set_rollout_targets
+        self._episode = None                # (episode_returns, episode_lengths, episode_partials) set by set_rollout_targets
         self._d_values = None               # staged_ce host pipeline: device image of host-resident critic values
         self._lib = _lib.load()
         # the step keeps these in L2 with evict_last (bezk.h, bezk_l2_release): demoted again when the env goes away
@@ -509,6 +510,14 @@ class KickEnv(VecTask):
             ro = self._rollout
             tail = ([C.byref(ro[0]), _ptr(ro[1]), _ptr(ro[2]), _ptr(ro[3])] if ro is not None else [None, None, None, None])
             t = f["tail"]
+            if self._episode is not None:     # + rl_games' episode return / length bookkeeping (set_rollout_targets)
+                rc = self._lib.bezk_post_physics_rollout_ep(ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed,
+                                                            self._rng_step, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], *tail,
+                                                            self.env_base, self.num_envs, *[_ptr(x) for x in self._episode],
+                                                            self._stream())
+                if rc:
+                    _lib.check(rc, "bezk_post_physics_rollout_ep")
+                return
             rc = self._lib.bezk_post_physics_rollout(ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed,
                                                      self._rng_step, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], *tail,
                                                      self.env_base, self.num_envs, self._stream())
@@ -794,17 +803,34 @@ class KickEnv(VecTask):
             self._post_fixed["tail"][5] = _ptr(tensor)
 
     def set_rollout_targets(self, values=None, shaped_rewards=None, dones_u8=None, gamma=0.99, scale_value=0.01, shift_value=0.0,
-                            value_bootstrap=True):
+                            value_bootstrap=True, episode_returns=None, episode_lengths=None, episode_partials=None):
         """Arm the reward epilogue of the fused step (SURVEY 8 a16; rl_games ``play_steps``): the NEXT steps also write
         ``shaped_rewards = (rew + shift) * scale + gamma * values * time_outs`` (e.g. ``mb_rewards[t]``) and the uint8 reset
         mask ``dones_u8`` (e.g. the experience buffer's ``dones`` slot ``t + 1``).  ``values``: the (N,)/(N,1) un-normalised
-        critic values of the step (what ``policy_head`` wrote).  Call with no arguments to disarm."""
+        critic values of the step (what ``policy_head`` wrote).
+        ``episode_returns`` / ``episode_lengths`` ((N,) float32) and ``episode_partials`` ((3, ceil(N/32)) float64), all three or
+        none, GPU pipeline only: the step also carries rl_games' ``current_rewards`` / ``current_lengths`` (unshaped reward; zeroed
+        by a multiply when the env is done) and writes its done envs' count / return sum / length sum per group of 32 envs, the
+        input of ``learner.EpisodeMeter``.  Call with no arguments to disarm everything."""
         if self.fusion != "fused":
             raise NotImplementedError("the reward epilogue rides in the fused step (fusion='fused')")
+        n, dev = self.num_envs, self.compute_device
+        eps = (episode_returns, episode_lengths, episode_partials)
+        if any(t is not None for t in eps):
+            if self.host_staged:
+                raise NotImplementedError("episode statistics need the GPU pipeline")
+            if any(t is None for t in eps):
+                raise ValueError("episode_returns, episode_lengths and episode_partials are armed together")
+            for t, dtype, numel, name in zip(eps, (torch.float32, torch.float32, torch.float64), (n, n, 3 * ((n + 31) // 32)),
+                                             ("episode_returns", "episode_lengths", "episode_partials")):
+                if t.dtype != dtype or t.numel() != numel or not t.is_contiguous() or t.device != dev:
+                    raise ValueError(f"{name} must be a contiguous {dtype} tensor with {numel} elements on {dev}")
+            self._episode = eps
+        else:
+            self._episode = None
         if shaped_rewards is None and dones_u8 is None:
             self._rollout = None
             return
-        n, dev = self.num_envs, self.compute_device
 
         def chk(t, dtype, name, host_ok=False):
             if t is None:

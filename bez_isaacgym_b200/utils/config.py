@@ -125,3 +125,14 @@ def agent_config(train_cfg):
     """``params.config`` of a resolved train yaml -> the ``config`` dict of ``learner.A2CAgent``."""
     c = train_cfg["params"]["config"]
     return {k: c[k] for k in AGENT_KEYS if k in c}
+
+
+#: rl_games ``params.config`` keys of the training loop (``A2CBase.train``: meters, checkpoints, stop rules) that
+#: ``learner.A2CAgent.train`` understands
+TRAIN_LOOP_KEYS = ("games_to_track", "save_best_after", "save_frequency", "score_to_win", "max_epochs", "name")
+
+
+def train_loop_config(train_cfg):
+    """``params.config`` of a resolved train yaml -> the training-loop keys of ``learner.A2CAgent``'s ``config``."""
+    c = train_cfg["params"]["config"]
+    return {k: c[k] for k in TRAIN_LOOP_KEYS if k in c}

@@ -367,6 +367,35 @@ int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_bod
                               int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped,
                               float* rew, const BezkRolloutCfg* rollout, const float* values,
                               float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n, void* stream);
+/* bezk_post_physics_rollout with rl_games' episode bookkeeping in the same epilogue (a2c_common.py play_steps:
+ * `current_rewards += rewards; current_lengths += 1; ...; current_rewards = current_rewards * not_dones`, likewise the lengths;
+ * `rewards` is the unshaped rew, `dones` the reset mask this step writes).  ep_return, ep_length, ep_partials: all NULL (then this
+ * is bezk_post_physics_rollout) or all non-NULL, DEVICE memory:
+ *   ep_return, ep_length (n,) f32 in/out: the episode return / length so far; every env adds this step's rew / 1 and writes the
+ *                                         sum back multiplied by (1 - done) -- a NaN return stays NaN, as in rl_games
+ *   ep_partials (3, W) f64 out, W = ceil(n / 32): per group of 32 envs (env / 32) the count of envs done in this step, the sum of
+ *                                         their returns and the sum of their lengths (this step's rew / 1 included).  Every slot is
+ *                                         written each step; the sums have a fixed order (the same bits every run).
+ * Accumulators armed: the one-shot fused kernel runs (BEZK_PERSIST is ignored); obs, rew, reset, progress, time-outs, reset rows,
+ * shaped rewards and dones_u8 are the same bytes as without them. */
+int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states,
+                                 float* net_contact, float* prev_lin_vel, float* goal, const float* goal_angle,
+                                 const float* ball_init, const float* initial_root_states,
+                                 const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step,
+                                 int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                 int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped,
+                                 float* rew, const BezkRolloutCfg* rollout, const float* values,
+                                 float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                 float* ep_return, float* ep_length, double* ep_partials, void* stream);
+/* rl_games' game_rewards / game_lengths meters (torch_ext.AverageMeter(1, games_to_track)) updated from `steps` consecutive
+ * ep_partials of bezk_post_physics_rollout_ep over n envs (partials: (steps, 3, ceil(n / 32)) f64), step by step in order:
+ *   new_mean = sum / count (fp64, rounded to fp32); size = min(count, games_to_track);
+ *   old_size = min(games_to_track - size, current_size); current_size = old_size + size;
+ *   mean = (mean * old_size + new_mean * size) / current_size          (fp32; a step with count 0 changes nothing)
+ * mean2 (2,) f32 and size2 (2,) i64, DEVICE memory, in/out: [returns meter, lengths meter].  No host synchronisation (graph
+ * capturable); steps == 0 or n == 0 is a no-op. */
+int bezk_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
+                              int64_t* size2, void* stream);
 /* bezk_reset_idx for any task: root rows are 13 floats for walk / orient, and their goal (n,2) rows are redrawn.
  * env_base: global id of local env 0 (Philox key = env_base + env id), as in bezk_post_physics_rollout. */
 int bezk_reset_idx_task(int task, const int64_t* env_ids, int64_t k, const float* uniforms, const float* goal_uniforms,
