@@ -62,6 +62,25 @@ static void set_rollout(bezk::TaskArgs& a, const BezkRolloutCfg* rollout, const 
     }
 }
 
+// The step's tensors as one TaskArgs: reset_buf / progress_buf are read and written in place, what an entry does not take is
+// NULL / 0 (fill_alignment derives the defaults)
+static bezk::TaskArgs step_args(float* dof_state, const float* rigid_body, float* root_states, float* net_contact, float* prev_lin_vel,
+                                float* goal, const float* goal_angle, const float* ball_init, const float* initial_root_states,
+                                const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step, int64_t* reset_buf,
+                                int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf, float* obs, float* obs_clipped,
+                                float* rew, int64_t n, int64_t env_base, float* dof_state_wb, float* root_states_wb) {
+    bezk::TaskArgs a;
+    memset(&a, 0, sizeof(a));
+    a.dof_state = dof_state; a.rigid_body = rigid_body; a.root_states = root_states; a.net_contact = net_contact;
+    a.prev_lin_vel = prev_lin_vel; a.goal = goal; a.goal_angle = goal_angle; a.goal_uniforms = goal_uniforms; a.ball_init = ball_init;
+    a.initial_root = initial_root_states; a.uniforms = uniforms; a.seed = seed; a.step = step; a.env_base = env_base;
+    a.dof_state_wb = dof_state_wb; a.root_states_wb = root_states_wb;
+    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
+    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
+    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    return a;
+}
+
 static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK,
                     bezk::EpArgs* ep = nullptr) {
     if (int rc = check_cfg(cfg)) return rc;
@@ -85,34 +104,26 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
     }
     bezk::fill_alignment(a, *cfg);
     bezk::set_l2_policy(task, cfg->flags, a, ep);
-    if (ep) {                              // the one-shot kernel with the episode accumulators (the persistent one has none)
-        ep->w = (a.n + 31) / 32;
-        return cuda_rc(bezk::launch_task_ep(task, a, *cfg, *ep, (cudaStream_t)stream), where);
-    }
-    if (bezk::persist_eligible(task, parts, a, *cfg))          // the persistent pipelined kernel (bezk_task_persist.cu)
-        return cuda_rc(bezk::launch_task_persist(a, *cfg, (cudaStream_t)stream), where);
-    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, (cudaStream_t)stream), where);
+    if (ep) ep->w = (a.n + 31) / 32;
+    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream), where);
 }
 
 int bezk_compute_observations(const float* dof_state, const float* rigid_body, const float* root_states, float* net_contact,
                               float* prev_lin_vel, const float* goal, const float* ball_init, const BezkTaskCfg* cfg,
                               float* obs, float* obs_clipped, int64_t n, void* stream) {
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = const_cast<float*>(dof_state); a.rigid_body = rigid_body; a.root_states = const_cast<float*>(root_states);
-    a.net_contact = net_contact; a.prev_lin_vel = prev_lin_vel; a.goal = const_cast<float*>(goal); a.ball_init = ball_init;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.n = n;
+    bezk::TaskArgs a = step_args(const_cast<float*>(dof_state), rigid_body, const_cast<float*>(root_states), net_contact, prev_lin_vel,
+                                 const_cast<float*>(goal), nullptr, ball_init, nullptr, nullptr, nullptr, 0, 0, nullptr, nullptr, nullptr,
+                                 nullptr, obs, obs_clipped, nullptr, n, 0, nullptr, nullptr);
     return run_task(BEZK_PART_OBS, a, cfg, stream, "bezk_compute_observations");
 }
 
 int bezk_compute_reward(const float* dof_state, const float* rigid_body, const float* root_states, const float* goal,
                         const float* ball_init, const int64_t* reset_in, const int64_t* progress, const BezkTaskCfg* cfg,
                         float* rew, int64_t* reset_out, int64_t n, void* stream) {
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = const_cast<float*>(dof_state); a.rigid_body = rigid_body; a.root_states = const_cast<float*>(root_states);
-    a.goal = const_cast<float*>(goal); a.ball_init = ball_init; a.reset_in = reset_in; a.reset_out = reset_out; a.progress_in = progress;
-    a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(const_cast<float*>(dof_state), rigid_body, const_cast<float*>(root_states), nullptr, nullptr,
+                                 const_cast<float*>(goal), nullptr, ball_init, nullptr, nullptr, nullptr, 0, 0, nullptr, nullptr, nullptr,
+                                 nullptr, nullptr, nullptr, rew, n, 0, nullptr, nullptr);
+    a.reset_in = reset_in; a.reset_out = reset_out; a.progress_in = progress;     // the reset mask goes to its own buffer; progress is only read
     return run_task(BEZK_PART_REWARD, a, cfg, stream, "bezk_compute_reward");
 }
 
@@ -148,14 +159,9 @@ int bezk_post_physics(float* dof_state, const float* rigid_body, float* root_sta
                       int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, int parts,
                       int64_t n, void* stream) {
     REQUIRE(parts >= 1 && parts <= 7, "parts must be a non-empty subset of {1,2,4}");
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = dof_state; a.rigid_body = rigid_body; a.root_states = root_states; a.net_contact = net_contact;
-    a.prev_lin_vel = prev_lin_vel; a.goal = const_cast<float*>(goal); a.ball_init = ball_init; a.initial_root = initial_root_states;
-    a.uniforms = uniforms; a.seed = seed; a.step = step;
-    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
-    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(dof_state, rigid_body, root_states, net_contact, prev_lin_vel, const_cast<float*>(goal), nullptr, ball_init,
+                                 initial_root_states, uniforms, nullptr, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf,
+                                 obs, obs_clipped, rew, n, 0, nullptr, nullptr);
     return run_task(parts, a, cfg, stream, "bezk_post_physics");
 }
 
@@ -166,15 +172,9 @@ int bezk_post_physics_chunk(float* dof_state, const float* rigid_body, float* ro
                             int64_t n, int64_t env_base, float* dof_state_wb, float* root_states_wb, void* stream) {
     REQUIRE(parts >= 1 && parts <= 7, "parts must be a non-empty subset of {1,2,4}");
     REQUIRE(env_base >= 0, "env_base < 0");
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = dof_state; a.rigid_body = rigid_body; a.root_states = root_states; a.net_contact = net_contact;
-    a.prev_lin_vel = prev_lin_vel; a.goal = const_cast<float*>(goal); a.ball_init = ball_init; a.initial_root = initial_root_states;
-    a.uniforms = uniforms; a.seed = seed; a.step = step; a.env_base = env_base; a.dof_state_wb = dof_state_wb;
-    a.root_states_wb = root_states_wb;
-    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
-    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(dof_state, rigid_body, root_states, net_contact, prev_lin_vel, const_cast<float*>(goal), nullptr, ball_init,
+                                 initial_root_states, uniforms, nullptr, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf,
+                                 obs, obs_clipped, rew, n, env_base, dof_state_wb, root_states_wb);
     return run_task(parts, a, cfg, stream, "bezk_post_physics_chunk");
 }
 
@@ -242,16 +242,9 @@ int bezk_post_physics_staged(int task, float* dof_state, const float* imu_stage,
     REQUIRE(!(shaped_rewards || dones_u8) || parts == 7, "the reward epilogue rides in the fused step (parts = 7)");
     REQUIRE(!shaped_rewards || rollout, "shaped_rewards requested without a BezkRolloutCfg");
     REQUIRE(!(shaped_rewards && rollout && rollout->value_bootstrap) || values, "value_bootstrap needs values");
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = dof_state; a.rigid_body = imu_stage; a.root_states = root_states; a.net_contact = feet_stage;
-    a.prev_lin_vel = prev_lin_vel; a.goal = goal; a.goal_angle = goal_angle; a.goal_uniforms = goal_uniforms; a.ball_init = ball_init;
-    a.initial_root = initial_root_states;
-    a.uniforms = uniforms; a.seed = seed; a.step = step; a.env_base = env_base; a.dof_state_wb = dof_state_wb;
-    a.root_states_wb = root_states_wb;
-    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
-    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(dof_state, imu_stage, root_states, feet_stage, prev_lin_vel, goal, goal_angle, ball_init, initial_root_states,
+                                 uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, obs, obs_clipped,
+                                 rew, n, env_base, dof_state_wb, root_states_wb);
     const bool cleats = (cfg->flags & BEZK_F_CLEATS) != 0;
     a.rb_stride = 10; a.rb_off = 0;
     a.cf_stride = cleats ? 24 : 8; a.cf_l_off = 0; a.cf_r_off = cleats ? 12 : 4;
@@ -278,16 +271,9 @@ int bezk_post_physics_packed(int task, float* dof_state, const float* records, f
     const bezk::PackLayout L = bezk::pack_layout(task, *cfg);
     if (int rc = cuda_rc(bezk::launch_unpack_root(task, records, L, root_states, n, (cudaStream_t)stream), "bezk_post_physics_packed (unpack)"))
         return rc;
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = dof_state; a.rigid_body = records; a.root_states = root_states; a.net_contact = const_cast<float*>(records);
-    a.prev_lin_vel = prev_lin_vel; a.goal = goal; a.goal_angle = goal_angle; a.goal_uniforms = goal_uniforms; a.ball_init = ball_init;
-    a.initial_root = initial_root_states;
-    a.uniforms = uniforms; a.seed = seed; a.step = step; a.env_base = env_base; a.dof_state_wb = dof_state_wb;
-    a.root_states_wb = root_states_wb;
-    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
-    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(dof_state, records, root_states, const_cast<float*>(records), prev_lin_vel, goal, goal_angle, ball_init,
+                                 initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf,
+                                 obs, obs_clipped, rew, n, env_base, dof_state_wb, root_states_wb);
     a.rb_stride = L.stride; a.rb_off = 0;
     a.cf_stride = L.stride; a.cf_l_off = L.l_off; a.cf_r_off = L.r_off;
     // values == NULL with value_bootstrap: the critic values ride in the records' last float (bezk_host_pack_begin's values_host)
@@ -304,14 +290,9 @@ int bezk_post_physics_task(int task, float* dof_state, const float* rigid_body, 
                            const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, int parts, int64_t n, void* stream) {
     REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
     REQUIRE(parts >= 1 && parts <= 7, "parts must be a non-empty subset of {1,2,4}");
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = dof_state; a.rigid_body = rigid_body; a.root_states = root_states; a.net_contact = net_contact;
-    a.prev_lin_vel = prev_lin_vel; a.goal = goal; a.goal_angle = goal_angle; a.goal_uniforms = goal_uniforms; a.ball_init = ball_init;
-    a.initial_root = initial_root_states; a.uniforms = uniforms; a.seed = seed; a.step = step;
-    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
-    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init, initial_root_states,
+                                 uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, obs, obs_clipped,
+                                 rew, n, 0, nullptr, nullptr);
     return run_task(parts, a, cfg, stream, "bezk_post_physics_task", task);
 }
 
@@ -330,14 +311,9 @@ int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_
     REQUIRE(armed == 0 || armed == 3, "ep_return, ep_length and ep_partials must be all NULL or all non-NULL");
     if (armed && !(ALIGNED(ep_return, 4) && ALIGNED(ep_length, 4) && ALIGNED(ep_partials, 8)))
         return fail(BEZK_E_ALIGN, "ep_return / ep_length must be 4-byte and ep_partials 8-byte aligned");
-    bezk::TaskArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dof_state = dof_state; a.rigid_body = rigid_body; a.root_states = root_states; a.net_contact = net_contact;
-    a.prev_lin_vel = prev_lin_vel; a.goal = goal; a.goal_angle = goal_angle; a.goal_uniforms = goal_uniforms; a.ball_init = ball_init;
-    a.initial_root = initial_root_states; a.uniforms = uniforms; a.seed = seed; a.step = step; a.env_base = env_base;
-    a.reset_in = reset_buf; a.reset_out = reset_buf; a.progress_in = progress_buf; a.progress_out = progress_buf;
-    a.timeout_buf = timeout_buf; a.randomize_buf = randomize_buf;
-    a.obs = obs; a.obs_clipped = obs_clipped; a.rew = rew; a.n = n;
+    bezk::TaskArgs a = step_args(dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init, initial_root_states,
+                                 uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, obs, obs_clipped,
+                                 rew, n, env_base, nullptr, nullptr);
     set_rollout(a, rollout, values, shaped_rewards, dones_u8);
     bezk::EpArgs ep = {ep_return, ep_length, ep_partials, 0};
     return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream,

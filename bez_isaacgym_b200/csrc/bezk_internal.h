@@ -77,16 +77,14 @@ struct PpoArgs {
     int slabs;
     int use_tma;
 };
-cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st);
-// the whole step (parts = 7) with the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel)
-cudaError_t launch_task_ep(int task, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st);
-// folds `steps` x (3, ceil(n / 32)) partials of launch_task_ep into the two AverageMeters (bezk_rollout.cu)
+// the tile kernel for (task, parts): kick takes parts 1..7, walk / orient 2, 3, 4 or 7; ep (the episode accumulators,
+// task_tile_ep_kernel / task_tile_ep_l2_kernel) only with parts = 7.  cudaErrorInvalidValue for any other combination.
+cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st);
+// folds `steps` x (3, ceil(n / 32)) partials of launch_task's episode accumulators into the two AverageMeters (bezk_rollout.cu)
 cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                                         int64_t* size2, cudaStream_t st);
 cudaError_t launch_goal_uniforms(uint64_t seed, uint64_t step, float* out2, cudaStream_t st);
 void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg);
-bool persist_eligible(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg);
-cudaError_t launch_task_persist(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st);
 cudaError_t stage_feet_gather(const float*, const BezkTaskCfg&, float*, int64_t, int64_t, cudaStream_t);
 cudaError_t stage_imu_rows(const float*, const BezkTaskCfg&, float*, int64_t, int64_t, cudaStream_t);
 cudaError_t stage_sparse_rows(const float*, const float*, const BezkTaskCfg&, float*, float*, int64_t, int64_t, cudaStream_t);

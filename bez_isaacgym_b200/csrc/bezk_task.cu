@@ -23,6 +23,7 @@
 #include <math.h>
 #include <stdlib.h>
 #include <atomic>
+#include <type_traits>
 
 namespace bezk {
 
@@ -561,39 +562,34 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     }
 
     // ---- 8. reward / termination (overlaps the bulk store) ----
-    if (REW && valid && TASK != BEZK_TASK_KICK) {
+    if (REW && valid) {
         float rew;
         int64_t reset;
-        Mth<true> mr;
-        if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr);
-        else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr);
-        if (mr.bad()) {
-            Mth<false> mp;
-            if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp);
-            else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp);
-        }
-        L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
-        L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
-        if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
-        if constexpr (EP) episode_epilogue<L2H>((eps, ...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
-    }
-    if (REW && valid && TASK == BEZK_TASK_KICK) {
-        RewardIn s;
-        s.bez[0] = bez[0]; s.bez[1] = bez[1]; s.bez[2] = bez[2];
-        s.ball_xy[0] = ball_xy[0]; s.ball_xy[1] = ball_xy[1];
-        s.ball_vxy[0] = ball_vxy[0]; s.ball_vxy[1] = ball_vxy[1];
-        s.goal[0] = goal[0]; s.goal[1] = goal[1];
-        s.ball_init[0] = binit[0]; s.ball_init[1] = binit[1];
+        if constexpr (TASK == BEZK_TASK_KICK) {
+            RewardIn s;
+            s.bez[0] = bez[0]; s.bez[1] = bez[1]; s.bez[2] = bez[2];
+            s.ball_xy[0] = ball_xy[0]; s.ball_xy[1] = ball_xy[1];
+            s.ball_vxy[0] = ball_vxy[0]; s.ball_vxy[1] = ball_vxy[1];
+            s.goal[0] = goal[0]; s.goal[1] = goal[1];
+            s.ball_init[0] = binit[0]; s.ball_init[1] = binit[1];
 #pragma unroll
-        for (int k = 0; k < 3; ++k) { s.v[k] = v[k]; s.w[k] = w[k]; }
-        s.pos_sq = pos_sq;
-        float rew;
-        int64_t reset;
-        Mth<true> mr;
-        reward_term(s, cfg, progress, reset_cur, &rew, &reset, mr);
-        if (mr.bad()) {
-            Mth<false> mp;
-            reward_term(s, cfg, progress, reset_cur, &rew, &reset, mp);
+            for (int k = 0; k < 3; ++k) { s.v[k] = v[k]; s.w[k] = w[k]; }
+            s.pos_sq = pos_sq;
+            Mth<true> mr;
+            reward_term(s, cfg, progress, reset_cur, &rew, &reset, mr);
+            if (mr.bad()) {
+                Mth<false> mp;
+                reward_term(s, cfg, progress, reset_cur, &rew, &reset, mp);
+            }
+        } else {
+            Mth<true> mr;
+            if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr);
+            else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr);
+            if (mr.bad()) {
+                Mth<false> mp;
+                if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp);
+                else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp);
+            }
         }
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
         L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
@@ -696,72 +692,65 @@ __global__ void philox_uniforms_kernel(uint64_t seed, uint64_t step, float* out,
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
 
-template <int PARTS, bool CLEATS, int TILE, int TASK>
-static cudaError_t launch_parts3(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st) {
+// Ep: empty (task_tile_kernel / task_tile_l2_kernel) or the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel);
+// a.l2_resident picks the L2 variant
+template <int PARTS, bool CLEATS, int TILE, int TASK, typename... Ep>
+static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st, const Ep&... eps) {
+    static_assert(sizeof...(Ep) == 0 || PARTS == 7, "the episode accumulators ride in the whole step");
+    const auto kernel = [&] {
+        if constexpr (sizeof...(Ep) == 0)
+            return a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
+        else
+            return a.l2_resident ? task_tile_ep_l2_kernel<CLEATS, TILE, TASK> : task_tile_ep_kernel<CLEATS, TILE, TASK>;
+    }();
     const size_t smem = (size_t)(smem_in_floats(TILE, TASK) + (a.obs_clipped ? smem_obs_floats(TILE, TASK) : 0)) * sizeof(float);
     static SmemOptIn opt_in, opt_in_l2;    // per instantiation, per device
-    const auto kernel = a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
     if (cudaError_t err = (a.l2_resident ? opt_in_l2 : opt_in).ensure(kernel, (smem_in_floats(TILE, TASK) + smem_obs_floats(TILE, TASK)) * sizeof(float)))
         return err;
     const int64_t tiles = (a.n + TILE - 1) / TILE;
-    return launch_ex(kernel, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg);
+    return launch_ex(kernel, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg, eps...);
 }
 
-template <bool CLEATS, int TILE, int TASK>
-static cudaError_t launch_ep3(const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st) {
-    const size_t smem = (size_t)(smem_in_floats(TILE, TASK) + (a.obs_clipped ? smem_obs_floats(TILE, TASK) : 0)) * sizeof(float);
-    static SmemOptIn opt_in, opt_in_l2;
-    const auto kernel = a.l2_resident ? task_tile_ep_l2_kernel<CLEATS, TILE, TASK> : task_tile_ep_kernel<CLEATS, TILE, TASK>;
-    if (cudaError_t err = (a.l2_resident ? opt_in_l2 : opt_in).ensure(kernel, (smem_in_floats(TILE, TASK) + smem_obs_floats(TILE, TASK)) * sizeof(float)))
-        return err;
-    const int64_t tiles = (a.n + TILE - 1) / TILE;
-    return launch_ex(kernel, dim3((unsigned)tiles), dim3(TILE), smem, st, a, cfg, ep);
-}
+template <int V>
+using Int = std::integral_constant<int, V>;
 
-template <int TASK>
-static cudaError_t launch_ep(const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st) {
-    return (cfg.flags & BEZK_F_CLEATS) ? launch_ep3<true, BEZK_TILE, TASK>(a, cfg, ep, st) : launch_ep3<false, BEZK_TILE, TASK>(a, cfg, ep, st);
-}
-
-cudaError_t launch_task_ep(int task, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs& ep, cudaStream_t st) {
+cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st) {
+    const bool cleats = (cfg.flags & BEZK_F_CLEATS) != 0;
+    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators only with the whole step
+    const auto tile = [&](auto task_c, auto parts_c) -> cudaError_t {
+        constexpr int TASK = decltype(task_c)::value, PARTS = decltype(parts_c)::value;
+        if constexpr (PARTS == 7) {
+            if (ep) return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep) : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep);
+        }
+        if (ep) return cudaErrorInvalidValue;
+        return cleats ? launch_tile<PARTS, true, BEZK_TILE, TASK>(a, cfg, st) : launch_tile<PARTS, false, BEZK_TILE, TASK>(a, cfg, st);
+    };
+    // walk / orient: the fused step (7), the observation kernel (2 or 3) and the reward kernel (4)
+    const auto sibling = [&](auto task_c) -> cudaError_t {
+        switch (parts) {
+            case 2: return tile(task_c, Int<2>{});
+            case 3: return tile(task_c, Int<3>{});
+            case 4: return tile(task_c, Int<4>{});
+            case 7: return tile(task_c, Int<7>{});
+            default: return cudaErrorInvalidValue;
+        }
+    };
     switch (task) {
-        case BEZK_TASK_KICK: return launch_ep<BEZK_TASK_KICK>(a, cfg, ep, st);
-        case BEZK_TASK_WALK: return launch_ep<BEZK_TASK_WALK>(a, cfg, ep, st);
-        case BEZK_TASK_ORIENT: return launch_ep<BEZK_TASK_ORIENT>(a, cfg, ep, st);
+        case BEZK_TASK_WALK: return sibling(Int<BEZK_TASK_WALK>{});
+        case BEZK_TASK_ORIENT: return sibling(Int<BEZK_TASK_ORIENT>{});
+        case BEZK_TASK_KICK: break;
         default: return cudaErrorInvalidValue;
     }
-}
-
-template <int PARTS, int TASK>
-static cudaError_t launch_parts(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st) {
-    return (cfg.flags & BEZK_F_CLEATS) ? launch_parts3<PARTS, true, BEZK_TILE, TASK>(a, cfg, st)
-                                       : launch_parts3<PARTS, false, BEZK_TILE, TASK>(a, cfg, st);
-}
-
-// walk / orient: the fused step (7), the observation kernel (2 or 3) and the reward kernel (4)
-template <int TASK>
-static cudaError_t launch_sibling(int parts, const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st) {
+    // BezKick: every non-empty subset of the three parts
+    constexpr Int<BEZK_TASK_KICK> kick{};
     switch (parts) {
-        case 2: return launch_parts<2, TASK>(a, cfg, st);
-        case 3: return launch_parts<3, TASK>(a, cfg, st);
-        case 4: return launch_parts<4, TASK>(a, cfg, st);
-        case 7: return launch_parts<7, TASK>(a, cfg, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st) {
-    if (task == BEZK_TASK_WALK) return launch_sibling<BEZK_TASK_WALK>(parts, a, cfg, st);
-    if (task == BEZK_TASK_ORIENT) return launch_sibling<BEZK_TASK_ORIENT>(parts, a, cfg, st);
-    if (task != BEZK_TASK_KICK) return cudaErrorInvalidValue;
-    switch (parts) {
-        case 1: return launch_parts<1, BEZK_TASK_KICK>(a, cfg, st);
-        case 2: return launch_parts<2, BEZK_TASK_KICK>(a, cfg, st);
-        case 3: return launch_parts<3, BEZK_TASK_KICK>(a, cfg, st);
-        case 4: return launch_parts<4, BEZK_TASK_KICK>(a, cfg, st);
-        case 5: return launch_parts<5, BEZK_TASK_KICK>(a, cfg, st);
-        case 6: return launch_parts<6, BEZK_TASK_KICK>(a, cfg, st);
-        case 7: return launch_parts<7, BEZK_TASK_KICK>(a, cfg, st);
+        case 1: return tile(kick, Int<1>{});
+        case 2: return tile(kick, Int<2>{});
+        case 3: return tile(kick, Int<3>{});
+        case 4: return tile(kick, Int<4>{});
+        case 5: return tile(kick, Int<5>{});
+        case 6: return tile(kick, Int<6>{});
+        case 7: return tile(kick, Int<7>{});
         default: return cudaErrorInvalidValue;
     }
 }

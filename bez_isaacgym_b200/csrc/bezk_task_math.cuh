@@ -1,5 +1,5 @@
 // Per-env math of the BezKick / walk / orient task step (device functions; arithmetic order follows the reference op by op).
-// Shared by the one-shot tile kernel (bezk_task.cu) and the persistent pipelined kernel (bezk_task_persist.cu).
+// Used by the tile kernel (bezk_task.cu).
 #pragma once
 #include "bezk_common.cuh"
 #include "bezk_internal.h"

@@ -376,8 +376,8 @@ int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_bod
  *   ep_partials (3, W) f64 out, W = ceil(n / 32): per group of 32 envs (env / 32) the count of envs done in this step, the sum of
  *                                         their returns and the sum of their lengths (this step's rew / 1 included).  Every slot is
  *                                         written each step; the sums have a fixed order (the same bits every run).
- * Accumulators armed: the one-shot fused kernel runs (BEZK_PERSIST is ignored); obs, rew, reset, progress, time-outs, reset rows,
- * shaped rewards and dones_u8 are the same bytes as without them. */
+ * Accumulators armed: obs, rew, reset, progress, time-outs, reset rows, shaped rewards and dones_u8 are the same bytes as without
+ * them. */
 int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states,
                                  float* net_contact, float* prev_lin_vel, float* goal, const float* goal_angle,
                                  const float* ball_init, const float* initial_root_states,

@@ -93,15 +93,6 @@ def test_fused_kernel_fits_five_ctas_worth_of_registers(sass):
     assert int(m.group(1)) <= 104, m.group(1)
 
 
-def test_persistent_variant_gathers_with_cp_async_and_tma(sass):
-    """The opt-in persistent variant (bezk_task_persist.cu): bulk copies for the dense sub-tiles, LDGSTS (cp.async, L1 bypassed)
-    for the sparse rows, mbarrier waits, one bulk store per tile."""
-    body = sass[_find(sass, "task_persist_kernel")[0]]
-    assert "UBLKCP.S.G" in body and "UBLKCP.G.S" in body and "SYNCS" in body
-    assert "LDGSTS" in body, "sparse rows arrive by cp.async"
-    assert "BAR.SYNC" not in body
-
-
 def test_cooperative_statistics_kernel_has_a_grid_barrier(sass):
     body = sass[_find(sass, "fused_stats_kernelILi1E")[0]]
     assert "STL" not in body and "LDL" not in body

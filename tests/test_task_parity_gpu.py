@@ -533,48 +533,6 @@ def test_branch_free_division_and_sqrt_are_ieee_exact():
     assert sq_ok == 120 * (1 << 23) + 1 + 2 and div_ok > (1 << 27)
 
 
-def test_persistent_kernel_variant_is_bit_identical():
-    """``BEZK_PERSIST=1`` selects the persistent software-pipelined variant of the fused step (csrc/bezk_task_persist.cu; opt-in,
-    read once per process -> a subprocess): same device functions in the same order, so every output equals the one-shot
-    kernel's bit for bit, resets and reward epilogue included."""
-    import os
-    import subprocess
-    import sys
-    code = r'''
-import sys, torch
-sys.path.insert(0, %r)
-from bez_isaacgym_b200 import ops, synthetic_gym as sg
-n = int(sys.argv[1])
-st = sg.make_state(n, seed=5).to("cuda")
-cfg = ops.make_task_cfg()
-goal, ball_init, *_ = sg.make_constants(n, "cuda")
-init_root = sg.make_initial_root_states(n, "cuda")
-progress, reset = sg.make_bookkeeping(n, seed=6, device="cuda", p_reset=0.1)
-progress[:4] = torch.tensor([899, 900, 897, 898], device="cuda")
-timeout = torch.empty(n, dtype=torch.long, device="cuda"); obs = torch.empty(n, 54, device="cuda"); rew = torch.empty(n, device="cuda")
-prev = torch.zeros(n, 3, device="cuda"); values = torch.randn(n, generator=torch.Generator().manual_seed(1)).cuda()
-shaped = torch.empty(n, device="cuda"); dones = torch.empty(n, dtype=torch.uint8, device="cuda")
-for step in range(3):
-    ops.post_physics_rollout("kick", st.dof_state, st.rigid_body, st.root_states, st.net_contact, goal, init_root, reset, progress, timeout,
-                             cfg, obs, rew, rollout_cfg=ops.make_rollout_cfg(), values=values, shaped_rewards=shaped, dones_u8=dones,
-                             ball_init=ball_init, prev_lin_vel=prev, seed=3, step=step)
-torch.cuda.synchronize()
-torch.save([t.cpu() for t in (obs, rew, reset, progress, timeout, shaped, dones, prev, st.dof_state, st.root_states, st.net_contact)], sys.argv[2])
-''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    import tempfile
-    with tempfile.TemporaryDirectory() as tmp:
-        for n in (4096, 65536 + 32):
-            outs = []
-            for mode in ("0", "1"):
-                path = os.path.join(tmp, f"o{mode}.pt")
-                env = dict(os.environ, BEZK_PERSIST=mode)
-                subprocess.run([sys.executable, "-c", code, str(n), path], check=True, env=env, timeout=300)
-                outs.append(torch.load(path))
-            for a, b in zip(*outs):
-                assert torch.equal(a, b) or bool(((a == b) | (a.isnan() & b.isnan())).all())
-            assert int(outs[0][2].sum()) > 0
-
-
 def test_default_host_pipeline_resolves_to_a_mode_that_serves_the_configuration():
     """``env.hostPipeline`` defaults to ``auto``: ``zero_copy`` for small tasks (two launches, nothing staged) and when the caller
     asks for what only that mode does (the two-kernel split, the in-place contact filter); a staged pipeline for the fused step of

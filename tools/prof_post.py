@@ -1,6 +1,5 @@
 #!/usr/bin/env python
-"""ncu target: a few fused post-physics launches at --envs through KickEnv (no graph), nothing else.
-    BEZK_PERSIST=1|0 selects the persistent / one-shot kernel (read once per process)."""
+"""ncu target: a few fused post-physics launches at --envs through KickEnv (no graph), nothing else."""
 import argparse
 import os
 import sys
