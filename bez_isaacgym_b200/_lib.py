@@ -107,6 +107,10 @@ SIGNATURES = {
                                                C.POINTER(BezkTaskCfg), _P, _P, _P, C.POINTER(BezkRolloutCfg), _P, _P, _P, _I64, _I64,
                                                _P, _P, _P, _P]),
     "bezk_episode_meter_update": (C.c_int, [_P, C.c_int, _I64, _I64, _P, _P, _P]),
+    "bezk_post_physics_rollout_ep_norm": (C.c_int, [C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _U64, _U64, _P, _P, _P, _P,
+                                                    C.POINTER(BezkTaskCfg), _P, _P, _P, C.POINTER(BezkRolloutCfg), _P, _P, _P, _I64,
+                                                    _I64, _P, _P, _P, _P, _P, C.c_float, _P, _P]),
+    "bezk_player_tally_update": (C.c_int, [_P, C.c_int, _I64, _I64, _P, _P, _P]),
     "bezk_reset_idx_task": (C.c_int, [C.c_int, _P, _I64, _P, _P, _U64, _U64, _P, _P, _P, _P, _P, _P, C.POINTER(BezkTaskCfg), _I64, _I64,
                                       _P]),
     "bezk_goal_uniforms": (C.c_int, [_U64, _U64, _P, _P]),

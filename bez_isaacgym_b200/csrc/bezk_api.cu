@@ -82,7 +82,7 @@ static bezk::TaskArgs step_args(float* dof_state, const float* rigid_body, float
 }
 
 static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK,
-                    bezk::EpArgs* ep = nullptr) {
+                    bezk::EpArgs* ep = nullptr, const bezk::NormArgs* nm = nullptr) {
     if (int rc = check_cfg(cfg)) return rc;
     REQUIRE(a.n >= 0, "n < 0");
     if (a.n == 0) return 0;
@@ -105,7 +105,7 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
     bezk::fill_alignment(a, *cfg);
     bezk::set_l2_policy(task, cfg->flags, a, ep);
     if (ep) ep->w = (a.n + 31) / 32;
-    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream), where);
+    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm), where);
 }
 
 int bezk_compute_observations(const float* dof_state, const float* rigid_body, const float* root_states, float* net_contact,
@@ -296,13 +296,14 @@ int bezk_post_physics_task(int task, float* dof_state, const float* rigid_body, 
     return run_task(parts, a, cfg, stream, "bezk_post_physics_task", task);
 }
 
-int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
-                                 float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
-                                 const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
-                                 uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf,
-                                 const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, const BezkRolloutCfg* rollout,
-                                 const float* values, float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
-                                 float* ep_return, float* ep_length, double* ep_partials, void* stream) {
+int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                      float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                      const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
+                                      uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                      int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew,
+                                      const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards, uint8_t* dones_u8,
+                                      int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
+                                      const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, void* stream) {
     REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
     REQUIRE(env_base >= 0, "env_base < 0");
     REQUIRE(!shaped_rewards || rollout, "shaped_rewards requested without a BezkRolloutCfg");
@@ -311,13 +312,37 @@ int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_
     REQUIRE(armed == 0 || armed == 3, "ep_return, ep_length and ep_partials must be all NULL or all non-NULL");
     if (armed && !(ALIGNED(ep_return, 4) && ALIGNED(ep_length, 4) && ALIGNED(ep_partials, 8)))
         return fail(BEZK_E_ALIGN, "ep_return / ep_length must be 4-byte and ep_partials 8-byte aligned");
+    const int norm = (obs_mean != nullptr) + (obs_var != nullptr) + (obs_norm != nullptr);
+    REQUIRE(norm == 0 || norm == 3, "obs_mean, obs_var and obs_norm must be all NULL or all non-NULL");
+    if (norm) {
+        REQUIRE(armed == 3, "obs_norm needs the episode accumulators: ep_return, ep_length and ep_partials are NULL");
+        REQUIRE(obs_eps >= 0.0f, "obs_eps must be >= 0");
+        if (!ALIGNED(obs_norm, 16)) return fail(BEZK_E_ALIGN, "obs_norm must be 16-byte aligned");
+        if (!(ALIGNED(obs_mean, 8) && ALIGNED(obs_var, 8))) return fail(BEZK_E_ALIGN, "obs_mean / obs_var must be 8-byte aligned");
+    }
     bezk::TaskArgs a = step_args(dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init, initial_root_states,
                                  uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, obs, obs_clipped,
                                  rew, n, env_base, nullptr, nullptr);
     set_rollout(a, rollout, values, shaped_rewards, dones_u8);
     bezk::EpArgs ep = {ep_return, ep_length, ep_partials, 0};
+    const bezk::NormArgs nm = {obs_mean, obs_var, obs_norm, obs_eps};
     return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream,
-                    armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout", task, armed ? &ep : nullptr);
+                    norm ? "bezk_post_physics_rollout_ep_norm" : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout"),
+                    task, armed ? &ep : nullptr, norm ? &nm : nullptr);
+}
+
+int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                 float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                 const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
+                                 uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf,
+                                 const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew, const BezkRolloutCfg* rollout,
+                                 const float* values, float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                 float* ep_return, float* ep_length, double* ep_partials, void* stream) {
+    return bezk_post_physics_rollout_ep_norm(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle,
+                                             ball_init, initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf,
+                                             timeout_buf, randomize_buf, cfg, obs, obs_clipped, rew, rollout, values, shaped_rewards,
+                                             dones_u8, env_base, n, ep_return, ep_length, ep_partials, nullptr, nullptr, 0.0f, nullptr,
+                                             stream);
 }
 
 int bezk_post_physics_rollout(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -343,6 +368,18 @@ int bezk_episode_meter_update(const double* partials, int steps, int64_t n, int6
         return fail(BEZK_E_ALIGN, "partials / size2 must be 8-byte and mean2 4-byte aligned");
     return cuda_rc(bezk::launch_episode_meter_update(partials, steps, n, games_to_track, mean2, size2, (cudaStream_t)stream),
                    "bezk_episode_meter_update");
+}
+
+int bezk_player_tally_update(const double* partials, int steps, int64_t n, int64_t games_num, double* tally, double* per_step,
+                             void* stream) {
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    REQUIRE(games_num > 0, "games_num must be positive");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(partials && tally, "partials / tally NULL");
+    if (!ALIGNED(partials, 8) || !ALIGNED(tally, 8) || !ALIGNED(per_step, 8))
+        return fail(BEZK_E_ALIGN, "partials / tally / per_step must be 8-byte aligned");
+    return cuda_rc(bezk::launch_player_tally_update(partials, steps, n, games_num, tally, per_step, (cudaStream_t)stream),
+                   "bezk_player_tally_update");
 }
 
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream) {

@@ -61,6 +61,15 @@ struct EpArgs {
     double* partials;            // (3, W), W = ceil(n / 32): per warp of 32 envs [count of done envs, sum of their return, sum of their length]
     int64_t w;                   // W
 };
+// Eval-mode observation normaliser of the fused step (bezk_post_physics_rollout_ep_norm; rl_games RunningMeanStd.forward with
+// frozen statistics, what PpoPlayerContinuous feeds the policy).  A separate kernel parameter of task_tile_obsnorm_kernel /
+// task_tile_obsnorm_l2_kernel, for the reason EpArgs is one.
+struct NormArgs {
+    const double* mean;          // (obs_row,) running_mean, read every launch
+    const double* var;           // (obs_row,) running_var
+    float* out;                  // (n, obs_row) clamp((x - mean) / sqrt(var + eps), -5, 5), x = the row step() returns
+    float eps;
+};
 // fills l2_resident (bezk_task.cu): after fill_alignment, before the launch; ep: the armed episode accumulators or nullptr
 void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a, const EpArgs* ep = nullptr);
 // demote [ptr, ptr + bytes) to the normal L2 eviction priority (the 128-byte lines entirely inside the range)
@@ -78,11 +87,17 @@ struct PpoArgs {
     int use_tma;
 };
 // the tile kernel for (task, parts): kick takes parts 1..7, walk / orient 2, 3, 4 or 7; ep (the episode accumulators,
-// task_tile_ep_kernel / task_tile_ep_l2_kernel) only with parts = 7.  cudaErrorInvalidValue for any other combination.
-cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st);
+// task_tile_ep_kernel / task_tile_ep_l2_kernel) only with parts = 7; nm (the observation normaliser, task_tile_obsnorm_kernel /
+// task_tile_obsnorm_l2_kernel) only together with ep.  cudaErrorInvalidValue for any other combination.
+cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
+                        const NormArgs* nm = nullptr);
 // folds `steps` x (3, ceil(n / 32)) partials of launch_task's episode accumulators into the two AverageMeters (bezk_rollout.cu)
 cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                                         int64_t* size2, cudaStream_t st);
+// folds the same partials into rl_games BasePlayer.run's game tally [games_played, sum_rewards, sum_steps, steps_folded]
+// up to games_num games (bezk_rollout.cu)
+cudaError_t launch_player_tally_update(const double* partials, int steps, int64_t n, int64_t games_num, double* tally,
+                                       double* per_step, cudaStream_t st);
 cudaError_t launch_goal_uniforms(uint64_t seed, uint64_t step, float* out2, cudaStream_t st);
 void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg);
 cudaError_t stage_feet_gather(const float*, const BezkTaskCfg&, float*, int64_t, int64_t, cudaStream_t);

@@ -627,4 +627,92 @@ cudaError_t launch_episode_meter_update(const double* partials, int steps, int64
     return e != cudaSuccess ? e : f;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Player tally: rl_games BasePlayer.run's per-step bookkeeping (RECALLED, v1.1.x)
+//   games_played += done_count; sum_rewards += cr[done].sum(); sum_steps += steps[done].sum(); stop once games_played >= games_num
+// fed by the same per-step partials.  One warp per step sums the step's 3 x W slots in a fixed order: lane l adds slots
+// l, l + 32, ... in order, then a shuffle-down tree (16, 8, 4, 2, 1) -- tests/rl_games_player_oracle.py restates it.  The last
+// warp to finish (ticket) goes through the steps in order: a step that starts with games_played >= games_num adds nothing (and
+// neither does any step of a later call, since the tally carries games_played), so the result does not depend on how the steps
+// are chunked; the step that reaches the cutoff is added whole, as in rl_games.
+//   tally (4,) f64 in/out: [games_played, sum_rewards, sum_steps, steps_folded];  per_step (steps, 3) f64 out (optional): each
+//   folded step's [count, return sum, length sum], zeros after the cutoff.
+// No barrier, no local memory, scratch from stream-ordered allocation: capturable in a CUDA graph.
+// ------------------------------------------------------------------------------------------------
+constexpr int PT_THREADS = 256;
+constexpr int PT_WARPS = PT_THREADS / 32;
+
+__global__ void __launch_bounds__(PT_THREADS) player_tally_kernel(const double* __restrict__ partials, int steps, int64_t w,
+                                                                   double games_num, double* step_sums, unsigned* ticket, double* tally,
+                                                                   double* per_step) {
+    const int lane = threadIdx.x & 31;
+    const int step = blockIdx.x * PT_WARPS + (threadIdx.x >> 5);
+    const unsigned full = 0xffffffffu;
+    pdl_launch_dependents();
+    pdl_wait();
+    if (step >= steps) return;                  // warp-uniform
+    const double* p = partials + (int64_t)step * 3 * w;
+    double acc[3] = {0.0, 0.0, 0.0};
+    for (int64_t i = lane; i < w; i += 32) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) acc[k] += p[k * w + i];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) acc[k] += __shfl_down_sync(full, acc[k], o);
+    }
+    int last = 0;
+    if (lane == 0) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) step_sums[(int64_t)step * 3 + k] = acc[k];
+        __threadfence();
+        last = atomicAdd(ticket, 1u) == (unsigned)steps - 1;
+    }
+    if (!__shfl_sync(full, last, 0)) return;
+    // the last step to finish: the fold, step by step in order.  Lane j loads step t0 + j's sums; every lane runs the same
+    // recurrence on the shuffled values and lane j writes step t0 + j's per_step row.
+    __threadfence();
+    double games = __ldcg(tally), sr = __ldcg(tally + 1), sl = __ldcg(tally + 2), folded = __ldcg(tally + 3);
+    for (int t0 = 0; t0 < steps; t0 += 32) {
+        double c = 0.0, r = 0.0, l = 0.0;
+        if (t0 + lane < steps) {
+            c = __ldcg(step_sums + 3 * (t0 + lane));
+            r = __ldcg(step_sums + 3 * (t0 + lane) + 1);
+            l = __ldcg(step_sums + 3 * (t0 + lane) + 2);
+        }
+        bool mine = false;                      // this lane's step was folded
+        const int m = steps - t0 < 32 ? steps - t0 : 32;
+        for (int j = 0; j < m; ++j) {
+            const double cj = __shfl_sync(full, c, j), rj = __shfl_sync(full, r, j), lj = __shfl_sync(full, l, j);
+            if (games >= games_num) continue;   // the cutoff was reached by an earlier step
+            folded += 1.0;
+            if (lane == j) mine = true;
+            if (cj > 0.0) { games += cj; sr += rj; sl += lj; }
+        }
+        if (per_step && t0 + lane < steps) {
+            double* q = per_step + 3 * (int64_t)(t0 + lane);
+            q[0] = mine ? c : 0.0; q[1] = mine ? r : 0.0; q[2] = mine ? l : 0.0;
+        }
+    }
+    if (lane == 0) { tally[0] = games; tally[1] = sr; tally[2] = sl; tally[3] = folded; }
+}
+
+cudaError_t launch_player_tally_update(const double* partials, int steps, int64_t n, int64_t games_num, double* tally,
+                                       double* per_step, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    const size_t bytes = (size_t)steps * 3 * sizeof(double) + sizeof(unsigned);
+    void* buf = nullptr;
+    cudaError_t e = cudaMallocAsync(&buf, bytes, st);
+    if (e != cudaSuccess) return e;
+    double* step_sums = static_cast<double*>(buf);
+    unsigned* ticket = reinterpret_cast<unsigned*>(step_sums + (size_t)steps * 3);
+    e = cudaMemsetAsync(ticket, 0, sizeof(unsigned), st);
+    if (e == cudaSuccess)
+        e = launch_ex(player_tally_kernel, dim3((unsigned)((steps + PT_WARPS - 1) / PT_WARPS)), dim3(PT_THREADS), 0, st, partials, steps,
+                      (n + 31) / 32, (double)games_num, step_sums, ticket, tally, per_step);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
 }  // namespace bezk

@@ -263,12 +263,18 @@ __device__ __forceinline__ void episode_epilogue(const EpArgs& ep, int64_t e, fl
     done = reset != 0;
 }
 
+__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep) { return ep; }
+__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const NormArgs&) { return ep; }
+__device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs& nm) { return nm; }
+
 // Ep: empty, or one EpArgs -- then EP is on and the episode accumulators ride along (task_tile_ep_kernel / task_tile_ep_l2_kernel;
-// whole step only).  A parameter pack rather than an always-present argument: the kernels without accumulators make exactly the
-// call they made before the accumulators existed (an unused EpArgs argument alone changes their register allocation).
+// whole step only) -- or EpArgs and NormArgs: the eval-mode observation normaliser too (task_tile_obsnorm_kernel /
+// task_tile_obsnorm_l2_kernel).  A parameter pack rather than always-present arguments: the kernels without accumulators make
+// exactly the call they made before the accumulators existed (an unused EpArgs argument alone changes their register allocation).
 template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H, typename... Ep>
 __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& cfg, const Ep&... eps) {
-    constexpr bool EP = sizeof...(Ep) == 1;
+    constexpr bool EP = sizeof...(Ep) >= 1;
+    constexpr bool NORM = sizeof...(Ep) == 2;
     static_assert(!EP || PARTS == 7, "the episode accumulators ride in the whole step");
     constexpr int ROOT_ROW = root_row(TASK);
     constexpr int OBS_ROW = obs_row(TASK);
@@ -318,7 +324,7 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     gather_env<OBS, (BOOK || REW), CLEATS, TASK, L2H>(a, cfg, e, valid, rb, cf_l, cf_r, g);
     float ep_ret = 0.0f, ep_len = 0.0f;    // carried like the bookkeeping: the same addresses every step
     if constexpr (EP) {
-        const EpArgs& ep = (eps, ...);
+        const EpArgs& ep = ep_of(eps...);
         if (valid) {
             const uint64_t pk = L2H ? policy_evict_last() : 0;
             ep_ret = L2HINT(ld_f32, pk, ep.ret + e);
@@ -594,14 +600,14 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
         L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
         if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
-        if constexpr (EP) episode_epilogue<L2H>((eps, ...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
+        if constexpr (EP) episode_epilogue<L2H>(ep_of(eps...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
     }
 
     // ---- 9. this warp's slot of the per-step episode statistics: [count of done envs, sum of their returns, sum of their
     // lengths] at (k, env / 32).  Fixed-order shuffle tree, one store per value, every step (zeros included): nothing needs
     // zeroing, no atomics, and the sums are the same bits from run to run ----
     if constexpr (EP) if (nv > 0) {
-        const EpArgs& ep = (eps, ...);
+        const EpArgs& ep = ep_of(eps...);
         const unsigned done_mask = __ballot_sync(0xffffffffu, ep_done);
         double sr = ep_done ? (double)ep_r : 0.0, sl = ep_done ? (double)ep_l : 0.0;
 #pragma unroll
@@ -617,6 +623,66 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
         }
     }
 
+    if constexpr (NORM) {
+        // ---- 10. rl_games RunningMeanStd.forward in eval mode on the row step() returns (the clipped one when a.obs_clipped),
+        // with rms_normalize_kernel's arithmetic: mean.float(), sqrtf(var.float() + eps), IEEE division (Mth fast sequence,
+        // plain operator for a chunk with an operand outside its range), clamp to +-5 with NaN propagating.  Lane j holds the
+        // statistics of columns j and 32 + j, read from the device every launch.  The tile is normalised in place once the
+        // stores above have read it, then leaves as one more bulk store (normal L2 priority: not part of the carried set) ----
+        const NormArgs& nm = norm_of(eps...);
+        if (nv == 0) return;                             // warp-uniform: a warp past the last env
+        const float m_lo = (float)nm.mean[lane], d_lo = sqrtf((float)nm.var[lane] + nm.eps);
+        float m_hi = 0.0f, d_hi = 1.0f;
+        if (32 + lane < OBS_ROW) { m_hi = (float)nm.mean[32 + lane]; d_hi = sqrtf((float)nm.var[32 + lane] + nm.eps); }
+        if (full && lane == 0) bulk_wait_read0();       // the obs (and clipped) stores have read the tile
+        __syncwarp();
+        float* x = a.obs_clipped ? s_obs_clip : s_obs;
+        float2* r2 = reinterpret_cast<float2*>(x + lane * OBS_ROW);
+        // every lane runs the loop (the statistics are shuffled across the warp); a tail warp's lanes >= nv work on rows that
+        // are never stored
+        constexpr int NF2 = OBS_ROW / 2, CH = 9;         // float2 per row, float2 per chunk
+#pragma unroll
+        for (int k0 = 0; k0 < NF2; k0 += CH) {
+            float in[2 * CH], mean[2 * CH], den[2 * CH], out[2 * CH];
+            Mth<true> mq;
+#pragma unroll
+            for (int k = 0; k < CH; ++k) {
+                if (k0 + k >= NF2) break;
+                const float2 t = r2[k0 + k];
+                in[2 * k] = t.x; in[2 * k + 1] = t.y;
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int c = 2 * (k0 + k) + h;
+                    mean[2 * k + h] = __shfl_sync(0xffffffffu, c < 32 ? m_lo : m_hi, c & 31);
+                    den[2 * k + h] = __shfl_sync(0xffffffffu, c < 32 ? d_lo : d_hi, c & 31);
+                    out[2 * k + h] = clamp_nan(mq.div(in[2 * k + h] - mean[2 * k + h], den[2 * k + h]), -5.0f, 5.0f);
+                }
+            }
+            if (mq.bad()) {
+#pragma unroll
+                for (int j = 0; j < 2 * CH; ++j)
+                    if (2 * k0 + j < OBS_ROW) out[j] = clamp_nan((in[j] - mean[j]) / den[j], -5.0f, 5.0f);
+            }
+#pragma unroll
+            for (int k = 0; k < CH; ++k) {
+                if (k0 + k >= NF2) break;
+                r2[k0 + k] = make_float2(out[2 * k], out[2 * k + 1]);
+            }
+        }
+        if (full) {
+            fence_proxy_async_smem();
+            __syncwarp();
+            if (lane == 0) {
+                bulk_s2g(nm.out + e0 * OBS_ROW, x, WT * OBS_ROW * 4);
+                bulk_commit();
+                bulk_wait_read0();
+            }
+        } else {
+            __syncwarp();
+            for (int i = lane; i < nv * OBS_ROW; i += WT) nm.out[e0 * OBS_ROW + i] = x[i];
+        }
+        return;
+    }
     if (OBS && full && lane == 0) bulk_wait_read0();   // shared memory must outlive the bulk store's reads
 }
 
@@ -639,6 +705,19 @@ template <bool CLEATS, int TILE, int TASK>
 __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_ep_l2_kernel(const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg,
                                                                                             const EpArgs ep) {
     task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep);
+}
+// the whole step with the episode accumulators and the eval-mode observation normaliser (bezk_post_physics_rollout_ep_norm)
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_obsnorm_kernel(const TaskArgs a,
+                                                                                              const __grid_constant__ BezkTaskCfg cfg,
+                                                                                              const EpArgs ep, const NormArgs nm) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, ep, nm);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_obsnorm_l2_kernel(const TaskArgs a,
+                                                                                                 const __grid_constant__ BezkTaskCfg cfg,
+                                                                                                 const EpArgs ep, const NormArgs nm) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, nm);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -692,16 +771,19 @@ __global__ void philox_uniforms_kernel(uint64_t seed, uint64_t step, float* out,
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
 
-// Ep: empty (task_tile_kernel / task_tile_l2_kernel) or the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel);
-// a.l2_resident picks the L2 variant
+// Ep: empty (task_tile_kernel / task_tile_l2_kernel), the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel) or
+// those and the observation normaliser (task_tile_obsnorm_kernel / task_tile_obsnorm_l2_kernel); a.l2_resident picks the L2
+// variant.  Every variant has the same shared memory: the normaliser works in the observation tile.
 template <int PARTS, bool CLEATS, int TILE, int TASK, typename... Ep>
 static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st, const Ep&... eps) {
     static_assert(sizeof...(Ep) == 0 || PARTS == 7, "the episode accumulators ride in the whole step");
     const auto kernel = [&] {
         if constexpr (sizeof...(Ep) == 0)
             return a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
-        else
+        else if constexpr (sizeof...(Ep) == 1)
             return a.l2_resident ? task_tile_ep_l2_kernel<CLEATS, TILE, TASK> : task_tile_ep_kernel<CLEATS, TILE, TASK>;
+        else
+            return a.l2_resident ? task_tile_obsnorm_l2_kernel<CLEATS, TILE, TASK> : task_tile_obsnorm_kernel<CLEATS, TILE, TASK>;
     }();
     const size_t smem = (size_t)(smem_in_floats(TILE, TASK) + (a.obs_clipped ? smem_obs_floats(TILE, TASK) : 0)) * sizeof(float);
     static SmemOptIn opt_in, opt_in_l2;    // per instantiation, per device
@@ -714,12 +796,17 @@ static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaSt
 template <int V>
 using Int = std::integral_constant<int, V>;
 
-cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st) {
+cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
+                        const NormArgs* nm) {
     const bool cleats = (cfg.flags & BEZK_F_CLEATS) != 0;
-    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators only with the whole step
+    if (nm && !ep) return cudaErrorInvalidValue;
+    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators (and the normaliser) only with the whole step
     const auto tile = [&](auto task_c, auto parts_c) -> cudaError_t {
         constexpr int TASK = decltype(task_c)::value, PARTS = decltype(parts_c)::value;
         if constexpr (PARTS == 7) {
+            if (nm)
+                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm)
+                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm);
             if (ep) return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep) : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep);
         }
         if (ep) return cudaErrorInvalidValue;

@@ -259,6 +259,54 @@ def episode_meter_update(partials, n, games_to_track, mean2, size2, steps=None):
                "bezk_episode_meter_update")
 
 
+def post_physics_rollout_ep_norm(task, dof_state, rigid_body, root_states, net_contact, goal, initial_root_states, reset_buf,
+                                 progress_buf, timeout_buf, cfg, obs, rew, episode_returns, episode_lengths, episode_partials,
+                                 obs_mean, obs_var, obs_norm, obs_eps=1e-5, rollout_cfg=None, values=None, shaped_rewards=None,
+                                 dones_u8=None, goal_angle=None, ball_init=None, prev_lin_vel=None, uniforms=None, goal_uniforms=None,
+                                 seed=0, step=0, randomize_buf=None, obs_clipped=None, env_base=0):
+    """``post_physics_rollout_ep`` that also writes ``obs_norm`` ((N, obs width) float32, CUDA): the row the step returns through
+    ``RunningMeanStd.forward`` in eval mode with ``obs_mean`` / ``obs_var`` ((obs width,) float64, CUDA) and ``obs_eps``
+    (``bezk_post_physics_rollout_ep_norm``)."""
+    n = progress_buf.shape[0]
+    nb = cfg.num_bodies
+    actors, _, width = bm.task_dims(task)
+    ret = _cuda(episode_returns, F32, "episode_returns", n)
+    length = _cuda(episode_lengths, F32, "episode_lengths", n)
+    part = _cuda(episode_partials, F64, "episode_partials", 3 * ((n + 31) // 32))
+    mean, var = _cuda(obs_mean, F64, "obs_mean", width), _cuda(obs_var, F64, "obs_var", width)
+    norm = _cuda(obs_norm, F32, "obs_norm", n * width)
+    lib = _lib.load()
+    _lib.check(lib.bezk_post_physics_rollout_ep_norm(
+        _TASK_ID[task], _p(dof_state, F32, "dof_state", n * 36), _p(rigid_body, F32, "rigid_body", n * nb * 13),
+        _p(root_states, F32, "root_states", n * actors * 13), _p(net_contact, F32, "net_contact", n * nb * 3),
+        _p(prev_lin_vel, F32, "prev_lin_vel", n * 3, True), _p(goal, F32, "goal", n * 2),
+        _p(goal_angle, F32, "goal_angle", n, True), _p(ball_init, F32, "ball_init", n * 2, True),
+        _p(initial_root_states, F32, "initial_root_states", n * actors * 13, True),
+        _p(uniforms, F32, "uniforms", n * 36, True), _p(goal_uniforms, F32, "goal_uniforms", 2, True), seed, step,
+        _p(reset_buf, I64, "reset_buf", n), _p(progress_buf, I64, "progress_buf", n),
+        _p(timeout_buf, I64, "timeout_buf", n), _p(randomize_buf, I64, "randomize_buf", n, True), C.byref(cfg),
+        _p(obs, F32, "obs", n * width), _p(obs_clipped, F32, "obs_clipped", n * width, True), _p(rew, F32, "rew", n),
+        C.byref(rollout_cfg) if rollout_cfg is not None else None, _p(values, F32, "values", n, True),
+        _p(shaped_rewards, F32, "shaped_rewards", n, True), _p(dones_u8, U8, "dones_u8", n, True), int(env_base), n,
+        ret, length, part, mean, var, float(obs_eps), norm, _stream(dof_state)), "bezk_post_physics_rollout_ep_norm")
+
+
+def player_tally_update(partials, n, games_num, tally, per_step=None, steps=None):
+    """Fold ``steps`` consecutive (3, ceil(n/32)) float64 partials of ``post_physics_rollout_ep`` (``partials``: (steps, 3, W) or
+    (3, W)) into rl_games ``BasePlayer.run``'s game tally ``tally`` ((4,) float64: games_played, sum_rewards, sum_steps,
+    steps_folded) up to ``games_num`` games; ``per_step`` ((steps, 3) float64, optional) gets each folded step's sums, on the device
+    (``bezk_player_tally_update``)."""
+    w = (int(n) + 31) // 32
+    if steps is None:
+        steps = partials.numel() // (3 * w) if w else 0
+    if not isinstance(partials, torch.Tensor) or partials.numel() != int(steps) * 3 * w:
+        raise BezkError(f"partials must hold steps x 3 x {w} float64 values")
+    ps = None if per_step is None else _cuda(per_step, F64, "per_step", int(steps) * 3)
+    lib = _lib.load()
+    _lib.check(lib.bezk_player_tally_update(_cuda(partials, F64, "partials", None), int(steps), int(n), int(games_num),
+                                            _cuda(tally, F64, "tally", 4), ps, _stream(partials)), "bezk_player_tally_update")
+
+
 def reset_idx_task(task, env_ids, dof_state, root_states, initial_root_states, goal, progress, reset, cfg, uniforms=None,
                    goal_uniforms=None, seed=0, step=0, env_base=0):
     k = int(env_ids.numel())

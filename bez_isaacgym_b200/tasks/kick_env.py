@@ -211,6 +211,7 @@ class KickEnv(VecTask):
         self._ce_copy_out = False
         self._rollout = None                # (BezkRolloutCfg, values, shaped_rewards, dones_u8) set by set_rollout_targets
         self._episode = None                # (episode_returns, episode_lengths, episode_partials) set by set_rollout_targets
+        self._obs_norm = None               # (obs_mean, obs_var, obs_eps, obs_norm) set by set_rollout_targets
         self._d_values = None               # staged_ce host pipeline: device image of host-resident critic values
         self._lib = _lib.load()
         # the step keeps these in L2 with evict_last (bezk.h, bezk_l2_release): demoted again when the env goes away
@@ -511,12 +512,14 @@ class KickEnv(VecTask):
             tail = ([C.byref(ro[0]), _ptr(ro[1]), _ptr(ro[2]), _ptr(ro[3])] if ro is not None else [None, None, None, None])
             t = f["tail"]
             if self._episode is not None:     # + rl_games' episode return / length bookkeeping (set_rollout_targets)
-                rc = self._lib.bezk_post_physics_rollout_ep(ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed,
-                                                            self._rng_step, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], *tail,
-                                                            self.env_base, self.num_envs, *[_ptr(x) for x in self._episode],
-                                                            self._stream())
+                # + the eval-mode observation normaliser when armed (all NULL: exactly bezk_post_physics_rollout_ep)
+                mean, var, eps, out = self._obs_norm or (None, None, 0.0, None)
+                rc = self._lib.bezk_post_physics_rollout_ep_norm(ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed,
+                                                                 self._rng_step, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], *tail,
+                                                                 self.env_base, self.num_envs, *[_ptr(x) for x in self._episode],
+                                                                 _ptr(mean), _ptr(var), eps, _ptr(out), self._stream())
                 if rc:
-                    _lib.check(rc, "bezk_post_physics_rollout_ep")
+                    _lib.check(rc, "bezk_post_physics_rollout_ep_norm")
                 return
             rc = self._lib.bezk_post_physics_rollout(ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed,
                                                      self._rng_step, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], *tail,
@@ -803,7 +806,8 @@ class KickEnv(VecTask):
             self._post_fixed["tail"][5] = _ptr(tensor)
 
     def set_rollout_targets(self, values=None, shaped_rewards=None, dones_u8=None, gamma=0.99, scale_value=0.01, shift_value=0.0,
-                            value_bootstrap=True, episode_returns=None, episode_lengths=None, episode_partials=None):
+                            value_bootstrap=True, episode_returns=None, episode_lengths=None, episode_partials=None, obs_norm=None,
+                            obs_mean=None, obs_var=None, obs_eps=1e-5):
         """Arm the reward epilogue of the fused step (SURVEY 8 a16; rl_games ``play_steps``): the NEXT steps also write
         ``shaped_rewards = (rew + shift) * scale + gamma * values * time_outs`` (e.g. ``mb_rewards[t]``) and the uint8 reset
         mask ``dones_u8`` (e.g. the experience buffer's ``dones`` slot ``t + 1``).  ``values``: the (N,)/(N,1) un-normalised
@@ -811,10 +815,33 @@ class KickEnv(VecTask):
         ``episode_returns`` / ``episode_lengths`` ((N,) float32) and ``episode_partials`` ((3, ceil(N/32)) float64), all three or
         none, GPU pipeline only: the step also carries rl_games' ``current_rewards`` / ``current_lengths`` (unshaped reward; zeroed
         by a multiply when the env is done) and writes its done envs' count / return sum / length sum per group of 32 envs, the
-        input of ``learner.EpisodeMeter``.  Call with no arguments to disarm everything."""
+        input of ``learner.EpisodeMeter``.
+        ``obs_norm`` ((N, obs width) float32), ``obs_mean`` / ``obs_var`` ((obs width,) float64), all three or none, with the episode
+        tensors armed, GPU pipeline only: the step also writes the row it returns through ``RunningMeanStd.forward`` in eval mode
+        (``running_mean`` / ``running_var``, epsilon ``obs_eps``; read on the device every step) into ``obs_norm`` -- the input of
+        ``learner.PpoPlayerContinuous``' policy.  Call with no arguments to disarm everything."""
         if self.fusion != "fused":
             raise NotImplementedError("the reward epilogue rides in the fused step (fusion='fused')")
         n, dev = self.num_envs, self.compute_device
+        norm = (obs_mean, obs_var, obs_norm)
+        if any(t is not None for t in norm):
+            if self.host_staged:
+                raise NotImplementedError("the fused observation normaliser needs the GPU pipeline")
+            if self.dr_randomizations.get("observations", None):
+                # the noise is applied after the step kernel: a normaliser inside it would see the noise-free rows
+                raise NotImplementedError("observation domain randomisation is active: normalise the noisy rows separately")
+            if any(t is None for t in norm):
+                raise ValueError("obs_norm, obs_mean and obs_var are armed together")
+            if episode_returns is None:
+                raise ValueError("obs_norm needs the episode tensors (episode_returns, episode_lengths, episode_partials)")
+            w = self._obs_width
+            for t, dtype, numel, name in zip(norm, (torch.float64, torch.float64, torch.float32), (w, w, n * w),
+                                             ("obs_mean", "obs_var", "obs_norm")):
+                if t.dtype != dtype or t.numel() != numel or not t.is_contiguous() or t.device != dev:
+                    raise ValueError(f"{name} must be a contiguous {dtype} tensor with {numel} elements on {dev}")
+            norm = (obs_mean, obs_var, float(obs_eps), obs_norm)
+        else:
+            norm = None
         eps = (episode_returns, episode_lengths, episode_partials)
         if any(t is not None for t in eps):
             if self.host_staged:
@@ -828,6 +855,7 @@ class KickEnv(VecTask):
             self._episode = eps
         else:
             self._episode = None
+        self._obs_norm = norm
         if shaped_rewards is None and dones_u8 is None:
             self._rollout = None
             return

@@ -136,3 +136,18 @@ def train_loop_config(train_cfg):
     """``params.config`` of a resolved train yaml -> the training-loop keys of ``learner.A2CAgent``'s ``config``."""
     c = train_cfg["params"]["config"]
     return {k: c[k] for k in TRAIN_LOOP_KEYS if k in c}
+
+
+#: rl_games ``params.config.player`` keys (``BasePlayer``) with their RECALLED defaults (v1.1.x); ``learner.PpoPlayerContinuous``
+#: takes them as its ``config``
+PLAYER_DEFAULTS = dict(games_num=2000, deterministic=True, print_stats=True, n_game_life=1)
+
+
+def player_config(train_cfg):
+    """``params.config.player`` of a resolved train yaml -> the ``config`` of ``learner.PpoPlayerContinuous``: ``games_num``,
+    ``deterministic`` (rl_games' older spelling ``determenistic`` is accepted), ``print_stats``, ``n_game_life``, defaults
+    filled in."""
+    p = dict(train_cfg["params"]["config"].get("player") or {})
+    if "deterministic" not in p and "determenistic" in p:
+        p["deterministic"] = p["determenistic"]
+    return {k: type(v)(p.get(k, v)) for k, v in PLAYER_DEFAULTS.items()}

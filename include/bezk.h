@@ -396,6 +396,33 @@ int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_
  * capturable); steps == 0 or n == 0 is a no-op. */
 int bezk_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                               int64_t* size2, void* stream);
+/* bezk_post_physics_rollout_ep that also writes the observation row through rl_games' RunningMeanStd.forward in eval mode (what
+ * the player feeds its policy), from the tile the step already holds:
+ *   obs_norm (n, obs_width) f32 out = clamp((x - (float)obs_mean) / sqrtf((float)obs_var + obs_eps), -5, 5)
+ * x = the row the step returns (obs_clipped when given, obs otherwise); IEEE division and square root, NaN propagating -- the same
+ * bits as bezk_rms_normalize(x, obs_mean, obs_var, obs_eps, 0, ...).  obs_mean / obs_var (obs_width,) f64, DEVICE memory, are
+ * read by every launch.  obs_mean, obs_var, obs_norm: all NULL (then this is bezk_post_physics_rollout_ep) or all non-NULL; armed,
+ * the episode accumulators must be armed too (BEZK_E_BADARG otherwise), obs_norm 16-byte and obs_mean / obs_var 8-byte aligned
+ * (BEZK_E_ALIGN).  Every other output is the same bytes as without obs_norm. */
+int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* rigid_body, float* root_states,
+                                      float* net_contact, float* prev_lin_vel, float* goal, const float* goal_angle,
+                                      const float* ball_init, const float* initial_root_states,
+                                      const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step,
+                                      int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                      int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped,
+                                      float* rew, const BezkRolloutCfg* rollout, const float* values,
+                                      float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                      float* ep_return, float* ep_length, double* ep_partials,
+                                      const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, void* stream);
+/* rl_games BasePlayer.run's game tally fed by `steps` consecutive ep_partials over n envs (partials: (steps, 3, ceil(n / 32)) f64),
+ * step by step in order: games_played += count; sum_rewards += return sum; sum_steps += length sum, where a step that starts with
+ * games_played >= games_num adds nothing (the step that reaches games_num is added whole).  Each step's sums over its slots have
+ * a fixed order, so the result does not depend on how the steps are split over calls.
+ *   tally (4,) f64 in/out, DEVICE memory: [games_played, sum_rewards, sum_steps, steps_folded]
+ *   per_step (steps, 3) f64 out or NULL: each folded step's [count, return sum, length sum], zeros for the steps not folded.
+ * No host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op; games_num <= 0 is BEZK_E_BADARG. */
+int bezk_player_tally_update(const double* partials, int steps, int64_t n, int64_t games_num, double* tally, double* per_step,
+                             void* stream);
 /* bezk_reset_idx for any task: root rows are 13 floats for walk / orient, and their goal (n,2) rows are redrawn.
  * env_base: global id of local env 0 (Philox key = env_base + env id), as in bezk_post_physics_rollout. */
 int bezk_reset_idx_task(int task, const int64_t* env_ids, int64_t k, const float* uniforms, const float* goal_uniforms,
