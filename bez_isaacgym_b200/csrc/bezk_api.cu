@@ -82,7 +82,7 @@ static bezk::TaskArgs step_args(float* dof_state, const float* rigid_body, float
 }
 
 static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK,
-                    bezk::EpArgs* ep = nullptr, const bezk::NormArgs* nm = nullptr) {
+                    bezk::EpArgs* ep = nullptr, const bezk::NormArgs* nm = nullptr, bezk::OutArgs* oa = nullptr) {
     if (int rc = check_cfg(cfg)) return rc;
     REQUIRE(a.n >= 0, "n < 0");
     if (a.n == 0) return 0;
@@ -105,7 +105,8 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
     bezk::fill_alignment(a, *cfg);
     bezk::set_l2_policy(task, cfg->flags, a, ep);
     if (ep) ep->w = (a.n + 31) / 32;
-    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm), where);
+    if (oa) oa->w = (a.n + 31) / 32;
+    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm, oa), where);
 }
 
 int bezk_compute_observations(const float* dof_state, const float* rigid_body, const float* root_states, float* net_contact,
@@ -296,14 +297,18 @@ int bezk_post_physics_task(int task, float* dof_state, const float* rigid_body, 
     return run_task(parts, a, cfg, stream, "bezk_post_physics_task", task);
 }
 
-int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
-                                      float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
-                                      const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
-                                      uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
-                                      int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew,
-                                      const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards, uint8_t* dones_u8,
-                                      int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
-                                      const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, void* stream) {
+}  // extern "C"
+
+// the whole step with the optional episode accumulators, observation normaliser and outcome counts: the body of
+// bezk_post_physics_rollout_ep_norm (outcome_partials NULL) and bezk_post_physics_rollout_ep_outcome
+static int rollout_step(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact, float* prev_lin_vel,
+                        float* goal, const float* goal_angle, const float* ball_init, const float* initial_root_states,
+                        const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step, int64_t* reset_buf,
+                        int64_t* progress_buf, int64_t* timeout_buf, int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs,
+                        float* obs_clipped, float* rew, const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards,
+                        uint8_t* dones_u8, int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
+                        const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, int32_t* outcome_partials,
+                        void* stream) {
     REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
     REQUIRE(env_base >= 0, "env_base < 0");
     REQUIRE(!shaped_rewards || rollout, "shaped_rewards requested without a BezkRolloutCfg");
@@ -326,9 +331,47 @@ int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* r
     set_rollout(a, rollout, values, shaped_rewards, dones_u8);
     bezk::EpArgs ep = {ep_return, ep_length, ep_partials, 0};
     const bezk::NormArgs nm = {obs_mean, obs_var, obs_norm, obs_eps};
+    bezk::OutArgs oa = {outcome_partials, 0};
     return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream,
-                    norm ? "bezk_post_physics_rollout_ep_norm" : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout"),
-                    task, armed ? &ep : nullptr, norm ? &nm : nullptr);
+                    outcome_partials ? "bezk_post_physics_rollout_ep_outcome"
+                                     : (norm ? "bezk_post_physics_rollout_ep_norm"
+                                             : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout")),
+                    task, armed ? &ep : nullptr, norm ? &nm : nullptr, outcome_partials ? &oa : nullptr);
+}
+
+extern "C" {
+
+int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                      float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                      const float* initial_root_states, const float* uniforms, const float* goal_uniforms, uint64_t seed,
+                                      uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                      int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew,
+                                      const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards, uint8_t* dones_u8,
+                                      int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
+                                      const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, void* stream) {
+    return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
+                        initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
+                        obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
+                        obs_mean, obs_var, obs_eps, obs_norm, nullptr, stream);
+}
+
+int bezk_post_physics_rollout_ep_outcome(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                         float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                         const float* initial_root_states, const float* uniforms, const float* goal_uniforms,
+                                         uint64_t seed, uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                         int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew,
+                                         const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards, uint8_t* dones_u8,
+                                         int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
+                                         const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm,
+                                         int32_t* outcome_partials, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(outcome_partials, "outcome_partials NULL");
+    REQUIRE(ep_return && ep_length && ep_partials, "the outcome counts need the episode accumulators: ep_return, ep_length and ep_partials must be non-NULL");
+    if (!ALIGNED(outcome_partials, 4)) return fail(BEZK_E_ALIGN, "outcome_partials must be 4-byte aligned");
+    return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
+                        initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
+                        obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
+                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, stream);
 }
 
 int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -380,6 +423,37 @@ int bezk_player_tally_update(const double* partials, int steps, int64_t n, int64
         return fail(BEZK_E_ALIGN, "partials / tally / per_step must be 8-byte aligned");
     return cuda_rc(bezk::launch_player_tally_update(partials, steps, n, games_num, tally, per_step, (cudaStream_t)stream),
                    "bezk_player_tally_update");
+}
+
+int bezk_outcome_classes(int task) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    return bezk::outcome_classes(task);
+}
+
+int bezk_outcome_meter_update(const int32_t* partials, int steps, int64_t n, int task, int64_t games_to_track, float* mean_k,
+                              int64_t* size, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    REQUIRE(games_to_track > 0, "games_to_track must be positive");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(partials && mean_k && size, "partials / mean_k / size NULL");
+    if (!ALIGNED(partials, 4) || !ALIGNED(mean_k, 4) || !ALIGNED(size, 8))
+        return fail(BEZK_E_ALIGN, "partials / mean_k must be 4-byte and size 8-byte aligned");
+    return cuda_rc(bezk::launch_outcome_meter_update(partials, steps, n, bezk::outcome_classes(task), games_to_track, mean_k, size,
+                                                     (cudaStream_t)stream), "bezk_outcome_meter_update");
+}
+
+int bezk_player_outcome_update(const int32_t* partials, int steps, int64_t n, int task, int64_t games_num, double* counts,
+                               double* per_step, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    REQUIRE(games_num > 0, "games_num must be positive");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(partials && counts, "partials / counts NULL");
+    if (!ALIGNED(partials, 4) || !ALIGNED(counts, 8) || !ALIGNED(per_step, 8))
+        return fail(BEZK_E_ALIGN, "partials must be 4-byte and counts / per_step 8-byte aligned");
+    return cuda_rc(bezk::launch_player_outcome_update(partials, steps, n, bezk::outcome_classes(task), games_num, counts, per_step,
+                                                      (cudaStream_t)stream), "bezk_player_outcome_update");
 }
 
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream) {

@@ -70,6 +70,19 @@ struct NormArgs {
     float* out;                  // (n, obs_row) clamp((x - mean) / sqrt(var + eps), -5, 5), x = the row step() returns
     float eps;
 };
+// Episode outcome classes: the last termination rule, in the reference's override order, whose condition held -- the rule whose
+// reward the env received.  BezKick: fell, strayed, kicked wide, scored, timed out; walk / orient: fell, reached (win state), out of
+// bounds, timed out.
+enum { KICK_FELL = 0, KICK_STRAYED, KICK_WIDE, KICK_SCORED, KICK_TIMEOUT, KICK_OUTCOMES };
+enum { WALK_FELL = 0, WALK_REACHED, WALK_OUT, WALK_TIMEOUT, WALK_OUTCOMES };
+__host__ __device__ constexpr int outcome_classes(int task) { return task == BEZK_TASK_KICK ? (int)KICK_OUTCOMES : (int)WALK_OUTCOMES; }
+// Per-warp episode outcome counts of the fused step (bezk_post_physics_rollout_ep_outcome): which termination rule ended each done
+// env's episode.  A separate kernel parameter of task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel (and their _l2 forms),
+// appended after EpArgs (and NormArgs), for the reason EpArgs is one.
+struct OutArgs {
+    int32_t* partials;           // (K, W): per warp of 32 envs the count of its done envs whose episode ended through class k
+    int64_t w;                   // W
+};
 // fills l2_resident (bezk_task.cu): after fill_alignment, before the launch; ep: the armed episode accumulators or nullptr
 void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a, const EpArgs* ep = nullptr);
 // demote [ptr, ptr + bytes) to the normal L2 eviction priority (the 128-byte lines entirely inside the range)
@@ -88,9 +101,10 @@ struct PpoArgs {
 };
 // the tile kernel for (task, parts): kick takes parts 1..7, walk / orient 2, 3, 4 or 7; ep (the episode accumulators,
 // task_tile_ep_kernel / task_tile_ep_l2_kernel) only with parts = 7; nm (the observation normaliser, task_tile_obsnorm_kernel /
-// task_tile_obsnorm_l2_kernel) only together with ep.  cudaErrorInvalidValue for any other combination.
+// task_tile_obsnorm_l2_kernel) and oa (the outcome counts, task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel) only
+// together with ep.  cudaErrorInvalidValue for any other combination.
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
-                        const NormArgs* nm = nullptr);
+                        const NormArgs* nm = nullptr, const OutArgs* oa = nullptr);
 // folds `steps` x (3, ceil(n / 32)) partials of launch_task's episode accumulators into the two AverageMeters (bezk_rollout.cu)
 cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                                         int64_t* size2, cudaStream_t st);
@@ -98,6 +112,13 @@ cudaError_t launch_episode_meter_update(const double* partials, int steps, int64
 // up to games_num games (bezk_rollout.cu)
 cudaError_t launch_player_tally_update(const double* partials, int steps, int64_t n, int64_t games_num, double* tally,
                                        double* per_step, cudaStream_t st);
+// rl_games AverageMeter(K, games_to_track) fed with one one-hot outcome row per done env, from `steps` x (K, ceil(n / 32)) outcome
+// partials (bezk_rollout.cu)
+cudaError_t launch_outcome_meter_update(const int32_t* partials, int steps, int64_t n, int k, int64_t games_to_track, float* mean_k,
+                                        int64_t* size, cudaStream_t st);
+// folds the same partials into [games_counted, count_0 .. count_{K-1}] with player_tally_kernel's cutoff (bezk_rollout.cu)
+cudaError_t launch_player_outcome_update(const int32_t* partials, int steps, int64_t n, int k, int64_t games_num, double* counts,
+                                         double* per_step, cudaStream_t st);
 cudaError_t launch_goal_uniforms(uint64_t seed, uint64_t step, float* out2, cudaStream_t st);
 void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg);
 cudaError_t stage_feet_gather(const float*, const BezkTaskCfg&, float*, int64_t, int64_t, cudaStream_t);

@@ -715,4 +715,181 @@ cudaError_t launch_player_tally_update(const double* partials, int steps, int64_
     return e != cudaSuccess ? e : f;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Episode outcomes: the per-step (K, W) int32 outcome partials of the fused step (per warp of 32 envs, the count of its done envs
+// whose episode ended through class k; K = 5 for BezKick, 4 for walk / orient) folded into
+//   * outcome_meter_kernel: rl_games' AverageMeter(K, games_to_track) fed with one one-hot row per done env -- the recurrence of
+//     episode_meter_kernel, step by step in order, with new_mean[k] = count_k / total (fp32 division of exact counts) and size =
+//     total, so this meter's size always equals the game meters' size;
+//   * player_outcome_kernel: [games_counted, count_0 .. count_{K-1}] with player_tally_kernel's cutoff -- a step that starts with
+//     games_counted >= games_num adds nothing, the step that reaches it is added whole -- and optionally each step's K counts
+//     (zeros for the steps not folded).  A step's done count is the sum of its K counts.
+// Integer sums do not depend on their order: every warp of a CTA strides over its step's slots, reduces with shuffles and adds its
+// K sums to the step's with 64-bit atomics; the last warp of the launch (ticket) runs the fold in one warp.  No barrier, no local
+// memory, scratch from stream-ordered allocation: capturable in a CUDA graph.
+// ------------------------------------------------------------------------------------------------
+constexpr int OC_THREADS = 256;
+constexpr int OC_WARPS = OC_THREADS / 32;
+constexpr int OC_MAX = 5;
+
+struct OcScratch {
+    unsigned long long* step_counts;   // (steps, OC_MAX) zeroed
+    unsigned* ticket;                  // zeroed
+};
+
+// this warp's share of step blockIdx.x's K class sums; true in every lane of the last warp of the launch to finish
+__device__ __forceinline__ bool outcome_step_counts(const int32_t* __restrict__ partials, int steps, int64_t w, int k, OcScratch sc) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int step = blockIdx.x;
+    const int32_t* p = partials + (int64_t)step * k * w;
+    unsigned long long acc[OC_MAX] = {0, 0, 0, 0, 0};
+    for (int64_t i = (int64_t)warp * 32 + lane; i < w; i += OC_THREADS) {
+#pragma unroll
+        for (int c = 0; c < OC_MAX; ++c)
+            if (c < k) acc[c] += (unsigned)p[c * w + i];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int c = 0; c < OC_MAX; ++c) acc[c] += __shfl_down_sync(0xffffffffu, acc[c], o);
+    }
+    int last = 0;
+    if (lane == 0) {
+#pragma unroll
+        for (int c = 0; c < OC_MAX; ++c)
+            if (c < k && acc[c]) atomicAdd(sc.step_counts + (int64_t)step * OC_MAX + c, acc[c]);
+        __threadfence();
+        last = atomicAdd(sc.ticket, 1u) == (unsigned)steps * OC_WARPS - 1;
+    }
+    if (!__shfl_sync(0xffffffffu, last, 0)) return false;
+    __threadfence();
+    return true;
+}
+
+__global__ void __launch_bounds__(OC_THREADS) outcome_meter_kernel(const int32_t* __restrict__ partials, int steps, int64_t w, int k,
+                                                                   int64_t max_size, OcScratch sc, float* mean_k, int64_t* size) {
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    pdl_launch_dependents();
+    pdl_wait();
+    if (!outcome_step_counts(partials, steps, w, k, sc)) return;
+    // the recurrence, step by step in order: lane j loads step t0 + j's counts, every lane runs the same arithmetic
+    float mean[OC_MAX];
+#pragma unroll
+    for (int c = 0; c < OC_MAX; ++c) mean[c] = c < k ? mean_k[c] : 0.0f;
+    int64_t cur = *size;
+    for (int t0 = 0; t0 < steps; t0 += 32) {
+        unsigned long long cnt[OC_MAX] = {0, 0, 0, 0, 0};
+        if (t0 + lane < steps) {
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c) cnt[c] = __ldcg(sc.step_counts + (int64_t)(t0 + lane) * OC_MAX + c);
+        }
+        const int m = steps - t0 < 32 ? steps - t0 : 32;
+        for (int j = 0; j < m; ++j) {
+            unsigned long long cj[OC_MAX], total = 0;
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c) { cj[c] = __shfl_sync(full, cnt[c], j); total += cj[c]; }
+            if (total == 0) continue;           // AverageMeter.update: size == 0 -> no-op
+            const int64_t sz = (int64_t)total < max_size ? (int64_t)total : max_size;
+            const int64_t old_size = (max_size - sz) < cur ? (max_size - sz) : cur;
+            const int64_t size_sum = old_size + sz;
+            cur = size_sum;
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c) {
+                const float new_mean = (float)cj[c] / (float)total;
+                mean[c] = (mean[c] * (float)old_size + new_mean * (float)sz) / (float)size_sum;
+            }
+        }
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int c = 0; c < OC_MAX; ++c)
+            if (c < k) mean_k[c] = mean[c];
+        *size = cur;
+    }
+}
+
+__global__ void __launch_bounds__(OC_THREADS) player_outcome_kernel(const int32_t* __restrict__ partials, int steps, int64_t w, int k,
+                                                                    double games_num, OcScratch sc, double* counts, double* per_step) {
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    pdl_launch_dependents();
+    pdl_wait();
+    if (!outcome_step_counts(partials, steps, w, k, sc)) return;
+    double games = __ldcg(counts), tot[OC_MAX];
+#pragma unroll
+    for (int c = 0; c < OC_MAX; ++c) tot[c] = c < k ? __ldcg(counts + 1 + c) : 0.0;
+    for (int t0 = 0; t0 < steps; t0 += 32) {
+        double cnt[OC_MAX] = {0.0, 0.0, 0.0, 0.0, 0.0};
+        if (t0 + lane < steps) {
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c) cnt[c] = (double)__ldcg(sc.step_counts + (int64_t)(t0 + lane) * OC_MAX + c);
+        }
+        bool mine = false;                      // this lane's step was folded
+        const int m = steps - t0 < 32 ? steps - t0 : 32;
+        for (int j = 0; j < m; ++j) {
+            double cj[OC_MAX], total = 0.0;
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c) { cj[c] = __shfl_sync(full, cnt[c], j); total += cj[c]; }
+            if (games >= games_num) continue;   // the cutoff was reached by an earlier step
+            if (lane == j) mine = true;
+            games += total;
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c) tot[c] += cj[c];
+        }
+        if (per_step && t0 + lane < steps) {
+            double* q = per_step + (int64_t)k * (t0 + lane);
+#pragma unroll
+            for (int c = 0; c < OC_MAX; ++c)
+                if (c < k) q[c] = mine ? cnt[c] : 0.0;
+        }
+    }
+    if (lane == 0) {
+        counts[0] = games;
+#pragma unroll
+        for (int c = 0; c < OC_MAX; ++c)
+            if (c < k) counts[1 + c] = tot[c];
+    }
+}
+
+// the class sums and the ticket live for one launch only: stream-ordered scratch, zeroed on the stream
+static cudaError_t outcome_scratch(int steps, cudaStream_t st, void** buf, OcScratch& sc) {
+    const size_t bytes = (size_t)steps * OC_MAX * sizeof(unsigned long long) + sizeof(unsigned);
+    cudaError_t e = cudaMallocAsync(buf, bytes, st);
+    if (e != cudaSuccess) return e;
+    sc.step_counts = static_cast<unsigned long long*>(*buf);
+    sc.ticket = reinterpret_cast<unsigned*>(sc.step_counts + (size_t)steps * OC_MAX);
+    return cudaMemsetAsync(*buf, 0, bytes, st);
+}
+
+cudaError_t launch_outcome_meter_update(const int32_t* partials, int steps, int64_t n, int k, int64_t games_to_track, float* mean_k,
+                                        int64_t* size, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    if (k < 1 || k > OC_MAX) return cudaErrorInvalidValue;
+    void* buf = nullptr;
+    OcScratch sc;
+    cudaError_t e = outcome_scratch(steps, st, &buf, sc);
+    if (buf == nullptr) return e;
+    if (e == cudaSuccess)
+        e = launch_ex(outcome_meter_kernel, dim3((unsigned)steps), dim3(OC_THREADS), 0, st, partials, steps, (n + 31) / 32, k,
+                      games_to_track, sc, mean_k, size);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
+cudaError_t launch_player_outcome_update(const int32_t* partials, int steps, int64_t n, int k, int64_t games_num, double* counts,
+                                         double* per_step, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    if (k < 1 || k > OC_MAX) return cudaErrorInvalidValue;
+    void* buf = nullptr;
+    OcScratch sc;
+    cudaError_t e = outcome_scratch(steps, st, &buf, sc);
+    if (buf == nullptr) return e;
+    if (e == cudaSuccess)
+        e = launch_ex(player_outcome_kernel, dim3((unsigned)steps), dim3(OC_THREADS), 0, st, partials, steps, (n + 31) / 32, k,
+                      (double)games_num, sc, counts, per_step);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
 }  // namespace bezk

@@ -265,16 +265,26 @@ __device__ __forceinline__ void episode_epilogue(const EpArgs& ep, int64_t e, fl
 
 __device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep) { return ep; }
 __device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const NormArgs&) { return ep; }
+__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const OutArgs&) { return ep; }
+__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const NormArgs&, const OutArgs&) { return ep; }
 __device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs& nm) { return nm; }
+__device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs& nm, const OutArgs&) { return nm; }
+__device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const OutArgs& oa) { return oa; }
+__device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const NormArgs&, const OutArgs& oa) { return oa; }
+template <typename T, typename... P>
+constexpr bool has_arg = (std::is_same<T, P>::value || ...);
 
 // Ep: empty, or one EpArgs -- then EP is on and the episode accumulators ride along (task_tile_ep_kernel / task_tile_ep_l2_kernel;
 // whole step only) -- or EpArgs and NormArgs: the eval-mode observation normaliser too (task_tile_obsnorm_kernel /
-// task_tile_obsnorm_l2_kernel).  A parameter pack rather than always-present arguments: the kernels without accumulators make
-// exactly the call they made before the accumulators existed (an unused EpArgs argument alone changes their register allocation).
+// task_tile_obsnorm_l2_kernel).  Either EP pack may end in OutArgs: the per-warp episode outcome counts too
+// (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms).  A parameter pack rather than always-present
+// arguments: the kernels without accumulators make exactly the call they made before the accumulators existed (an unused EpArgs
+// argument alone changes their register allocation).
 template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H, typename... Ep>
 __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& cfg, const Ep&... eps) {
     constexpr bool EP = sizeof...(Ep) >= 1;
-    constexpr bool NORM = sizeof...(Ep) == 2;
+    constexpr bool NORM = has_arg<NormArgs, Ep...>;
+    constexpr bool OUT = has_arg<OutArgs, Ep...>;
     static_assert(!EP || PARTS == 7, "the episode accumulators ride in the whole step");
     constexpr int ROOT_ROW = root_row(TASK);
     constexpr int OBS_ROW = obs_row(TASK);
@@ -333,6 +343,7 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     }
     bool ep_done = false;                  // this env's episode ended in this step, with return ep_r and length ep_l
     float ep_r = 0.0f, ep_l = 0.0f;
+    int ep_oc = OUTCOME_NONE;              // OUT: the rule that ended it (the outcome class), from the reward call whose rew is stored
 
 
     // ---- 2. dense tiles: TMA bulk copies (full sub-tiles) or cooperative coalesced loads (tail) ----
@@ -582,19 +593,19 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
             for (int k = 0; k < 3; ++k) { s.v[k] = v[k]; s.w[k] = w[k]; }
             s.pos_sq = pos_sq;
             Mth<true> mr;
-            reward_term(s, cfg, progress, reset_cur, &rew, &reset, mr);
+            reward_term<true, OUT>(s, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc);
             if (mr.bad()) {
                 Mth<false> mp;
-                reward_term(s, cfg, progress, reset_cur, &rew, &reset, mp);
+                reward_term<false, OUT>(s, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc);
             }
         } else {
             Mth<true> mr;
-            if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr);
-            else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr);
+            if (TASK == BEZK_TASK_WALK) reward_walk<true, OUT>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc);
+            else reward_orient<true, OUT>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc);
             if (mr.bad()) {
                 Mth<false> mp;
-                if (TASK == BEZK_TASK_WALK) reward_walk(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp);
-                else reward_orient(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp);
+                if (TASK == BEZK_TASK_WALK) reward_walk<false, OUT>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc);
+                else reward_orient<false, OUT>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc);
             }
         }
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
@@ -620,6 +631,20 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
             ep.partials[slot] = (double)__popc(done_mask);
             ep.partials[ep.w + slot] = sr;
             ep.partials[2 * ep.w + slot] = sl;
+        }
+        if constexpr (OUT) {
+            // ... and the count of its done envs per outcome class at (k, env / 32): one ballot per class, lane k stores class k.
+            // In the whole step an env is done exactly when a rule fired (reset_cur is 0 on entry), so the K counts sum to the
+            // done count above
+            const OutArgs& oa = out_of(eps...);
+            constexpr int K = outcome_classes(TASK);
+            unsigned mine = 0;
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+                const unsigned m = __ballot_sync(0xffffffffu, ep_oc == k);
+                if (lane == k) mine = m;
+            }
+            if (lane < K) oa.partials[lane * oa.w + e0 / WT] = __popc(mine);
         }
     }
 
@@ -719,6 +744,29 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_o
                                                                                                  const EpArgs ep, const NormArgs nm) {
     task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, nm);
 }
+// the EP and the EP + normaliser steps that also count their done envs per outcome class (bezk_post_physics_rollout_ep_outcome)
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_outcome_kernel(const TaskArgs a,
+                                                                                              const __grid_constant__ BezkTaskCfg cfg,
+                                                                                              const EpArgs ep, const OutArgs oa) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, ep, oa);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_outcome_l2_kernel(const TaskArgs a,
+                                                                                                 const __grid_constant__ BezkTaskCfg cfg,
+                                                                                                 const EpArgs ep, const OutArgs oa) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, oa);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_obsnorm_outcome_kernel(
+    const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg, const EpArgs ep, const NormArgs nm, const OutArgs oa) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, ep, nm, oa);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_obsnorm_outcome_l2_kernel(
+    const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg, const EpArgs ep, const NormArgs nm, const OutArgs oa) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, nm, oa);
+}
 
 // ------------------------------------------------------------------------------------------------
 // K3 (function level): reset_idx over an explicit id list; one thread per (id, dof) pair + root rows.
@@ -772,18 +820,24 @@ static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t
 static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
 
 // Ep: empty (task_tile_kernel / task_tile_l2_kernel), the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel) or
-// those and the observation normaliser (task_tile_obsnorm_kernel / task_tile_obsnorm_l2_kernel); a.l2_resident picks the L2
+// those and the observation normaliser (task_tile_obsnorm_kernel / task_tile_obsnorm_l2_kernel), either EP pack followed by the
+// outcome counts (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms); a.l2_resident picks the L2
 // variant.  Every variant has the same shared memory: the normaliser works in the observation tile.
 template <int PARTS, bool CLEATS, int TILE, int TASK, typename... Ep>
 static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st, const Ep&... eps) {
     static_assert(sizeof...(Ep) == 0 || PARTS == 7, "the episode accumulators ride in the whole step");
     const auto kernel = [&] {
+        constexpr bool NORM = has_arg<NormArgs, Ep...>, OUT = has_arg<OutArgs, Ep...>;
         if constexpr (sizeof...(Ep) == 0)
             return a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
-        else if constexpr (sizeof...(Ep) == 1)
-            return a.l2_resident ? task_tile_ep_l2_kernel<CLEATS, TILE, TASK> : task_tile_ep_kernel<CLEATS, TILE, TASK>;
-        else
+        else if constexpr (NORM && OUT)
+            return a.l2_resident ? task_tile_obsnorm_outcome_l2_kernel<CLEATS, TILE, TASK> : task_tile_obsnorm_outcome_kernel<CLEATS, TILE, TASK>;
+        else if constexpr (OUT)
+            return a.l2_resident ? task_tile_outcome_l2_kernel<CLEATS, TILE, TASK> : task_tile_outcome_kernel<CLEATS, TILE, TASK>;
+        else if constexpr (NORM)
             return a.l2_resident ? task_tile_obsnorm_l2_kernel<CLEATS, TILE, TASK> : task_tile_obsnorm_kernel<CLEATS, TILE, TASK>;
+        else
+            return a.l2_resident ? task_tile_ep_l2_kernel<CLEATS, TILE, TASK> : task_tile_ep_kernel<CLEATS, TILE, TASK>;
     }();
     const size_t smem = (size_t)(smem_in_floats(TILE, TASK) + (a.obs_clipped ? smem_obs_floats(TILE, TASK) : 0)) * sizeof(float);
     static SmemOptIn opt_in, opt_in_l2;    // per instantiation, per device
@@ -797,13 +851,20 @@ template <int V>
 using Int = std::integral_constant<int, V>;
 
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
-                        const NormArgs* nm) {
+                        const NormArgs* nm, const OutArgs* oa) {
     const bool cleats = (cfg.flags & BEZK_F_CLEATS) != 0;
-    if (nm && !ep) return cudaErrorInvalidValue;
-    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators (and the normaliser) only with the whole step
+    if ((nm || oa) && !ep) return cudaErrorInvalidValue;
+    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators (and the normaliser / outcome counts) only with the
+    // whole step
     const auto tile = [&](auto task_c, auto parts_c) -> cudaError_t {
         constexpr int TASK = decltype(task_c)::value, PARTS = decltype(parts_c)::value;
         if constexpr (PARTS == 7) {
+            if (nm && oa)
+                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm, *oa)
+                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm, *oa);
+            if (oa)
+                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa)
+                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa);
             if (nm)
                 return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm)
                               : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm);

@@ -115,11 +115,18 @@ __device__ __forceinline__ WalkTerms walk_terms(const float (&q)[4], const float
     return t;
 }
 
-// shared tail of the two reward functions: fall, win state, (task rule), horizon
+// The outcome class (bezk_internal.h) of an env no termination rule fired for.  Written only by the OC instantiations of the reward
+// functions below.
+constexpr int OUTCOME_NONE = -1;
+
+// shared tail of the two reward functions: fall, win state, (task rule), horizon.  OC: also the outcome class into *oc_out.
+template <bool OC = false>
 __device__ __forceinline__ void walk_tail(const WalkTerms& t, bool close, float rew, bool out_rule, float out_value, const BezkTaskCfg& c,
-                                          int64_t progress, int64_t reset_cur, float* rew_out, int64_t* reset_out) {
+                                          int64_t progress, int64_t reset_cur, float* rew_out, int64_t* reset_out,
+                                          int* oc_out = nullptr) {
     int64_t reset = reset_cur;
-    if (t.up_proj < 0.7f) { reset = 1; rew = -100.0f; }                                          // fall
+    int oc = OUTCOME_NONE;
+    if (t.up_proj < 0.7f) { reset = 1; rew = -100.0f; if constexpr (OC) oc = WALK_FELL; }       // fall
     float state = close ? 1.0f : 0.0f;
     if (t.pos < 0.15f) state += 1.0f;
     if (t.vel_ang < 0.1f) state += 1.0f;
@@ -127,18 +134,21 @@ __device__ __forceinline__ void walk_tail(const WalkTerms& t, bool close, float 
     if (state == 4.0f) {                                                                          // win state
         reset = 1;
         rew = 1.0f * (1000.0f - 1000.0f * ((float)progress / (float)c.max_episode_length));
+        if constexpr (OC) oc = WALK_REACHED;
     }
-    if (out_rule) { reset = 1; rew = out_value; }                                                 // out of bound
-    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; }                     // horizon
+    if (out_rule) { reset = 1; rew = out_value; if constexpr (OC) oc = WALK_OUT; }               // out of bound
+    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; if constexpr (OC) oc = WALK_TIMEOUT; }   // horizon
     *rew_out = rew;
     *reset_out = reset;
+    if constexpr (OC) *oc_out = oc;
 }
 
 // compute_bez_reward of tasks/walk_env.py:827-997 (debug prints and dead terms dropped)
-template <bool F>
+template <bool F, bool OC = false>
 __device__ __forceinline__ void reward_walk(const float (&bez)[3], const float (&q)[4], const float (&v)[3], const float (&w)[3],
                                             float pos_sq, const float (&goal)[2], const BezkTaskCfg& c, int64_t progress,
-                                            int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m) {
+                                            int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m,
+                                            int* oc_out = nullptr) {
     const float dx = goal[0] - bez[0], dy = goal[1] - bez[1];
     const float n_goal = m.sqr(dx * dx + dy * dy);
     const float ux = m.div(dx, n_goal), uy = m.div(dy, n_goal);
@@ -156,14 +166,15 @@ __device__ __forceinline__ void reward_walk(const float (&bez)[3], const float (
     const float ang_now = atan2f_z(uy, ux);
     const float ang_init = atan2f_z(m.div(iy, n_i), m.div(ix, n_i));
     const bool out = fabsf(ang_init - ang_now) > 1.5708f;
-    walk_tail(t, close, rew, out, -100.0f, c, progress, reset_cur, rew_out, reset_out);
+    walk_tail<OC>(t, close, rew, out, -100.0f, c, progress, reset_cur, rew_out, reset_out, oc_out);
 }
 
 // compute_bez_reward of tasks/orient_env.py:845-1014
-template <bool F>
+template <bool F, bool OC = false>
 __device__ __forceinline__ void reward_orient(const float (&bez)[3], const float (&q)[4], const float (&v)[3], const float (&w)[3],
                                               float pos_sq, float goal_angle, const BezkTaskCfg& c, int64_t progress,
-                                              int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m) {
+                                              int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m,
+                                              int* oc_out = nullptr) {
     const float ang = angle_to_goal(q, goal_angle);
     const WalkTerms t = walk_terms(q, v, w, pos_sq, m);
     const float dist_h = fabsf(1.0f - t.up_proj);
@@ -174,7 +185,7 @@ __device__ __forceinline__ void reward_orient(const float (&bez)[3], const float
     const float rew = close ? height_vel_pos : vel_height;
     const float tx = bez[0] - c.bez_init_xy[0], ty = bez[1] - c.bez_init_xy[1];
     const bool out = m.sqr(tx * tx + ty * ty) > 0.3f;
-    walk_tail(t, close, rew, out, -5.0f, c, progress, reset_cur, rew_out, reset_out);
+    walk_tail<OC>(t, close, rew, out, -5.0f, c, progress, reset_cur, rew_out, reset_out, oc_out);
 }
 
 struct RewardIn {
@@ -187,10 +198,12 @@ struct RewardIn {
     float pos_sq;          // sum_j (default_j - dof_pos_j)^2, sequential
 };
 
-// compute_bez_reward, kick_env.py:1224-1395 (SURVEY A.1).  `progress` is the post-increment value.
-template <bool F>
+// compute_bez_reward, kick_env.py:1224-1395 (SURVEY A.1).  `progress` is the post-increment value.  OC: also the outcome class
+// into *oc_out.
+template <bool F, bool OC = false>
 __device__ __forceinline__ void reward_term(const RewardIn& s, const BezkTaskCfg& c, int64_t progress,
-                                            int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m) {
+                                            int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m,
+                                            int* oc_out = nullptr) {
     const float dbx = s.ball_xy[0] - s.bez[0], dby = s.ball_xy[1] - s.bez[1];
     const float nbb = m.sqr(dbx * dbx + dby * dby);
     const float vel_fwd = m.div(dbx, nbb) * s.v[0] + m.div(dby, nbb) * s.v[1];
@@ -219,18 +232,21 @@ __device__ __forceinline__ void reward_term(const RewardIn& s, const BezkTaskCfg
     const float near_r = ball_fwd * 0.1f + (vel_fwd * 0.05f - height);
     float rew = (kicked > 0.3f) ? far_r : near_r;
     int64_t reset = reset_cur;
+    int oc = OUTCOME_NONE;
 
-    if (s.bez[2] < 0.275f) { reset = 1; rew = -1.0f; }                                    // rule 1
+    if (s.bez[2] < 0.275f) { reset = 1; rew = -1.0f; if constexpr (OC) oc = KICK_FELL; }                 // rule 1
     const float tx = s.bez[0] - c.bez_init_xy[0], ty = s.bez[1] - c.bez_init_xy[1];
-    if (m.sqr(tx * tx + ty * ty) > 0.5f) { reset = 1; rew = -1.0f; }                      // rule 2
-    if (angle_diff > 1.5708f) { reset = 1; rew = -1.0f; }                                 // rule 3
-    if (n_goal < 0.05f) {                                                                 // rule 4
+    if (m.sqr(tx * tx + ty * ty) > 0.5f) { reset = 1; rew = -1.0f; if constexpr (OC) oc = KICK_STRAYED; }   // rule 2
+    if (angle_diff > 1.5708f) { reset = 1; rew = -1.0f; if constexpr (OC) oc = KICK_WIDE; }                // rule 3
+    if (n_goal < 0.05f) {                                                                                // rule 4
         reset = 1;
         rew = 1.0f * (100.0f - 100.0f * ((float)progress / (float)c.max_episode_length));
+        if constexpr (OC) oc = KICK_SCORED;
     }
-    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; }             // rule 5
+    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; if constexpr (OC) oc = KICK_TIMEOUT; }   // rule 5
     *rew_out = rew;
     *reset_out = reset;
+    if constexpr (OC) *oc_out = oc;
 }
 
 // rl_games play_steps reward path (a2c_common.py play_steps + tr_helpers.DefaultRewardsShaper; cfg/train/bez_kickPPO.yaml:53-56):

@@ -22,7 +22,7 @@ from torch import nn
 
 from .. import dist as bdist
 from . import a2c_common, experience, losses
-from .episode_meter import EpisodeMeter
+from .episode_meter import EpisodeMeter, OutcomeMeter
 from .policy_head import policy_head as _policy_head
 from .running_mean_std import RunningMeanStd
 
@@ -72,6 +72,9 @@ DEFAULT_CONFIG = dict(gamma=0.99, tau=0.95, learning_rate=3e-4, lr_schedule="ada
 #: stop when the best mean return exceeds ``score_to_win`` or after ``max_epochs`` epochs
 TRAIN_DEFAULTS = dict(games_to_track=100, save_best_after=100, save_frequency=0, score_to_win=1e9, max_epochs=int(1e6),
                       name="Bez_Kick")
+#: this project's own options (not rl_games settings): ``track_outcomes`` -- count how each episode ended (the env's ``OUTCOMES``)
+#: in the step kernel, into the ``game_outcomes`` meter and an ``outcomes`` entry of each ``train()`` history row
+OUTCOME_DEFAULTS = dict(track_outcomes=False)
 
 
 class A2CAgent:
@@ -82,7 +85,7 @@ class A2CAgent:
         ``global_advantage_stats``) the advantage moments all use the same group, so a rank-0 checkpoint carries the
         statistics of every shard.  Pass ``env.env_base`` = the rank's shard offset (``cfg['env']['envBase']``) so that the
         reset / exploration noise is keyed by global env ids."""
-        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS)
+        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS, **OUTCOME_DEFAULTS)
         cfg.update(config or {})
         process_group = bdist.resolve_group(process_group)
         self.config, self.env, self.group = cfg, env, process_group
@@ -134,6 +137,11 @@ class A2CAgent:
         self.current_lengths = torch.zeros(N, **f32)
         self._ep_partials = torch.zeros(T, 3, (N + 31) // 32, dtype=torch.float64, device=self.device)
         self.game_rewards, self.game_lengths = EpisodeMeter.pair(int(cfg["games_to_track"]), self.device)
+        # track_outcomes: the per-step outcome partials (done envs per outcome class per 32 envs) and their meter
+        self.track_outcomes = bool(cfg["track_outcomes"])
+        if self.track_outcomes:
+            self._oc_partials = torch.zeros(T, len(env.OUTCOMES), (N + 31) // 32, dtype=torch.int32, device=self.device)
+            self.game_outcomes = OutcomeMeter(env.OUTCOMES, int(cfg["games_to_track"]), self.device)
         self.obs = env.reset()["obs"].clone()
         self.dones = torch.zeros(N, dtype=torch.uint8, device=self.device)
         self.dataset = None
@@ -178,13 +186,16 @@ class A2CAgent:
                                         dones_u8=buf.slot("dones", t + 1) if t + 1 < T else self.dones, gamma=self.gamma,
                                         scale_value=shaper.get("scale_value", 1.0), shift_value=shaper.get("shift_value", 0.0),
                                         value_bootstrap=self.config["value_bootstrap"], episode_returns=self.current_rewards,
-                                        episode_lengths=self.current_lengths, episode_partials=self._ep_partials[t])
+                                        episode_lengths=self.current_lengths, episode_partials=self._ep_partials[t],
+                                        episode_outcomes=self._oc_partials[t] if self.track_outcomes else None)
                 if head_targets:
                     env.step_precomputed_targets(res["env_actions"])
                 else:
                     env.step(res["env_actions"])
             env.set_rollout_targets()
             self.game_rewards.update(self._ep_partials, self.num_actors)      # both meters, the T steps in order
+            if self.track_outcomes:
+                self.game_outcomes.update(self._oc_partials, self.num_actors)
             _, last_v = self._forward(self._norm_obs(self.obs))
             last_values = self.value_mean_std(last_v, unnorm=True) if self.config["normalize_value"] else last_v
             a2c_common.discount_values(self.dones, last_values, buf.tensor_dict["dones"], buf.tensor_dict["values"], self.mb_rewards,
@@ -320,7 +331,8 @@ class A2CAgent:
         ``last_<name>_ep_<epoch>.pth`` every ``save_frequency`` epochs; the loop stops after ``max_epochs`` epochs.  The meters
         are per rank, as in rl_games.  Deviation: rank 0 broadcasts its stop decision every epoch, so every rank leaves on the
         same epoch (in rl_games the other ranks would wait in the next epoch's collectives).  Returns ``(last_mean_rewards,
-        epoch)`` and a per-epoch history (mean return / length or None before the first finished game, losses, lr)."""
+        epoch)`` and a per-epoch history (mean return / length or None before the first finished game, losses, lr; with
+        ``track_outcomes`` also ``outcomes``: outcome name -> share of the tracked games, None before the first finished game)."""
         cfg = self.config
         rank0 = not bdist.is_distributed(self.group) or torch.distributed.get_rank() == 0
         if rank0:
@@ -331,11 +343,15 @@ class A2CAgent:
             epoch = self.epoch_num
             row = dict(epoch=epoch, mean_reward=None, mean_length=None, a_loss=float(info["a_loss"]), c_loss=float(info["c_loss"]),
                        kl=float(info["kl"]), lr=float(info["lr"]))
+            if self.track_outcomes:
+                row["outcomes"] = None
             should_exit = False
             if rank0:
                 if self.game_rewards.current_size > 0:
                     mean_rewards = float(self.game_rewards.get_mean()[0])
                     row["mean_reward"], row["mean_length"] = mean_rewards, float(self.game_lengths.get_mean()[0])
+                    if self.track_outcomes:
+                        row["outcomes"] = self.game_outcomes.as_dict()
                     if cfg["save_frequency"] > 0 and epoch % cfg["save_frequency"] == 0 and mean_rewards <= self.last_mean_rewards:
                         self.save(os.path.join(directory, f"last_{cfg['name']}_ep_{epoch}"))
                     if mean_rewards > self.last_mean_rewards and epoch >= cfg["save_best_after"]:

@@ -45,3 +45,47 @@ class EpisodeMeter:
         """Both meters of the pair: they are only ever updated together."""
         self._mean2.zero_()
         self._size2.zero_()
+
+
+class OutcomeMeter:
+    """``AverageMeter(K, games_to_track)`` fed with one one-hot row per finished episode, over the outcome classes ``names`` (the
+    env's ``OUTCOMES``): the share of the last ``games_to_track`` episodes that ended through each termination rule.  Kept on the
+    device and fed by the fused step's outcome partials (``KickEnv.set_rollout_targets(episode_outcomes=...)``) with
+    ``EpisodeMeter``'s recurrence and step order, so after the same updates ``current_size`` equals the game meters'."""
+
+    def __init__(self, names, games_to_track=100, device="cuda"):
+        from ..tasks import KickEnv, WalkEnv
+        if int(games_to_track) <= 0:
+            raise ValueError("games_to_track must be positive")
+        self.names = tuple(names)
+        # the fold takes the task whose classes these are (walk and orient share theirs)
+        tasks = {KickEnv.OUTCOMES: KickEnv.TASK, WalkEnv.OUTCOMES: WalkEnv.TASK}
+        if self.names not in tasks:
+            raise ValueError(f"names must be the OUTCOMES of an env: {KickEnv.OUTCOMES} or {WalkEnv.OUTCOMES}")
+        self.task = tasks[self.names]
+        self.max_size = int(games_to_track)
+        self.device = torch.device(device)
+        self._mean = torch.zeros(len(self.names), dtype=torch.float32, device=self.device)
+        self._size = torch.zeros(1, dtype=torch.int64, device=self.device)
+
+    def update(self, partials, num_envs):
+        """Fold (T, K, ceil(num_envs/32)) int32 outcome partials -- T consecutive steps -- step by step in order, one launch."""
+        k, w = len(self.names), (int(num_envs) + 31) // 32
+        ops.outcome_meter_update(partials, num_envs, self.task, self.max_size, self._mean, self._size,
+                                 steps=partials.numel() // (k * w))
+
+    @property
+    def current_size(self):
+        return int(self._size[0])
+
+    def get_mean(self):
+        """numpy (K,): the share of each class among the tracked episodes."""
+        return self._mean.cpu().numpy()
+
+    def as_dict(self):
+        """name -> share, one device-to-host read."""
+        return dict(zip(self.names, (float(x) for x in self.get_mean())))
+
+    def clear(self):
+        self._mean.zero_()
+        self._size.zero_()

@@ -10,7 +10,9 @@ One player step is three launches and no host synchronisation:
 
 rl_games' per-step tally (``done.nonzero()``, ``cr[done].sum().item()``, ``steps[done].sum().item()``) is one fold launch
 (``bezk_player_tally_update``) and one host read every ``sync_every`` steps; the fold stops adding at the step that reaches
-``games_num * n_game_life`` games, so the result does not depend on ``sync_every``.  With observation domain randomisation the
+``games_num * n_game_life`` games, so the result does not depend on ``sync_every``.  With ``track_outcomes`` the step also counts
+how each episode ended (the env's ``OUTCOMES``), and a second fold with the same cutoff (``bezk_player_outcome_update``) joins the
+same host read.  With observation domain randomisation the
 noise lands after the step kernel, so the player then normalises the noisy rows with ``RunningMeanStd`` (eval mode) instead.
 """
 import math
@@ -27,10 +29,11 @@ MAX_STEPS = 108000 // 4
 
 
 class PpoPlayerContinuous:
-    def __init__(self, env, config=None, seed=0, sync_every=32):
+    def __init__(self, env, config=None, seed=0, sync_every=32, track_outcomes=False):
         """``config``: ``PLAYER_DEFAULTS`` keys (``utils.config.player_config``; the older spelling ``determenistic`` is accepted)
         and ``normalize_input`` (default True, as ``learner.A2CAgent``).  ``seed``: Philox key of the sampled actions.
-        ``sync_every``: env steps per tally fold and host read."""
+        ``sync_every``: env steps per tally fold and host read.  ``track_outcomes``: also count the games per outcome class
+        (``run()`` then returns ``outcomes`` / ``outcome_rates`` and prints an ``outcomes:`` line)."""
         config = dict(config or {})
         if "determenistic" in config:
             config.setdefault("deterministic", config.pop("determenistic"))
@@ -59,6 +62,11 @@ class PpoPlayerContinuous:
         self._per_step = torch.zeros(self.sync_every, 3, **f64)
         self._env_actions = torch.zeros(n, env.num_acts, **f32)
         self._targets = torch.zeros(n, env.num_acts, **f32)        # K0 output when env.step recomputes the targets
+        # track_outcomes: the outcome partials of one chunk and [games_counted, count per class]
+        self.track_outcomes = bool(track_outcomes)
+        if self.track_outcomes:
+            self._oc_partials = torch.zeros(self.sync_every, len(env.OUTCOMES), w, dtype=torch.int32, device=self.device)
+            self._oc_counts = torch.zeros(1 + len(env.OUTCOMES), **f64)
 
     # ------------------------------------------------------------------ checkpoints
     def restore(self, fn):
@@ -111,6 +119,8 @@ class PpoPlayerContinuous:
     def _arm(self, t, fused):
         rms = self.running_mean_std
         extra = dict(obs_norm=self.obs_norm, obs_mean=rms.running_mean, obs_var=rms.running_var, obs_eps=rms.epsilon) if fused else {}
+        if self.track_outcomes:
+            extra["episode_outcomes"] = self._oc_partials[t]
         self.env.set_rollout_targets(episode_returns=self.current_rewards, episode_lengths=self.current_lengths,
                                      episode_partials=self._partials[t], **extra)
 
@@ -134,11 +144,15 @@ class PpoPlayerContinuous:
         """rl_games ``BasePlayer.run``: play until ``games_num * n_game_life`` games have finished (the last step may overshoot),
         restarting from ``env_reset()`` every ``max_steps`` steps.  Prints rl_games' ``reward: ... steps: ...`` line for every
         step with finished games (``print_stats``) and the final ``av reward: ... av steps: ...``.  Returns dict(games_played,
-        sum_rewards, sum_steps, av_reward, av_steps)."""
+        sum_rewards, sum_steps, av_reward, av_steps); with ``track_outcomes`` also ``outcomes`` (outcome name -> games) and
+        ``outcome_rates`` (outcome name -> share of the games played), printed as one ``outcomes:`` line after ``av reward``."""
         env, n = self.env, self.env.num_envs
         n_games = self.games_num * self.n_game_life
         tally = self._tally.zero_()
+        if self.track_outcomes:
+            self._oc_counts.zero_()
         games_played = sum_rewards = sum_steps = 0.0
+        oc_host = None
         try:
             with torch.no_grad():
                 for _ in range(n_games):
@@ -155,8 +169,15 @@ class PpoPlayerContinuous:
                             obs = self._env_step(actions)
                         done_steps += k
                         ops.player_tally_update(self._partials[:k], n, n_games, tally, self._per_step[:k], steps=k)
-                        host = torch.cat([tally, self._per_step[:k].reshape(-1)]).cpu()      # the one host read of the chunk
+                        parts = [tally, self._per_step[:k].reshape(-1)]
+                        if self.track_outcomes:
+                            ops.player_outcome_update(self._oc_partials[:k], n, env.TASK, n_games, self._oc_counts, steps=k)
+                            parts.append(self._oc_counts)
+                        host = torch.cat(parts).cpu()      # the one host read of the chunk
                         games_played, sum_rewards, sum_steps = float(host[0]), float(host[1]), float(host[2])
+                        if self.track_outcomes:
+                            oc_host = host[4 + 3 * k:]
+                            host = host[:4 + 3 * k]
                         if self.print_stats:
                             for cnt, r, s in host[4:].view(k, 3).tolist():
                                 if cnt > 0:
@@ -167,4 +188,11 @@ class PpoPlayerContinuous:
         av_steps = sum_steps / games_played * self.n_game_life if games_played else math.nan
         print(sum_rewards)
         print("av reward:", av_reward, "av steps:", av_steps)
-        return dict(games_played=games_played, sum_rewards=sum_rewards, sum_steps=sum_steps, av_reward=av_reward, av_steps=av_steps)
+        res = dict(games_played=games_played, sum_rewards=sum_rewards, sum_steps=sum_steps, av_reward=av_reward, av_steps=av_steps)
+        if self.track_outcomes:
+            counts = [0.0] * len(env.OUTCOMES) if oc_host is None else [float(x) for x in oc_host[1:]]
+            res["outcomes"] = dict(zip(env.OUTCOMES, counts))
+            res["outcome_rates"] = {name: (c / games_played if games_played else math.nan) for name, c in res["outcomes"].items()}
+            print("outcomes:", " ".join(f"{name} {int(c)} ({100.0 * res['outcome_rates'][name]:.1f} %)"
+                                        for name, c in res["outcomes"].items()))
+        return res

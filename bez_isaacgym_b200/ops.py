@@ -307,6 +307,88 @@ def player_tally_update(partials, n, games_num, tally, per_step=None, steps=None
                                             _cuda(tally, F64, "tally", 4), ps, _stream(partials)), "bezk_player_tally_update")
 
 
+I32 = torch.int32
+
+
+def outcome_classes(task):
+    """K, the number of episode outcome classes of ``task`` (5 for ``"kick"``, 4 for ``"walk"`` / ``"orient"``;
+    ``bezk_outcome_classes``)."""
+    k = _lib.load().bezk_outcome_classes(_TASK_ID[task])
+    if k == 10001:                                   # BEZK_E_BADARG
+        _lib.check(k, "bezk_outcome_classes")
+    return k
+
+
+def post_physics_rollout_ep_outcome(task, dof_state, rigid_body, root_states, net_contact, goal, initial_root_states, reset_buf,
+                                    progress_buf, timeout_buf, cfg, obs, rew, episode_returns, episode_lengths, episode_partials,
+                                    outcome_partials, obs_mean=None, obs_var=None, obs_norm=None, obs_eps=1e-5, rollout_cfg=None,
+                                    values=None, shaped_rewards=None, dones_u8=None, goal_angle=None, ball_init=None, prev_lin_vel=None,
+                                    uniforms=None, goal_uniforms=None, seed=0, step=0, randomize_buf=None, obs_clipped=None, env_base=0):
+    """``post_physics_rollout_ep`` (or ``_ep_norm`` when ``obs_mean`` / ``obs_var`` / ``obs_norm`` are given) that also writes the
+    per-warp count of done envs per outcome class (``outcome_partials``, (K, ceil(N/32)) int32, CUDA;
+    ``bezk_post_physics_rollout_ep_outcome``)."""
+    n = progress_buf.shape[0]
+    nb = cfg.num_bodies
+    actors, _, width = bm.task_dims(task)
+    ret = _cuda(episode_returns, F32, "episode_returns", n)
+    length = _cuda(episode_lengths, F32, "episode_lengths", n)
+    part = _cuda(episode_partials, F64, "episode_partials", 3 * ((n + 31) // 32))
+    oc = _cuda(outcome_partials, I32, "outcome_partials", outcome_classes(task) * ((n + 31) // 32))
+    norm = (obs_mean, obs_var, obs_norm)
+    if any(t is not None for t in norm):
+        mean, var = _cuda(obs_mean, F64, "obs_mean", width), _cuda(obs_var, F64, "obs_var", width)
+        out = _cuda(obs_norm, F32, "obs_norm", n * width)
+    else:
+        mean = var = out = None
+    lib = _lib.load()
+    _lib.check(lib.bezk_post_physics_rollout_ep_outcome(
+        _TASK_ID[task], _p(dof_state, F32, "dof_state", n * 36), _p(rigid_body, F32, "rigid_body", n * nb * 13),
+        _p(root_states, F32, "root_states", n * actors * 13), _p(net_contact, F32, "net_contact", n * nb * 3),
+        _p(prev_lin_vel, F32, "prev_lin_vel", n * 3, True), _p(goal, F32, "goal", n * 2),
+        _p(goal_angle, F32, "goal_angle", n, True), _p(ball_init, F32, "ball_init", n * 2, True),
+        _p(initial_root_states, F32, "initial_root_states", n * actors * 13, True),
+        _p(uniforms, F32, "uniforms", n * 36, True), _p(goal_uniforms, F32, "goal_uniforms", 2, True), seed, step,
+        _p(reset_buf, I64, "reset_buf", n), _p(progress_buf, I64, "progress_buf", n),
+        _p(timeout_buf, I64, "timeout_buf", n), _p(randomize_buf, I64, "randomize_buf", n, True), C.byref(cfg),
+        _p(obs, F32, "obs", n * width), _p(obs_clipped, F32, "obs_clipped", n * width, True), _p(rew, F32, "rew", n),
+        C.byref(rollout_cfg) if rollout_cfg is not None else None, _p(values, F32, "values", n, True),
+        _p(shaped_rewards, F32, "shaped_rewards", n, True), _p(dones_u8, U8, "dones_u8", n, True), int(env_base), n,
+        ret, length, part, mean, var, float(obs_eps), out, oc, _stream(dof_state)), "bezk_post_physics_rollout_ep_outcome")
+
+
+def _outcome_steps(partials, n, k, steps):
+    w = (int(n) + 31) // 32
+    if steps is None:
+        steps = partials.numel() // (k * w) if w else 0
+    if not isinstance(partials, torch.Tensor) or partials.numel() != int(steps) * k * w:
+        raise BezkError(f"partials must hold steps x {k} x {w} int32 values")
+    return int(steps)
+
+
+def outcome_meter_update(partials, n, task, games_to_track, mean_k, size, steps=None):
+    """Fold ``steps`` consecutive (K, ceil(n/32)) int32 outcome partials (``partials``: (steps, K, W) or (K, W)) into rl_games'
+    ``AverageMeter(K, games_to_track)`` ``mean_k`` ((K,) float32) / ``size`` ((1,) int64), on the device
+    (``bezk_outcome_meter_update``)."""
+    k = outcome_classes(task)
+    steps = _outcome_steps(partials, n, k, steps)
+    lib = _lib.load()
+    _lib.check(lib.bezk_outcome_meter_update(_cuda(partials, I32, "partials", None), steps, int(n), _TASK_ID[task], int(games_to_track),
+                                             _cuda(mean_k, F32, "mean_k", k), _cuda(size, I64, "size", 1), _stream(partials)),
+               "bezk_outcome_meter_update")
+
+
+def player_outcome_update(partials, n, task, games_num, counts, per_step=None, steps=None):
+    """Fold ``steps`` consecutive (K, ceil(n/32)) int32 outcome partials into ``counts`` ((1 + K,) float64: games_counted, then the
+    games per class) up to ``games_num`` games, with ``player_tally_update``'s cutoff; ``per_step`` ((steps, K) float64, optional)
+    gets each folded step's counts (``bezk_player_outcome_update``)."""
+    k = outcome_classes(task)
+    steps = _outcome_steps(partials, n, k, steps)
+    ps = None if per_step is None else _cuda(per_step, F64, "per_step", steps * k)
+    lib = _lib.load()
+    _lib.check(lib.bezk_player_outcome_update(_cuda(partials, I32, "partials", None), steps, int(n), _TASK_ID[task], int(games_num),
+                                              _cuda(counts, F64, "counts", 1 + k), ps, _stream(partials)), "bezk_player_outcome_update")
+
+
 def reset_idx_task(task, env_ids, dof_state, root_states, initial_root_states, goal, progress, reset, cfg, uniforms=None,
                    goal_uniforms=None, seed=0, step=0, env_base=0):
     k = int(env_ids.numel())

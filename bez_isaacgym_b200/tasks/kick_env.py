@@ -51,6 +51,10 @@ class KickEnv(VecTask):
     #: "kick" here; the sibling tasks (tasks/walk_env.py, tasks/orient_env.py) subclass this with "walk" / "orient": same
     #: skeleton, one actor per env, 52-wide observation, their own heading term / reward / goal randomisation (bezk.h)
     TASK = "kick"
+    #: episode outcome classes, in the order of the fused step's outcome counts (``set_rollout_targets(episode_outcomes=...)``):
+    #: the termination rule of ``compute_bez_reward`` whose reward a done env received -- the last one, in the reference's
+    #: override order, whose condition held
+    OUTCOMES = ("fell", "strayed", "wide", "scored", "timeout")
     #: host pipelines (``sim.use_gpu_pipeline: False``), selected by ``env.hostPipeline``
     HOST_PIPELINES = ("zero_copy", "staged", "staged_ce", "staged_pack")
 
@@ -212,6 +216,7 @@ class KickEnv(VecTask):
         self._rollout = None                # (BezkRolloutCfg, values, shaped_rewards, dones_u8) set by set_rollout_targets
         self._episode = None                # (episode_returns, episode_lengths, episode_partials) set by set_rollout_targets
         self._obs_norm = None               # (obs_mean, obs_var, obs_eps, obs_norm) set by set_rollout_targets
+        self._outcomes = None               # (K, ceil(N/32)) int32 outcome partials set by set_rollout_targets
         self._d_values = None               # staged_ce host pipeline: device image of host-resident critic values
         self._lib = _lib.load()
         # the step keeps these in L2 with evict_last (bezk.h, bezk_l2_release): demoted again when the env goes away
@@ -514,6 +519,14 @@ class KickEnv(VecTask):
             if self._episode is not None:     # + rl_games' episode return / length bookkeeping (set_rollout_targets)
                 # + the eval-mode observation normaliser when armed (all NULL: exactly bezk_post_physics_rollout_ep)
                 mean, var, eps, out = self._obs_norm or (None, None, 0.0, None)
+                if self._outcomes is not None:    # + the per-warp episode outcome counts
+                    rc = self._lib.bezk_post_physics_rollout_ep_outcome(
+                        ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed, self._rng_step, t[0], t[1], t[2], t[3],
+                        t[4], t[5], t[6], t[7], *tail, self.env_base, self.num_envs, *[_ptr(x) for x in self._episode], _ptr(mean),
+                        _ptr(var), eps, _ptr(out), _ptr(self._outcomes), self._stream())
+                    if rc:
+                        _lib.check(rc, "bezk_post_physics_rollout_ep_outcome")
+                    return
                 rc = self._lib.bezk_post_physics_rollout_ep_norm(ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed,
                                                                  self._rng_step, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], *tail,
                                                                  self.env_base, self.num_envs, *[_ptr(x) for x in self._episode],
@@ -807,7 +820,7 @@ class KickEnv(VecTask):
 
     def set_rollout_targets(self, values=None, shaped_rewards=None, dones_u8=None, gamma=0.99, scale_value=0.01, shift_value=0.0,
                             value_bootstrap=True, episode_returns=None, episode_lengths=None, episode_partials=None, obs_norm=None,
-                            obs_mean=None, obs_var=None, obs_eps=1e-5):
+                            obs_mean=None, obs_var=None, obs_eps=1e-5, episode_outcomes=None):
         """Arm the reward epilogue of the fused step (SURVEY 8 a16; rl_games ``play_steps``): the NEXT steps also write
         ``shaped_rewards = (rew + shift) * scale + gamma * values * time_outs`` (e.g. ``mb_rewards[t]``) and the uint8 reset
         mask ``dones_u8`` (e.g. the experience buffer's ``dones`` slot ``t + 1``).  ``values``: the (N,)/(N,1) un-normalised
@@ -819,7 +832,10 @@ class KickEnv(VecTask):
         ``obs_norm`` ((N, obs width) float32), ``obs_mean`` / ``obs_var`` ((obs width,) float64), all three or none, with the episode
         tensors armed, GPU pipeline only: the step also writes the row it returns through ``RunningMeanStd.forward`` in eval mode
         (``running_mean`` / ``running_var``, epsilon ``obs_eps``; read on the device every step) into ``obs_norm`` -- the input of
-        ``learner.PpoPlayerContinuous``' policy.  Call with no arguments to disarm everything."""
+        ``learner.PpoPlayerContinuous``' policy.
+        ``episode_outcomes`` ((K, ceil(N/32)) int32, K = ``len(OUTCOMES)``), with the episode tensors armed, GPU pipeline only: the
+        step also writes, per group of 32 envs, how many of its done envs ended through each class of ``OUTCOMES`` -- the input of
+        ``learner.OutcomeMeter`` and of the player's outcome counts.  Call with no arguments to disarm everything."""
         if self.fusion != "fused":
             raise NotImplementedError("the reward epilogue rides in the fused step (fusion='fused')")
         n, dev = self.num_envs, self.compute_device
@@ -842,6 +858,15 @@ class KickEnv(VecTask):
             norm = (obs_mean, obs_var, float(obs_eps), obs_norm)
         else:
             norm = None
+        if episode_outcomes is not None:
+            if self.host_staged:
+                raise NotImplementedError("episode outcomes need the GPU pipeline")
+            if episode_returns is None:
+                raise ValueError("episode_outcomes needs the episode tensors (episode_returns, episode_lengths, episode_partials)")
+            numel = len(self.OUTCOMES) * ((n + 31) // 32)
+            t = episode_outcomes
+            if t.dtype != torch.int32 or t.numel() != numel or not t.is_contiguous() or t.device != dev:
+                raise ValueError(f"episode_outcomes must be a contiguous torch.int32 tensor with {numel} elements on {dev}")
         eps = (episode_returns, episode_lengths, episode_partials)
         if any(t is not None for t in eps):
             if self.host_staged:
@@ -856,6 +881,7 @@ class KickEnv(VecTask):
         else:
             self._episode = None
         self._obs_norm = norm
+        self._outcomes = episode_outcomes
         if shaped_rewards is None and dones_u8 is None:
             self._rollout = None
             return

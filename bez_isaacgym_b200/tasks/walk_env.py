@@ -21,6 +21,8 @@ from .kick_env import KickEnv
 
 class WalkEnv(KickEnv):
     TASK = "walk"
+    #: fell (up-vector projection < 0.7), reached (win state), out (out of bounds), timeout -- OrientEnv shares them
+    OUTCOMES = ("fell", "reached", "out", "timeout")
 
     def _read_task_cfg(self, env_cfg):
         """No ball actor (walk_env.py:146-149); the yaml carries no ``ballInitState``."""

@@ -423,6 +423,43 @@ int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* r
  * No host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op; games_num <= 0 is BEZK_E_BADARG. */
 int bezk_player_tally_update(const double* partials, int steps, int64_t n, int64_t games_num, double* tally, double* per_step,
                              void* stream);
+/* Episode outcomes: which termination rule of compute_bez_reward ended each episode -- the last rule, in the reference's override
+ * order, whose condition held, i.e. the rule whose reward the env received.  Classes, in index order:
+ *   BEZK_TASK_KICK (K = 5):             fell, strayed, wide (kicked wide), scored, timeout
+ *   BEZK_TASK_WALK / _ORIENT (K = 4):   fell, reached (win state), out (out of bounds), timeout
+ * bezk_outcome_classes returns K for a task, BEZK_E_BADARG for an unknown one. */
+int bezk_outcome_classes(int task);
+/* bezk_post_physics_rollout_ep_norm that also counts its done envs per outcome class:
+ *   outcome_partials (K, W) int32 out, DEVICE memory, W = ceil(n / 32), 4-byte aligned: at [k * W + env / 32] the number of envs
+ *                    of that group of 32 whose episode ended in this step through class k.  Every slot is written each step
+ *                    (zeros included), so the buffer needs no zeroing; the K counts of a group sum to its count in ep_partials.
+ * outcome_partials and the episode accumulators are required (BEZK_E_BADARG); the normaliser arguments stay optional (all NULL:
+ * bezk_post_physics_rollout_ep with outcomes).  Every other output is the same bytes as without outcome_partials. */
+int bezk_post_physics_rollout_ep_outcome(int task, float* dof_state, const float* rigid_body, float* root_states,
+                                         float* net_contact, float* prev_lin_vel, float* goal, const float* goal_angle,
+                                         const float* ball_init, const float* initial_root_states,
+                                         const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step,
+                                         int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                         int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped,
+                                         float* rew, const BezkRolloutCfg* rollout, const float* values,
+                                         float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                         float* ep_return, float* ep_length, double* ep_partials,
+                                         const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm,
+                                         int32_t* outcome_partials, void* stream);
+/* rl_games' AverageMeter(K, games_to_track) fed with one one-hot outcome row per done env, from `steps` consecutive
+ * outcome_partials over n envs ((steps, K, ceil(n / 32)) int32), step by step in order, with bezk_episode_meter_update's
+ * recurrence: size = the step's done count (sum of its K counts), new_mean[k] = (float)count_k / (float)size.  A step with no done
+ * env changes nothing, so *size always equals the game meters' size.  mean_k (K,) f32 and size (1,) i64, DEVICE memory, in/out.
+ * No host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op. */
+int bezk_outcome_meter_update(const int32_t* partials, int steps, int64_t n, int task, int64_t games_to_track, float* mean_k,
+                              int64_t* size, void* stream);
+/* BasePlayer.run's game tally per outcome: `steps` consecutive outcome_partials folded into counts (1 + K,) f64 in/out, DEVICE
+ * memory: [games_counted, count_0 .. count_{K-1}], with bezk_player_tally_update's cutoff (a step that starts with
+ * games_counted >= games_num adds nothing, the step that reaches it is added whole), so over the same steps games_counted equals
+ * that tally's games_played.  per_step (steps, K) f64 out or NULL: each folded step's K counts, zeros for the steps not folded.
+ * No host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op; games_num <= 0 is BEZK_E_BADARG. */
+int bezk_player_outcome_update(const int32_t* partials, int steps, int64_t n, int task, int64_t games_num, double* counts,
+                               double* per_step, void* stream);
 /* bezk_reset_idx for any task: root rows are 13 floats for walk / orient, and their goal (n,2) rows are redrawn.
  * env_base: global id of local env 0 (Philox key = env_base + env id), as in bezk_post_physics_rollout. */
 int bezk_reset_idx_task(int task, const int64_t* env_ids, int64_t k, const float* uniforms, const float* goal_uniforms,
