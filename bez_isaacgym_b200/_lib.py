@@ -117,6 +117,11 @@ SIGNATURES = {
                                                        _I64, _I64, _P, _P, _P, _P, _P, C.c_float, _P, _P, _P]),
     "bezk_outcome_meter_update": (C.c_int, [_P, C.c_int, _I64, C.c_int, _I64, _P, _P, _P]),
     "bezk_player_outcome_update": (C.c_int, [_P, C.c_int, _I64, C.c_int, _I64, _P, _P, _P]),
+    "bezk_reward_terms": (C.c_int, [C.c_int]),
+    "bezk_post_physics_rollout_ep_terms": (C.c_int, [C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _U64, _U64, _P, _P, _P,
+                                                     _P, C.POINTER(BezkTaskCfg), _P, _P, _P, C.POINTER(BezkRolloutCfg), _P, _P, _P,
+                                                     _I64, _I64, _P, _P, _P, _P, _P, C.c_float, _P, _P, _P, _P]),
+    "bezk_reward_terms_update": (C.c_int, [_P, C.c_int, _I64, C.c_int, _P, _P]),
     "bezk_reset_idx_task": (C.c_int, [C.c_int, _P, _I64, _P, _P, _U64, _U64, _P, _P, _P, _P, _P, _P, C.POINTER(BezkTaskCfg), _I64, _I64,
                                       _P]),
     "bezk_goal_uniforms": (C.c_int, [_U64, _U64, _P, _P]),

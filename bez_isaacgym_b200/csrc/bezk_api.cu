@@ -82,7 +82,8 @@ static bezk::TaskArgs step_args(float* dof_state, const float* rigid_body, float
 }
 
 static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK,
-                    bezk::EpArgs* ep = nullptr, const bezk::NormArgs* nm = nullptr, bezk::OutArgs* oa = nullptr) {
+                    bezk::EpArgs* ep = nullptr, const bezk::NormArgs* nm = nullptr, bezk::OutArgs* oa = nullptr,
+                    bezk::TermArgs* ta = nullptr) {
     if (int rc = check_cfg(cfg)) return rc;
     REQUIRE(a.n >= 0, "n < 0");
     if (a.n == 0) return 0;
@@ -106,7 +107,8 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
     bezk::set_l2_policy(task, cfg->flags, a, ep);
     if (ep) ep->w = (a.n + 31) / 32;
     if (oa) oa->w = (a.n + 31) / 32;
-    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm, oa), where);
+    if (ta) ta->w = (a.n + 31) / 32;
+    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm, oa, ta), where);
 }
 
 int bezk_compute_observations(const float* dof_state, const float* rigid_body, const float* root_states, float* net_contact,
@@ -299,8 +301,9 @@ int bezk_post_physics_task(int task, float* dof_state, const float* rigid_body, 
 
 }  // extern "C"
 
-// the whole step with the optional episode accumulators, observation normaliser and outcome counts: the body of
-// bezk_post_physics_rollout_ep_norm (outcome_partials NULL) and bezk_post_physics_rollout_ep_outcome
+// the whole step with the optional episode accumulators, observation normaliser, outcome counts and reward terms: the body of
+// bezk_post_physics_rollout_ep_norm (outcome_partials and term_partials NULL), bezk_post_physics_rollout_ep_outcome (term_partials
+// NULL) and bezk_post_physics_rollout_ep_terms
 static int rollout_step(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact, float* prev_lin_vel,
                         float* goal, const float* goal_angle, const float* ball_init, const float* initial_root_states,
                         const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step, int64_t* reset_buf,
@@ -308,7 +311,7 @@ static int rollout_step(int task, float* dof_state, const float* rigid_body, flo
                         float* obs_clipped, float* rew, const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards,
                         uint8_t* dones_u8, int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
                         const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, int32_t* outcome_partials,
-                        void* stream) {
+                        double* term_partials, void* stream) {
     REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
     REQUIRE(env_base >= 0, "env_base < 0");
     REQUIRE(!shaped_rewards || rollout, "shaped_rewards requested without a BezkRolloutCfg");
@@ -332,11 +335,13 @@ static int rollout_step(int task, float* dof_state, const float* rigid_body, flo
     bezk::EpArgs ep = {ep_return, ep_length, ep_partials, 0};
     const bezk::NormArgs nm = {obs_mean, obs_var, obs_norm, obs_eps};
     bezk::OutArgs oa = {outcome_partials, 0};
+    bezk::TermArgs ta = {term_partials, 0};
     return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream,
-                    outcome_partials ? "bezk_post_physics_rollout_ep_outcome"
-                                     : (norm ? "bezk_post_physics_rollout_ep_norm"
-                                             : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout")),
-                    task, armed ? &ep : nullptr, norm ? &nm : nullptr, outcome_partials ? &oa : nullptr);
+                    term_partials ? "bezk_post_physics_rollout_ep_terms"
+                                  : (outcome_partials ? "bezk_post_physics_rollout_ep_outcome"
+                                                      : (norm ? "bezk_post_physics_rollout_ep_norm"
+                                                              : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout"))),
+                    task, armed ? &ep : nullptr, norm ? &nm : nullptr, outcome_partials ? &oa : nullptr, term_partials ? &ta : nullptr);
 }
 
 extern "C" {
@@ -352,7 +357,7 @@ int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* r
     return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
                         initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
                         obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
-                        obs_mean, obs_var, obs_eps, obs_norm, nullptr, stream);
+                        obs_mean, obs_var, obs_eps, obs_norm, nullptr, nullptr, stream);
 }
 
 int bezk_post_physics_rollout_ep_outcome(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -371,7 +376,28 @@ int bezk_post_physics_rollout_ep_outcome(int task, float* dof_state, const float
     return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
                         initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
                         obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
-                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, stream);
+                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, nullptr, stream);
+}
+
+int bezk_post_physics_rollout_ep_terms(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                       float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                       const float* initial_root_states, const float* uniforms, const float* goal_uniforms,
+                                       uint64_t seed, uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                       int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew,
+                                       const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards, uint8_t* dones_u8,
+                                       int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
+                                       const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm,
+                                       int32_t* outcome_partials, double* term_partials, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(term_partials, "term_partials NULL");
+    REQUIRE(ep_return && ep_length && ep_partials, "the reward terms need the episode accumulators: ep_return, ep_length and ep_partials must be non-NULL");
+    REQUIRE(!obs_mean && !obs_var && !obs_norm, "the reward terms do not ride with the observation normaliser: obs_mean, obs_var and obs_norm must be NULL");
+    if (!ALIGNED(term_partials, 8)) return fail(BEZK_E_ALIGN, "term_partials must be 8-byte aligned");
+    if (!ALIGNED(outcome_partials, 4)) return fail(BEZK_E_ALIGN, "outcome_partials must be 4-byte aligned");
+    return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
+                        initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
+                        obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
+                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, term_partials, stream);
 }
 
 int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -454,6 +480,21 @@ int bezk_player_outcome_update(const int32_t* partials, int steps, int64_t n, in
         return fail(BEZK_E_ALIGN, "partials must be 4-byte and counts / per_step 8-byte aligned");
     return cuda_rc(bezk::launch_player_outcome_update(partials, steps, n, bezk::outcome_classes(task), games_num, counts, per_step,
                                                       (cudaStream_t)stream), "bezk_player_outcome_update");
+}
+
+int bezk_reward_terms(int task) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    return bezk::reward_terms(task);
+}
+
+int bezk_reward_terms_update(const double* partials, int steps, int64_t n, int task, double* mean_k, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(partials && mean_k, "partials / mean_k NULL");
+    if (!ALIGNED(partials, 8) || !ALIGNED(mean_k, 8)) return fail(BEZK_E_ALIGN, "partials / mean_k must be 8-byte aligned");
+    return cuda_rc(bezk::launch_reward_terms_update(partials, steps, n, bezk::reward_terms(task), mean_k, (cudaStream_t)stream),
+                   "bezk_reward_terms_update");
 }
 
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream) {

@@ -83,6 +83,19 @@ struct OutArgs {
     int32_t* partials;           // (K, W): per warp of 32 envs the count of its done envs whose episode ended through class k
     int64_t w;                   // W
 };
+// Reward terms: the reward each env received this step split into additive pieces -- the shaping terms of the branch it took
+// (0 for the pieces of the other branch) and, last, the termination override (0 when no rule fired; then every shaping term is 0).
+// BezKick: ball velocity, approach, height, body velocity, posture, termination; walk: goal velocity, uprightness, body velocity,
+// posture, termination; orient: heading, uprightness, body velocity, posture, termination.
+enum { KICK_TERMS = 6, WALK_TERMS = 5 };
+__host__ __device__ constexpr int reward_terms(int task) { return task == BEZK_TASK_KICK ? (int)KICK_TERMS : (int)WALK_TERMS; }
+// Per-warp reward term sums of the fused step (bezk_post_physics_rollout_ep_terms).  A separate kernel parameter of
+// task_tile_terms_kernel / task_tile_outcome_terms_kernel (and their _l2 forms), appended after EpArgs (and OutArgs), for the reason
+// EpArgs is one.
+struct TermArgs {
+    double* partials;            // (K, W): per warp of 32 envs the fp64 sum of term k over its envs
+    int64_t w;                   // W
+};
 // fills l2_resident (bezk_task.cu): after fill_alignment, before the launch; ep: the armed episode accumulators or nullptr
 void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a, const EpArgs* ep = nullptr);
 // demote [ptr, ptr + bytes) to the normal L2 eviction priority (the 128-byte lines entirely inside the range)
@@ -102,9 +115,10 @@ struct PpoArgs {
 // the tile kernel for (task, parts): kick takes parts 1..7, walk / orient 2, 3, 4 or 7; ep (the episode accumulators,
 // task_tile_ep_kernel / task_tile_ep_l2_kernel) only with parts = 7; nm (the observation normaliser, task_tile_obsnorm_kernel /
 // task_tile_obsnorm_l2_kernel) and oa (the outcome counts, task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel) only
-// together with ep.  cudaErrorInvalidValue for any other combination.
+// together with ep; ta (the reward terms, task_tile_terms_kernel / task_tile_outcome_terms_kernel) only together with ep and
+// without nm.  cudaErrorInvalidValue for any other combination.
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
-                        const NormArgs* nm = nullptr, const OutArgs* oa = nullptr);
+                        const NormArgs* nm = nullptr, const OutArgs* oa = nullptr, const TermArgs* ta = nullptr);
 // folds `steps` x (3, ceil(n / 32)) partials of launch_task's episode accumulators into the two AverageMeters (bezk_rollout.cu)
 cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                                         int64_t* size2, cudaStream_t st);
@@ -119,6 +133,8 @@ cudaError_t launch_outcome_meter_update(const int32_t* partials, int steps, int6
 // folds the same partials into [games_counted, count_0 .. count_{K-1}] with player_tally_kernel's cutoff (bezk_rollout.cu)
 cudaError_t launch_player_outcome_update(const int32_t* partials, int steps, int64_t n, int k, int64_t games_num, double* counts,
                                          double* per_step, cudaStream_t st);
+// folds `steps` x (K, ceil(n / 32)) reward term partials into the (K,) means per env-step over steps x n (bezk_rollout.cu)
+cudaError_t launch_reward_terms_update(const double* partials, int steps, int64_t n, int k, double* mean_k, cudaStream_t st);
 cudaError_t launch_goal_uniforms(uint64_t seed, uint64_t step, float* out2, cudaStream_t st);
 void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg);
 cudaError_t stage_feet_gather(const float*, const BezkTaskCfg&, float*, int64_t, int64_t, cudaStream_t);

@@ -892,4 +892,69 @@ cudaError_t launch_player_outcome_update(const int32_t* partials, int steps, int
     return e != cudaSuccess ? e : f;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Reward terms: the per-step (K, W) fp64 reward term partials of the fused step (per warp of 32 envs the sum of term k over its
+// envs) folded into the (K,) means per env-step, sum over steps x W slots / (steps * n).  CTA (t, k) sums step t's W slots of term
+// k -- thread i adds slots i, i + 256, ... in order, then a shuffle-down tree (16, 8, 4, 2, 1) per warp and the 8 warp sums in
+// order -- and the last CTA to finish (ticket) adds each term's step sums in step order and divides: the same bits every run,
+// restated in tests/test_reward_terms.py.  Scratch from stream-ordered allocation, no host synchronisation: capturable in a graph.
+// ------------------------------------------------------------------------------------------------
+constexpr int RT_THREADS = 256;
+constexpr int RT_WARPS = RT_THREADS / 32;
+
+struct RtScratch {
+    double* step_sums;     // (K, steps)
+    unsigned* ticket;      // zeroed
+};
+
+__global__ void __launch_bounds__(RT_THREADS) reward_terms_kernel(const double* __restrict__ partials, int steps, int64_t w,
+                                                                  int64_t n, RtScratch sc, double* mean_k) {
+    __shared__ double s_warp[RT_WARPS];
+    __shared__ int s_last;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int step = blockIdx.x, k = blockIdx.y, nk = gridDim.y;
+    pdl_launch_dependents();
+    pdl_wait();
+    const double* p = partials + ((int64_t)step * nk + k) * w;
+    double acc = 0.0;
+    for (int64_t i = threadIdx.x; i < w; i += RT_THREADS) acc += p[i];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
+    if (lane == 0) s_warp[warp] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double v = 0.0;
+#pragma unroll
+        for (int j = 0; j < RT_WARPS; ++j) v += s_warp[j];
+        sc.step_sums[(int64_t)k * steps + step] = v;
+        __threadfence();
+        s_last = atomicAdd(sc.ticket, 1u) == (unsigned)steps * nk - 1;
+    }
+    __syncthreads();
+    if (!s_last || threadIdx.x >= nk) return;
+    // the last CTA: thread c adds term c's step sums in step order
+    __threadfence();
+    double v = 0.0;
+    for (int t = 0; t < steps; ++t) v += __ldcg(sc.step_sums + (int64_t)threadIdx.x * steps + t);
+    mean_k[threadIdx.x] = v / ((double)steps * (double)n);
+}
+
+cudaError_t launch_reward_terms_update(const double* partials, int steps, int64_t n, int k, double* mean_k, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    if (k < 1 || k > RT_THREADS) return cudaErrorInvalidValue;
+    const size_t bytes = (size_t)k * steps * sizeof(double) + sizeof(unsigned);
+    void* buf = nullptr;
+    cudaError_t e = cudaMallocAsync(&buf, bytes, st);
+    if (e != cudaSuccess) return e;
+    RtScratch sc;
+    sc.step_sums = static_cast<double*>(buf);
+    sc.ticket = reinterpret_cast<unsigned*>(sc.step_sums + (size_t)k * steps);
+    e = cudaMemsetAsync(sc.ticket, 0, sizeof(unsigned), st);
+    if (e == cudaSuccess)
+        e = launch_ex(reward_terms_kernel, dim3((unsigned)steps, (unsigned)k), dim3(RT_THREADS), 0, st, partials, steps, (n + 31) / 32,
+                      n, sc, mean_k);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
 }  // namespace bezk

@@ -271,20 +271,27 @@ __device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs
 __device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs& nm, const OutArgs&) { return nm; }
 __device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const OutArgs& oa) { return oa; }
 __device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const NormArgs&, const OutArgs& oa) { return oa; }
+__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const TermArgs&) { return ep; }
+__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const OutArgs&, const TermArgs&) { return ep; }
+__device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const OutArgs& oa, const TermArgs&) { return oa; }
+__device__ __forceinline__ const TermArgs& terms_of(const EpArgs&, const TermArgs& ta) { return ta; }
+__device__ __forceinline__ const TermArgs& terms_of(const EpArgs&, const OutArgs&, const TermArgs& ta) { return ta; }
 template <typename T, typename... P>
 constexpr bool has_arg = (std::is_same<T, P>::value || ...);
 
 // Ep: empty, or one EpArgs -- then EP is on and the episode accumulators ride along (task_tile_ep_kernel / task_tile_ep_l2_kernel;
 // whole step only) -- or EpArgs and NormArgs: the eval-mode observation normaliser too (task_tile_obsnorm_kernel /
 // task_tile_obsnorm_l2_kernel).  Either EP pack may end in OutArgs: the per-warp episode outcome counts too
-// (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms).  A parameter pack rather than always-present
-// arguments: the kernels without accumulators make exactly the call they made before the accumulators existed (an unused EpArgs
-// argument alone changes their register allocation).
+// (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms).  EpArgs (and OutArgs) may be followed by
+// TermArgs: the per-warp reward term sums too (task_tile_terms_kernel / task_tile_outcome_terms_kernel and their _l2 forms).  A
+// parameter pack rather than always-present arguments: the kernels without accumulators make exactly the call they made before the
+// accumulators existed (an unused EpArgs argument alone changes their register allocation).
 template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H, typename... Ep>
 __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& cfg, const Ep&... eps) {
     constexpr bool EP = sizeof...(Ep) >= 1;
     constexpr bool NORM = has_arg<NormArgs, Ep...>;
     constexpr bool OUT = has_arg<OutArgs, Ep...>;
+    constexpr bool TERMS = has_arg<TermArgs, Ep...>;
     static_assert(!EP || PARTS == 7, "the episode accumulators ride in the whole step");
     constexpr int ROOT_ROW = root_row(TASK);
     constexpr int OBS_ROW = obs_row(TASK);
@@ -344,6 +351,7 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     bool ep_done = false;                  // this env's episode ended in this step, with return ep_r and length ep_l
     float ep_r = 0.0f, ep_l = 0.0f;
     int ep_oc = OUTCOME_NONE;              // OUT: the rule that ended it (the outcome class), from the reward call whose rew is stored
+    float tm[reward_terms(TASK)] = {};     // TERMS: this env's reward terms, from the same call (0 in lanes past the last env)
 
 
     // ---- 2. dense tiles: TMA bulk copies (full sub-tiles) or cooperative coalesced loads (tail) ----
@@ -593,19 +601,21 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
             for (int k = 0; k < 3; ++k) { s.v[k] = v[k]; s.w[k] = w[k]; }
             s.pos_sq = pos_sq;
             Mth<true> mr;
-            reward_term<true, OUT>(s, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc);
+            reward_term<true, OUT, TERMS>(s, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
             if (mr.bad()) {
                 Mth<false> mp;
-                reward_term<false, OUT>(s, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc);
+                reward_term<false, OUT, TERMS>(s, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
             }
         } else {
             Mth<true> mr;
-            if (TASK == BEZK_TASK_WALK) reward_walk<true, OUT>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc);
-            else reward_orient<true, OUT>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc);
+            if (TASK == BEZK_TASK_WALK)
+                reward_walk<true, OUT, TERMS>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
+            else reward_orient<true, OUT, TERMS>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
             if (mr.bad()) {
                 Mth<false> mp;
-                if (TASK == BEZK_TASK_WALK) reward_walk<false, OUT>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc);
-                else reward_orient<false, OUT>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc);
+                if (TASK == BEZK_TASK_WALK)
+                    reward_walk<false, OUT, TERMS>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
+                else reward_orient<false, OUT, TERMS>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
             }
         }
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
@@ -645,6 +655,17 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
                 if (lane == k) mine = m;
             }
             if (lane < K) oa.partials[lane * oa.w + e0 / WT] = __popc(mine);
+        }
+        if constexpr (TERMS) {
+            // ... and the fp64 sum of each reward term over its envs at (k, env / 32), with the same fixed-order tree
+            const TermArgs& ta = terms_of(eps...);
+#pragma unroll
+            for (int k = 0; k < reward_terms(TASK); ++k) {
+                double s = (double)tm[k];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+                if (lane == 0) ta.partials[k * ta.w + e0 / WT] = s;
+            }
         }
     }
 
@@ -767,6 +788,29 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_o
     const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg, const EpArgs ep, const NormArgs nm, const OutArgs oa) {
     task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, nm, oa);
 }
+// the EP and the EP + outcome steps that also sum their envs' reward terms per warp (bezk_post_physics_rollout_ep_terms)
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_terms_kernel(const TaskArgs a,
+                                                                                            const __grid_constant__ BezkTaskCfg cfg,
+                                                                                            const EpArgs ep, const TermArgs ta) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, ep, ta);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_terms_l2_kernel(const TaskArgs a,
+                                                                                               const __grid_constant__ BezkTaskCfg cfg,
+                                                                                               const EpArgs ep, const TermArgs ta) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, ta);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_outcome_terms_kernel(
+    const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg, const EpArgs ep, const OutArgs oa, const TermArgs ta) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, ep, oa, ta);
+}
+template <bool CLEATS, int TILE, int TASK>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_outcome_terms_l2_kernel(
+    const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg, const EpArgs ep, const OutArgs oa, const TermArgs ta) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, oa, ta);
+}
 
 // ------------------------------------------------------------------------------------------------
 // K3 (function level): reset_idx over an explicit id list; one thread per (id, dof) pair + root rows.
@@ -821,15 +865,20 @@ static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>
 
 // Ep: empty (task_tile_kernel / task_tile_l2_kernel), the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel) or
 // those and the observation normaliser (task_tile_obsnorm_kernel / task_tile_obsnorm_l2_kernel), either EP pack followed by the
-// outcome counts (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms); a.l2_resident picks the L2
+// outcome counts (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms), the EP or EP + outcome pack
+// followed by the reward terms (task_tile_terms_kernel / task_tile_outcome_terms_kernel and their _l2 forms); a.l2_resident picks the L2
 // variant.  Every variant has the same shared memory: the normaliser works in the observation tile.
 template <int PARTS, bool CLEATS, int TILE, int TASK, typename... Ep>
 static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st, const Ep&... eps) {
     static_assert(sizeof...(Ep) == 0 || PARTS == 7, "the episode accumulators ride in the whole step");
     const auto kernel = [&] {
-        constexpr bool NORM = has_arg<NormArgs, Ep...>, OUT = has_arg<OutArgs, Ep...>;
+        constexpr bool NORM = has_arg<NormArgs, Ep...>, OUT = has_arg<OutArgs, Ep...>, TERMS = has_arg<TermArgs, Ep...>;
         if constexpr (sizeof...(Ep) == 0)
             return a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
+        else if constexpr (TERMS && OUT)
+            return a.l2_resident ? task_tile_outcome_terms_l2_kernel<CLEATS, TILE, TASK> : task_tile_outcome_terms_kernel<CLEATS, TILE, TASK>;
+        else if constexpr (TERMS)
+            return a.l2_resident ? task_tile_terms_l2_kernel<CLEATS, TILE, TASK> : task_tile_terms_kernel<CLEATS, TILE, TASK>;
         else if constexpr (NORM && OUT)
             return a.l2_resident ? task_tile_obsnorm_outcome_l2_kernel<CLEATS, TILE, TASK> : task_tile_obsnorm_outcome_kernel<CLEATS, TILE, TASK>;
         else if constexpr (OUT)
@@ -851,14 +900,21 @@ template <int V>
 using Int = std::integral_constant<int, V>;
 
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
-                        const NormArgs* nm, const OutArgs* oa) {
+                        const NormArgs* nm, const OutArgs* oa, const TermArgs* ta) {
     const bool cleats = (cfg.flags & BEZK_F_CLEATS) != 0;
-    if ((nm || oa) && !ep) return cudaErrorInvalidValue;
+    if ((nm || oa || ta) && !ep) return cudaErrorInvalidValue;
+    if (ta && nm) return cudaErrorInvalidValue;
     // one (TASK, PARTS) pair, with or without cleats; the episode accumulators (and the normaliser / outcome counts) only with the
     // whole step
     const auto tile = [&](auto task_c, auto parts_c) -> cudaError_t {
         constexpr int TASK = decltype(task_c)::value, PARTS = decltype(parts_c)::value;
         if constexpr (PARTS == 7) {
+            if (ta && oa)
+                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa, *ta)
+                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa, *ta);
+            if (ta)
+                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *ta)
+                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *ta);
             if (nm && oa)
                 return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm, *oa)
                               : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm, *oa);

@@ -119,14 +119,15 @@ __device__ __forceinline__ WalkTerms walk_terms(const float (&q)[4], const float
 // functions below.
 constexpr int OUTCOME_NONE = -1;
 
-// shared tail of the two reward functions: fall, win state, (task rule), horizon.  OC: also the outcome class into *oc_out.
-template <bool OC = false>
+// shared tail of the two reward functions: fall, win state, (task rule), horizon.  OC: also the outcome class into *oc_out.  TM:
+// tm_out holds the caller's 4 shaping terms; they become 0 when a rule fired, and tm_out[4] gets the override (0 otherwise).
+template <bool OC = false, bool TM = false>
 __device__ __forceinline__ void walk_tail(const WalkTerms& t, bool close, float rew, bool out_rule, float out_value, const BezkTaskCfg& c,
                                           int64_t progress, int64_t reset_cur, float* rew_out, int64_t* reset_out,
-                                          int* oc_out = nullptr) {
+                                          int* oc_out = nullptr, float* tm_out = nullptr) {
     int64_t reset = reset_cur;
     int oc = OUTCOME_NONE;
-    if (t.up_proj < 0.7f) { reset = 1; rew = -100.0f; if constexpr (OC) oc = WALK_FELL; }       // fall
+    if (t.up_proj < 0.7f) { reset = 1; rew = -100.0f; if constexpr (OC || TM) oc = WALK_FELL; }       // fall
     float state = close ? 1.0f : 0.0f;
     if (t.pos < 0.15f) state += 1.0f;
     if (t.vel_ang < 0.1f) state += 1.0f;
@@ -134,21 +135,28 @@ __device__ __forceinline__ void walk_tail(const WalkTerms& t, bool close, float 
     if (state == 4.0f) {                                                                          // win state
         reset = 1;
         rew = 1.0f * (1000.0f - 1000.0f * ((float)progress / (float)c.max_episode_length));
-        if constexpr (OC) oc = WALK_REACHED;
+        if constexpr (OC || TM) oc = WALK_REACHED;
     }
-    if (out_rule) { reset = 1; rew = out_value; if constexpr (OC) oc = WALK_OUT; }               // out of bound
-    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; if constexpr (OC) oc = WALK_TIMEOUT; }   // horizon
+    if (out_rule) { reset = 1; rew = out_value; if constexpr (OC || TM) oc = WALK_OUT; }               // out of bound
+    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; if constexpr (OC || TM) oc = WALK_TIMEOUT; }   // horizon
     *rew_out = rew;
     *reset_out = reset;
     if constexpr (OC) *oc_out = oc;
+    if constexpr (TM) {
+        const bool fired = oc != OUTCOME_NONE;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) tm_out[k] = fired ? 0.0f : tm_out[k];
+        tm_out[4] = fired ? rew : 0.0f;
+    }
 }
 
-// compute_bez_reward of tasks/walk_env.py:827-997 (debug prints and dead terms dropped)
-template <bool F, bool OC = false>
+// compute_bez_reward of tasks/walk_env.py:827-997 (debug prints and dead terms dropped).  TM: also the WALK_TERMS reward terms
+// into tm_out (goal velocity, uprightness, body velocity, posture, termination).
+template <bool F, bool OC = false, bool TM = false>
 __device__ __forceinline__ void reward_walk(const float (&bez)[3], const float (&q)[4], const float (&v)[3], const float (&w)[3],
                                             float pos_sq, const float (&goal)[2], const BezkTaskCfg& c, int64_t progress,
                                             int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m,
-                                            int* oc_out = nullptr) {
+                                            int* oc_out = nullptr, float* tm_out = nullptr) {
     const float dx = goal[0] - bez[0], dy = goal[1] - bez[1];
     const float n_goal = m.sqr(dx * dx + dy * dy);
     const float ux = m.div(dx, n_goal), uy = m.div(dy, n_goal);
@@ -166,15 +174,22 @@ __device__ __forceinline__ void reward_walk(const float (&bez)[3], const float (
     const float ang_now = atan2f_z(uy, ux);
     const float ang_init = atan2f_z(m.div(iy, n_i), m.div(ix, n_i));
     const bool out = fabsf(ang_init - ang_now) > 1.5708f;
-    walk_tail<OC>(t, close, rew, out, -100.0f, c, progress, reset_cur, rew_out, reset_out, oc_out);
+    if constexpr (TM) {
+        tm_out[0] = close ? 0.0f : vel_fwd * 10.0f;
+        tm_out[1] = -dist_h;
+        tm_out[2] = close ? -vel_s : 0.0f;
+        tm_out[3] = close ? -pos_s : -(5.0f * pos_s);
+    }
+    walk_tail<OC, TM>(t, close, rew, out, -100.0f, c, progress, reset_cur, rew_out, reset_out, oc_out, tm_out);
 }
 
-// compute_bez_reward of tasks/orient_env.py:845-1014
-template <bool F, bool OC = false>
+// compute_bez_reward of tasks/orient_env.py:845-1014.  TM: also the WALK_TERMS reward terms into tm_out (heading, uprightness,
+// body velocity, posture, termination).
+template <bool F, bool OC = false, bool TM = false>
 __device__ __forceinline__ void reward_orient(const float (&bez)[3], const float (&q)[4], const float (&v)[3], const float (&w)[3],
                                               float pos_sq, float goal_angle, const BezkTaskCfg& c, int64_t progress,
                                               int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m,
-                                              int* oc_out = nullptr) {
+                                              int* oc_out = nullptr, float* tm_out = nullptr) {
     const float ang = angle_to_goal(q, goal_angle);
     const WalkTerms t = walk_terms(q, v, w, pos_sq, m);
     const float dist_h = fabsf(1.0f - t.up_proj);
@@ -185,7 +200,13 @@ __device__ __forceinline__ void reward_orient(const float (&bez)[3], const float
     const float rew = close ? height_vel_pos : vel_height;
     const float tx = bez[0] - c.bez_init_xy[0], ty = bez[1] - c.bez_init_xy[1];
     const bool out = m.sqr(tx * tx + ty * ty) > 0.3f;
-    walk_tail<OC>(t, close, rew, out, -5.0f, c, progress, reset_cur, rew_out, reset_out, oc_out);
+    if constexpr (TM) {
+        tm_out[0] = close ? 0.0f : fabsf(ang) * -0.5f;
+        tm_out[1] = -dist_h;
+        tm_out[2] = close ? -vel_s : 0.0f;
+        tm_out[3] = close ? -pos_s : -(0.05f * pos_s);
+    }
+    walk_tail<OC, TM>(t, close, rew, out, -5.0f, c, progress, reset_cur, rew_out, reset_out, oc_out, tm_out);
 }
 
 struct RewardIn {
@@ -199,11 +220,12 @@ struct RewardIn {
 };
 
 // compute_bez_reward, kick_env.py:1224-1395 (SURVEY A.1).  `progress` is the post-increment value.  OC: also the outcome class
-// into *oc_out.
-template <bool F, bool OC = false>
+// into *oc_out.  TM: also the KICK_TERMS reward terms into tm_out (ball velocity, approach, height, body velocity, posture,
+// termination).
+template <bool F, bool OC = false, bool TM = false>
 __device__ __forceinline__ void reward_term(const RewardIn& s, const BezkTaskCfg& c, int64_t progress,
                                             int64_t reset_cur, float* rew_out, int64_t* reset_out, Mth<F>& m,
-                                            int* oc_out = nullptr) {
+                                            int* oc_out = nullptr, float* tm_out = nullptr) {
     const float dbx = s.ball_xy[0] - s.bez[0], dby = s.ball_xy[1] - s.bez[1];
     const float nbb = m.sqr(dbx * dbx + dby * dby);
     const float vel_fwd = m.div(dbx, nbb) * s.v[0] + m.div(dby, nbb) * s.v[1];
@@ -234,19 +256,28 @@ __device__ __forceinline__ void reward_term(const RewardIn& s, const BezkTaskCfg
     int64_t reset = reset_cur;
     int oc = OUTCOME_NONE;
 
-    if (s.bez[2] < 0.275f) { reset = 1; rew = -1.0f; if constexpr (OC) oc = KICK_FELL; }                 // rule 1
+    if (s.bez[2] < 0.275f) { reset = 1; rew = -1.0f; if constexpr (OC || TM) oc = KICK_FELL; }                 // rule 1
     const float tx = s.bez[0] - c.bez_init_xy[0], ty = s.bez[1] - c.bez_init_xy[1];
-    if (m.sqr(tx * tx + ty * ty) > 0.5f) { reset = 1; rew = -1.0f; if constexpr (OC) oc = KICK_STRAYED; }   // rule 2
-    if (angle_diff > 1.5708f) { reset = 1; rew = -1.0f; if constexpr (OC) oc = KICK_WIDE; }                // rule 3
+    if (m.sqr(tx * tx + ty * ty) > 0.5f) { reset = 1; rew = -1.0f; if constexpr (OC || TM) oc = KICK_STRAYED; }   // rule 2
+    if (angle_diff > 1.5708f) { reset = 1; rew = -1.0f; if constexpr (OC || TM) oc = KICK_WIDE; }                // rule 3
     if (n_goal < 0.05f) {                                                                                // rule 4
         reset = 1;
         rew = 1.0f * (100.0f - 100.0f * ((float)progress / (float)c.max_episode_length));
-        if constexpr (OC) oc = KICK_SCORED;
+        if constexpr (OC || TM) oc = KICK_SCORED;
     }
-    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; if constexpr (OC) oc = KICK_TIMEOUT; }   // rule 5
+    if (progress >= (int64_t)c.max_episode_length) { reset = 1; rew = 0.0f; if constexpr (OC || TM) oc = KICK_TIMEOUT; }   // rule 5
     *rew_out = rew;
     *reset_out = reset;
     if constexpr (OC) *oc_out = oc;
+    if constexpr (TM) {
+        const bool fired = oc != OUTCOME_NONE, far = kicked > 0.3f;
+        tm_out[0] = fired ? 0.0f : ball_fwd * 0.1f;
+        tm_out[1] = (fired || far) ? 0.0f : vel_fwd * 0.05f;
+        tm_out[2] = fired ? 0.0f : -height;
+        tm_out[3] = (fired || !far) ? 0.0f : -vel_r;
+        tm_out[4] = (fired || !far) ? 0.0f : -pos_r;
+        tm_out[5] = fired ? rew : 0.0f;
+    }
 }
 
 // rl_games play_steps reward path (a2c_common.py play_steps + tr_helpers.DefaultRewardsShaper; cfg/train/bez_kickPPO.yaml:53-56):

@@ -22,7 +22,7 @@ from torch import nn
 
 from .. import dist as bdist
 from . import a2c_common, experience, losses
-from .episode_meter import EpisodeMeter, OutcomeMeter
+from .episode_meter import EpisodeMeter, OutcomeMeter, RewardTerms
 from .policy_head import policy_head as _policy_head
 from .running_mean_std import RunningMeanStd
 
@@ -75,6 +75,9 @@ TRAIN_DEFAULTS = dict(games_to_track=100, save_best_after=100, save_frequency=0,
 #: this project's own options (not rl_games settings): ``track_outcomes`` -- count how each episode ended (the env's ``OUTCOMES``)
 #: in the step kernel, into the ``game_outcomes`` meter and an ``outcomes`` entry of each ``train()`` history row
 OUTCOME_DEFAULTS = dict(track_outcomes=False)
+#: this project's own option: ``track_reward_terms`` -- sum each of the env's ``REWARD_TERMS`` in the step kernel and add a
+#: ``reward_terms`` entry (term name -> mean per env-step of the epoch's rollout) to each ``train()`` history row
+REWARD_TERM_DEFAULTS = dict(track_reward_terms=False)
 
 
 class A2CAgent:
@@ -85,7 +88,7 @@ class A2CAgent:
         ``global_advantage_stats``) the advantage moments all use the same group, so a rank-0 checkpoint carries the
         statistics of every shard.  Pass ``env.env_base`` = the rank's shard offset (``cfg['env']['envBase']``) so that the
         reset / exploration noise is keyed by global env ids."""
-        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS, **OUTCOME_DEFAULTS)
+        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS, **OUTCOME_DEFAULTS, **REWARD_TERM_DEFAULTS)
         cfg.update(config or {})
         process_group = bdist.resolve_group(process_group)
         self.config, self.env, self.group = cfg, env, process_group
@@ -142,6 +145,11 @@ class A2CAgent:
         if self.track_outcomes:
             self._oc_partials = torch.zeros(T, len(env.OUTCOMES), (N + 31) // 32, dtype=torch.int32, device=self.device)
             self.game_outcomes = OutcomeMeter(env.OUTCOMES, int(cfg["games_to_track"]), self.device)
+        # track_reward_terms: the per-step reward term partials (term sums per 32 envs) and their per-rollout means
+        self.track_reward_terms = bool(cfg["track_reward_terms"])
+        if self.track_reward_terms:
+            self._rt_partials = torch.zeros(T, len(env.REWARD_TERMS), (N + 31) // 32, dtype=torch.float64, device=self.device)
+            self.reward_terms = RewardTerms(env.REWARD_TERMS, self.device)
         self.obs = env.reset()["obs"].clone()
         self.dones = torch.zeros(N, dtype=torch.uint8, device=self.device)
         self.dataset = None
@@ -187,7 +195,8 @@ class A2CAgent:
                                         scale_value=shaper.get("scale_value", 1.0), shift_value=shaper.get("shift_value", 0.0),
                                         value_bootstrap=self.config["value_bootstrap"], episode_returns=self.current_rewards,
                                         episode_lengths=self.current_lengths, episode_partials=self._ep_partials[t],
-                                        episode_outcomes=self._oc_partials[t] if self.track_outcomes else None)
+                                        episode_outcomes=self._oc_partials[t] if self.track_outcomes else None,
+                                        reward_terms=self._rt_partials[t] if self.track_reward_terms else None)
                 if head_targets:
                     env.step_precomputed_targets(res["env_actions"])
                 else:
@@ -196,6 +205,8 @@ class A2CAgent:
             self.game_rewards.update(self._ep_partials, self.num_actors)      # both meters, the T steps in order
             if self.track_outcomes:
                 self.game_outcomes.update(self._oc_partials, self.num_actors)
+            if self.track_reward_terms:
+                self.reward_terms.update(self._rt_partials, self.num_actors)
             _, last_v = self._forward(self._norm_obs(self.obs))
             last_values = self.value_mean_std(last_v, unnorm=True) if self.config["normalize_value"] else last_v
             a2c_common.discount_values(self.dones, last_values, buf.tensor_dict["dones"], buf.tensor_dict["values"], self.mb_rewards,
@@ -332,7 +343,8 @@ class A2CAgent:
         are per rank, as in rl_games.  Deviation: rank 0 broadcasts its stop decision every epoch, so every rank leaves on the
         same epoch (in rl_games the other ranks would wait in the next epoch's collectives).  Returns ``(last_mean_rewards,
         epoch)`` and a per-epoch history (mean return / length or None before the first finished game, losses, lr; with
-        ``track_outcomes`` also ``outcomes``: outcome name -> share of the tracked games, None before the first finished game)."""
+        ``track_outcomes`` also ``outcomes``: outcome name -> share of the tracked games, None before the first finished game; with
+        ``track_reward_terms`` also ``reward_terms``: term name -> mean per env-step of the epoch's rollout, on this rank's envs)."""
         cfg = self.config
         rank0 = not bdist.is_distributed(self.group) or torch.distributed.get_rank() == 0
         if rank0:
@@ -345,6 +357,8 @@ class A2CAgent:
                        kl=float(info["kl"]), lr=float(info["lr"]))
             if self.track_outcomes:
                 row["outcomes"] = None
+            if self.track_reward_terms:
+                row["reward_terms"] = self.reward_terms.as_dict()
             should_exit = False
             if rank0:
                 if self.game_rewards.current_size > 0:

@@ -89,3 +89,34 @@ class OutcomeMeter:
     def clear(self):
         self._mean.zero_()
         self._size.zero_()
+
+
+class RewardTerms:
+    """The mean per env-step of each reward term ``names`` (the env's ``REWARD_TERMS``) over the last folded rollout, an fp64 (K,)
+    vector on the device: ``update`` folds the fused step's per-warp term sums (``KickEnv.set_rollout_targets(reward_terms=...)``)
+    of T steps over N envs into sum / (T * N) with one launch and no host synchronisation.  Summed over the terms it is the
+    rollout's mean unshaped reward."""
+
+    def __init__(self, names, device="cuda"):
+        from ..tasks import KickEnv, OrientEnv, WalkEnv
+        self.names = tuple(names)
+        # the fold takes the task whose terms these are
+        tasks = {env.REWARD_TERMS: env.TASK for env in (KickEnv, WalkEnv, OrientEnv)}
+        if self.names not in tasks:
+            raise ValueError(f"names must be the REWARD_TERMS of an env: {', '.join(map(str, tasks))}")
+        self.task = tasks[self.names]
+        self.device = torch.device(device)
+        self._mean = torch.zeros(len(self.names), dtype=torch.float64, device=self.device)
+
+    def update(self, partials, num_envs):
+        """Fold (T, K, ceil(num_envs/32)) float64 term partials -- T consecutive steps -- into the means, replacing the last ones."""
+        ops.reward_terms_update(partials, num_envs, self.task, self._mean)
+
+    @property
+    def mean(self):
+        """(K,) float64 on the device."""
+        return self._mean
+
+    def as_dict(self):
+        """name -> mean per env-step, one device-to-host read."""
+        return dict(zip(self.names, self._mean.tolist()))

@@ -389,6 +389,61 @@ def player_outcome_update(partials, n, task, games_num, counts, per_step=None, s
                                               _cuda(counts, F64, "counts", 1 + k), ps, _stream(partials)), "bezk_player_outcome_update")
 
 
+def reward_terms(task):
+    """K, the number of reward terms of ``task`` (6 for ``"kick"``, 5 for ``"walk"`` / ``"orient"``; ``bezk_reward_terms``)."""
+    k = _lib.load().bezk_reward_terms(_TASK_ID[task])
+    if k == 10001:                                   # BEZK_E_BADARG
+        _lib.check(k, "bezk_reward_terms")
+    return k
+
+
+def post_physics_rollout_ep_terms(task, dof_state, rigid_body, root_states, net_contact, goal, initial_root_states, reset_buf,
+                                  progress_buf, timeout_buf, cfg, obs, rew, episode_returns, episode_lengths, episode_partials,
+                                  term_partials, outcome_partials=None, rollout_cfg=None, values=None, shaped_rewards=None,
+                                  dones_u8=None, goal_angle=None, ball_init=None, prev_lin_vel=None, uniforms=None, goal_uniforms=None,
+                                  seed=0, step=0, randomize_buf=None, obs_clipped=None, env_base=0):
+    """``post_physics_rollout_ep`` (or ``_ep_outcome`` when ``outcome_partials`` is given) that also writes the per-warp sum of
+    each reward term (``term_partials``, (K, ceil(N/32)) float64, CUDA; ``bezk_post_physics_rollout_ep_terms``)."""
+    n = progress_buf.shape[0]
+    nb = cfg.num_bodies
+    actors, _, width = bm.task_dims(task)
+    w = (n + 31) // 32
+    ret = _cuda(episode_returns, F32, "episode_returns", n)
+    length = _cuda(episode_lengths, F32, "episode_lengths", n)
+    part = _cuda(episode_partials, F64, "episode_partials", 3 * w)
+    tm = _cuda(term_partials, F64, "term_partials", reward_terms(task) * w)
+    oc = None if outcome_partials is None else _cuda(outcome_partials, I32, "outcome_partials", outcome_classes(task) * w)
+    lib = _lib.load()
+    _lib.check(lib.bezk_post_physics_rollout_ep_terms(
+        _TASK_ID[task], _p(dof_state, F32, "dof_state", n * 36), _p(rigid_body, F32, "rigid_body", n * nb * 13),
+        _p(root_states, F32, "root_states", n * actors * 13), _p(net_contact, F32, "net_contact", n * nb * 3),
+        _p(prev_lin_vel, F32, "prev_lin_vel", n * 3, True), _p(goal, F32, "goal", n * 2),
+        _p(goal_angle, F32, "goal_angle", n, True), _p(ball_init, F32, "ball_init", n * 2, True),
+        _p(initial_root_states, F32, "initial_root_states", n * actors * 13, True),
+        _p(uniforms, F32, "uniforms", n * 36, True), _p(goal_uniforms, F32, "goal_uniforms", 2, True), seed, step,
+        _p(reset_buf, I64, "reset_buf", n), _p(progress_buf, I64, "progress_buf", n),
+        _p(timeout_buf, I64, "timeout_buf", n), _p(randomize_buf, I64, "randomize_buf", n, True), C.byref(cfg),
+        _p(obs, F32, "obs", n * width), _p(obs_clipped, F32, "obs_clipped", n * width, True), _p(rew, F32, "rew", n),
+        C.byref(rollout_cfg) if rollout_cfg is not None else None, _p(values, F32, "values", n, True),
+        _p(shaped_rewards, F32, "shaped_rewards", n, True), _p(dones_u8, U8, "dones_u8", n, True), int(env_base), n,
+        ret, length, part, None, None, 0.0, None, oc, tm, _stream(dof_state)), "bezk_post_physics_rollout_ep_terms")
+
+
+def reward_terms_update(partials, n, task, mean_k, steps=None):
+    """Fold ``steps`` consecutive (K, ceil(n/32)) float64 reward term partials (``partials``: (steps, K, W) or (K, W)) into
+    ``mean_k`` ((K,) float64): each term's mean per env-step over the steps x n env-steps, on the device
+    (``bezk_reward_terms_update``)."""
+    k = reward_terms(task)
+    w = (int(n) + 31) // 32
+    if steps is None:
+        steps = partials.numel() // (k * w) if w else 0
+    if not isinstance(partials, torch.Tensor) or partials.numel() != int(steps) * k * w:
+        raise BezkError(f"partials must hold steps x {k} x {w} float64 values")
+    lib = _lib.load()
+    _lib.check(lib.bezk_reward_terms_update(_cuda(partials, F64, "partials", None), int(steps), int(n), _TASK_ID[task],
+                                            _cuda(mean_k, F64, "mean_k", k), _stream(partials)), "bezk_reward_terms_update")
+
+
 def reset_idx_task(task, env_ids, dof_state, root_states, initial_root_states, goal, progress, reset, cfg, uniforms=None,
                    goal_uniforms=None, seed=0, step=0, env_base=0):
     k = int(env_ids.numel())

@@ -55,6 +55,11 @@ class KickEnv(VecTask):
     #: the termination rule of ``compute_bez_reward`` whose reward a done env received -- the last one, in the reference's
     #: override order, whose condition held
     OUTCOMES = ("fell", "strayed", "wide", "scored", "timeout")
+    #: reward terms, in the order of the fused step's term sums (``set_rollout_targets(reward_terms=...)``): the reward an env
+    #: received split into additive pieces -- the shaping terms of the branch it took (0 for the other branch's pieces) and the
+    #: termination override (0 when no rule fired; then every shaping term is 0).  Ball velocity (ball_fwd * 0.1), approach
+    #: (vel_fwd * 0.05, near branch), height (-height), body velocity (-vel_r, far branch), posture (-pos_r, far branch)
+    REWARD_TERMS = ("ball_velocity", "approach", "height", "body_velocity", "posture", "termination")
     #: host pipelines (``sim.use_gpu_pipeline: False``), selected by ``env.hostPipeline``
     HOST_PIPELINES = ("zero_copy", "staged", "staged_ce", "staged_pack")
 
@@ -217,6 +222,7 @@ class KickEnv(VecTask):
         self._episode = None                # (episode_returns, episode_lengths, episode_partials) set by set_rollout_targets
         self._obs_norm = None               # (obs_mean, obs_var, obs_eps, obs_norm) set by set_rollout_targets
         self._outcomes = None               # (K, ceil(N/32)) int32 outcome partials set by set_rollout_targets
+        self._reward_terms = None           # (K, ceil(N/32)) float64 reward term partials set by set_rollout_targets
         self._d_values = None               # staged_ce host pipeline: device image of host-resident critic values
         self._lib = _lib.load()
         # the step keeps these in L2 with evict_last (bezk.h, bezk_l2_release): demoted again when the env goes away
@@ -519,6 +525,14 @@ class KickEnv(VecTask):
             if self._episode is not None:     # + rl_games' episode return / length bookkeeping (set_rollout_targets)
                 # + the eval-mode observation normaliser when armed (all NULL: exactly bezk_post_physics_rollout_ep)
                 mean, var, eps, out = self._obs_norm or (None, None, 0.0, None)
+                if self._reward_terms is not None:    # + the per-warp reward term sums (and the outcome counts when armed)
+                    rc = self._lib.bezk_post_physics_rollout_ep_terms(
+                        ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed, self._rng_step, t[0], t[1], t[2], t[3],
+                        t[4], t[5], t[6], t[7], *tail, self.env_base, self.num_envs, *[_ptr(x) for x in self._episode], None, None,
+                        0.0, None, _ptr(self._outcomes), _ptr(self._reward_terms), self._stream())
+                    if rc:
+                        _lib.check(rc, "bezk_post_physics_rollout_ep_terms")
+                    return
                 if self._outcomes is not None:    # + the per-warp episode outcome counts
                     rc = self._lib.bezk_post_physics_rollout_ep_outcome(
                         ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed, self._rng_step, t[0], t[1], t[2], t[3],
@@ -820,7 +834,7 @@ class KickEnv(VecTask):
 
     def set_rollout_targets(self, values=None, shaped_rewards=None, dones_u8=None, gamma=0.99, scale_value=0.01, shift_value=0.0,
                             value_bootstrap=True, episode_returns=None, episode_lengths=None, episode_partials=None, obs_norm=None,
-                            obs_mean=None, obs_var=None, obs_eps=1e-5, episode_outcomes=None):
+                            obs_mean=None, obs_var=None, obs_eps=1e-5, episode_outcomes=None, reward_terms=None):
         """Arm the reward epilogue of the fused step (SURVEY 8 a16; rl_games ``play_steps``): the NEXT steps also write
         ``shaped_rewards = (rew + shift) * scale + gamma * values * time_outs`` (e.g. ``mb_rewards[t]``) and the uint8 reset
         mask ``dones_u8`` (e.g. the experience buffer's ``dones`` slot ``t + 1``).  ``values``: the (N,)/(N,1) un-normalised
@@ -835,7 +849,10 @@ class KickEnv(VecTask):
         ``learner.PpoPlayerContinuous``' policy.
         ``episode_outcomes`` ((K, ceil(N/32)) int32, K = ``len(OUTCOMES)``), with the episode tensors armed, GPU pipeline only: the
         step also writes, per group of 32 envs, how many of its done envs ended through each class of ``OUTCOMES`` -- the input of
-        ``learner.OutcomeMeter`` and of the player's outcome counts.  Call with no arguments to disarm everything."""
+        ``learner.OutcomeMeter`` and of the player's outcome counts.
+        ``reward_terms`` ((K, ceil(N/32)) float64, K = ``len(REWARD_TERMS)``), with the episode tensors armed and without
+        ``obs_norm``, GPU pipeline only: the step also writes, per group of 32 envs, the sum of each of ``REWARD_TERMS`` over its envs
+        -- the input of ``learner.RewardTerms``.  Call with no arguments to disarm everything."""
         if self.fusion != "fused":
             raise NotImplementedError("the reward epilogue rides in the fused step (fusion='fused')")
         n, dev = self.num_envs, self.compute_device
@@ -867,6 +884,17 @@ class KickEnv(VecTask):
             t = episode_outcomes
             if t.dtype != torch.int32 or t.numel() != numel or not t.is_contiguous() or t.device != dev:
                 raise ValueError(f"episode_outcomes must be a contiguous torch.int32 tensor with {numel} elements on {dev}")
+        if reward_terms is not None:
+            if self.host_staged:
+                raise NotImplementedError("reward terms need the GPU pipeline")
+            if episode_returns is None:
+                raise ValueError("reward_terms needs the episode tensors (episode_returns, episode_lengths, episode_partials)")
+            if norm is not None:
+                raise ValueError("reward_terms and obs_norm are not armed together")
+            numel = len(self.REWARD_TERMS) * ((n + 31) // 32)
+            t = reward_terms
+            if t.dtype != torch.float64 or t.numel() != numel or not t.is_contiguous() or t.device != dev:
+                raise ValueError(f"reward_terms must be a contiguous torch.float64 tensor with {numel} elements on {dev}")
         eps = (episode_returns, episode_lengths, episode_partials)
         if any(t is not None for t in eps):
             if self.host_staged:
@@ -882,6 +910,7 @@ class KickEnv(VecTask):
             self._episode = None
         self._obs_norm = norm
         self._outcomes = episode_outcomes
+        self._reward_terms = reward_terms
         if shaped_rewards is None and dones_u8 is None:
             self._rollout = None
             return

@@ -18,6 +18,9 @@ from .walk_env import WalkEnv
 
 class OrientEnv(WalkEnv):
     TASK = "orient"
+    #: heading (|ang| * -0.5, not close), uprightness (-dist_h), body velocity (-vel_s, close only), posture (-pos_s close,
+    #: -(0.05 * pos_s) not close), termination
+    REWARD_TERMS = ("heading", "uprightness", "body_velocity", "posture", "termination")
 
     def _init_task_tensors(self, env_cfg, n, f32):
         super()._init_task_tensors(env_cfg, n, f32)

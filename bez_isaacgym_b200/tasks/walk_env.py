@@ -23,6 +23,9 @@ class WalkEnv(KickEnv):
     TASK = "walk"
     #: fell (up-vector projection < 0.7), reached (win state), out (out of bounds), timeout -- OrientEnv shares them
     OUTCOMES = ("fell", "reached", "out", "timeout")
+    #: the fused step's reward terms (``set_rollout_targets(reward_terms=...)``): goal velocity (vel_fwd * 10, not close),
+    #: uprightness (-dist_h), body velocity (-vel_s, close only), posture (-pos_s close, -(5 * pos_s) not close), termination
+    REWARD_TERMS = ("goal_velocity", "uprightness", "body_velocity", "posture", "termination")
 
     def _read_task_cfg(self, env_cfg):
         """No ball actor (walk_env.py:146-149); the yaml carries no ``ballInitState``."""

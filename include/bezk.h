@@ -460,6 +460,39 @@ int bezk_outcome_meter_update(const int32_t* partials, int steps, int64_t n, int
  * No host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op; games_num <= 0 is BEZK_E_BADARG. */
 int bezk_player_outcome_update(const int32_t* partials, int steps, int64_t n, int task, int64_t games_num, double* counts,
                                double* per_step, void* stream);
+/* Reward terms: the reward an env received in a step split into additive pieces.  Each shaping term is the fp32 value the step
+ * computes for that piece of compute_bez_reward's chosen branch (0 for the pieces of the branch not taken); the last term is the
+ * termination override when a rule fired (then every shaping term is 0, so the terms sum to rew exactly) and 0 otherwise (then
+ * they sum to rew up to fp32 re-association).  Terms, in index order:
+ *   BEZK_TASK_KICK (K = 6):    ball_velocity (ball_fwd * 0.1), approach (vel_fwd * 0.05, near branch), height (-height),
+ *                              body_velocity (-vel_r, far branch), posture (-pos_r, far branch), termination
+ *   BEZK_TASK_WALK (K = 5):    goal_velocity (vel_fwd * 10, not close), uprightness (-dist_h), body_velocity (-vel_s, close),
+ *                              posture (-pos_s close, -(5 * pos_s) not close), termination
+ *   BEZK_TASK_ORIENT (K = 5):  heading (|ang| * -0.5, not close), uprightness (-dist_h), body_velocity (-vel_s, close),
+ *                              posture (-pos_s close, -(0.05 * pos_s) not close), termination
+ * bezk_reward_terms returns K for a task, BEZK_E_BADARG for an unknown one. */
+int bezk_reward_terms(int task);
+/* bezk_post_physics_rollout_ep_outcome that also sums its envs' reward terms:
+ *   term_partials (K, W) f64 out, DEVICE memory, W = ceil(n / 32), 8-byte aligned: at [k * W + env / 32] the sum of term k over
+ *                 the envs of that group of 32 (a fixed-order shuffle tree: the same bits every run).  Every slot is written each
+ *                 step, so the buffer needs no zeroing.
+ * term_partials and the episode accumulators are required, outcome_partials is optional (NULL: no outcome counts) and the
+ * normaliser arguments must be NULL (BEZK_E_BADARG).  Every other output is the same bytes as without term_partials. */
+int bezk_post_physics_rollout_ep_terms(int task, float* dof_state, const float* rigid_body, float* root_states,
+                                       float* net_contact, float* prev_lin_vel, float* goal, const float* goal_angle,
+                                       const float* ball_init, const float* initial_root_states,
+                                       const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step,
+                                       int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                       int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped,
+                                       float* rew, const BezkRolloutCfg* rollout, const float* values,
+                                       float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                       float* ep_return, float* ep_length, double* ep_partials,
+                                       const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm,
+                                       int32_t* outcome_partials, double* term_partials, void* stream);
+/* The mean of each reward term per env-step over `steps` consecutive term_partials of n envs ((steps, K, ceil(n / 32)) f64):
+ * mean_k[k] = (sum of term k over the steps x n env-steps) / (steps * n), written to mean_k (K,) f64, DEVICE memory.  Fixed
+ * summation order (the same bits every run); no host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op. */
+int bezk_reward_terms_update(const double* partials, int steps, int64_t n, int task, double* mean_k, void* stream);
 /* bezk_reset_idx for any task: root rows are 13 floats for walk / orient, and their goal (n,2) rows are redrawn.
  * env_base: global id of local env 0 (Philox key = env_base + env id), as in bezk_post_physics_rollout. */
 int bezk_reset_idx_task(int task, const int64_t* env_ids, int64_t k, const float* uniforms, const float* goal_uniforms,
