@@ -181,7 +181,7 @@ __global__ void __launch_bounds__(FUSED_THREADS) fused_stats_kernel(const FusedR
         const double mu = S / B;
         const double var = (SS - S * mu) / (B - 1.0);
         s_stat[0] = (float)mu;
-        s_stat[1] = (float)sqrt(var > 0.0 ? var : 0.0) + 1e-8f;
+        s_stat[1] = (float)sqrt(var < 0.0 ? 0.0 : var) + 1e-8f;       // as adv_normalize_kernel: NaN passes, negatives are 0
     }
     __syncthreads();
 

@@ -570,15 +570,15 @@ cudaError_t launch_rms_moments(const float* x, const double* pivot, double* acc,
 }
 
 // The moments of n_batches equally spaced minibatches in ONE pair of launches (partials + fold, blockIdx.y = batch): batch b is
-// the slab view based at x + b * x_batch_rows * c; acc (n_batches, 1 + 2c).  Only the TMA path is batched; anything else falls
-// back to one launch_rms_moments per batch.
+// the slab view based at x + b * x_batch_rows * c; acc (n_batches, 1 + 2c).  Only the TMA path is batched, and only while every
+// batch gets at least one of the RMS_MAX_BLOCKS partial rows; anything else falls back to one launch_rms_moments per batch.
 cudaError_t launch_rms_moments_batched(const float* x, const double* pivot, double* acc, double* partials, int64_t m, int c,
                                        int64_t slab_rows, int64_t slab_stride, int64_t x_batch_rows, int n_batches, cudaStream_t st) {
     if (n_batches <= 0) return cudaSuccess;
     if (slab_rows <= 0 || slab_rows >= m) { slab_rows = m; slab_stride = m; }
     if (m % slab_rows != 0) return cudaErrorInvalidValue;
     const bool slabs = slab_rows < m;
-    const bool tma_ok = c > 1 && c <= RMS_MAX_C && n_batches <= 65535 && aligned16(x) && ((RMS_TR * c * 4) % 16 == 0) &&
+    const bool tma_ok = c > 1 && c <= RMS_MAX_C && n_batches <= RMS_MAX_BLOCKS && aligned16(x) && ((RMS_TR * c * 4) % 16 == 0) &&
                         (((m % RMS_TR) * c * 4) % 16 == 0) && m >= 4 * RMS_TR && ((x_batch_rows * c * 4) % 16 == 0) &&
                         (!slabs || (slab_rows % RMS_TR == 0 && (slab_stride * c * 4) % 16 == 0)) &&
                         (size_t)RMS_STAGES * RMS_TR * c * sizeof(float) <= 220 * 1024;
@@ -602,8 +602,7 @@ cudaError_t launch_rms_moments_batched(const float* x, const double* pivot, doub
     int64_t cap = 148LL * per_sm;
     if (cap > RMS_MAX_BLOCKS) cap = RMS_MAX_BLOCKS;
     int64_t per_batch = cap / n_batches;                 // the batches share the resident CTAs (and the partials scratch)
-    if (per_batch < 1) per_batch = 1;
-    if ((int64_t)n_batches * per_batch > RMS_MAX_BLOCKS) return cudaErrorInvalidValue;
+    if (per_batch < 1) per_batch = 1;                    // n_batches <= RMS_MAX_BLOCKS above: the partials still fit
     const int nblocks = (int)(ntiles < per_batch ? ntiles : per_batch);
     const dim3 grid((unsigned)nblocks, (unsigned)n_batches);
     cudaError_t err = slabs ? launch_pdl(learner_pdl(), rms_partials_tma_kernel<true>, grid, dim3(RMS_THREADS), smem, st, x, pivot, partials, m, c,
@@ -703,7 +702,8 @@ __global__ void __launch_bounds__(256) adv_normalize_kernel(const float* __restr
         const double mu = S / B;
         const double var = (SS - S * mu) / (B - 1.0);              // unbiased, torch.std default
         mean = (float)mu;
-        den = (float)sqrt(var > 0.0 ? var : 0.0) + 1e-8f;
+        // a rounding-negative variance is 0; a NaN one (B == 1) stays NaN, like torch.std
+        den = (float)sqrt(var < 0.0 ? 0.0 : var) + 1e-8f;
     }
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

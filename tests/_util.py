@@ -86,6 +86,36 @@ def assert_close(actual, expected, scale=None, rtol=RTOL, atol=ATOL, what=""):
                              f"first at {i}: got {actual[i].item()!r} want {expected[i].item()!r}")
 
 
+GUARD = 4096          # bytes each side
+
+
+class Guarded:
+    """Out-of-bounds WRITE canaries: every buffer ``make`` hands out lives between two guard bands filled with a sentinel;
+    ``check`` asserts that the bands came back untouched."""
+
+    def __init__(self):
+        self.bufs = []
+
+    def make(self, shape, dtype=torch.float32, fill=None):
+        numel = 1
+        for s in shape:
+            numel *= s
+        nbytes = numel * torch.empty((), dtype=dtype).element_size()
+        pad = (-nbytes) % 16
+        raw = torch.full((GUARD + nbytes + pad + GUARD,), 0x5A, dtype=torch.uint8, device="cuda")
+        view = raw[GUARD:GUARD + nbytes].view(dtype).view(shape)
+        if fill is not None:
+            view.copy_(fill)
+        self.bufs.append((raw, nbytes))
+        return view
+
+    def check(self):
+        torch.cuda.synchronize()
+        for raw, nbytes in self.bufs:
+            assert bool((raw[:GUARD] == 0x5A).all()), "write BEFORE an output buffer"
+            assert bool((raw[GUARD + nbytes:] == 0x5A).all()), "write PAST an output buffer"
+
+
 def ulp(x):
     return float(np.spacing(np.float32(x)))
 

@@ -5,33 +5,9 @@ import pytest
 import torch
 
 from bez_isaacgym_b200 import synthetic_gym as sg
+from tests._util import Guarded
 
 pytestmark = pytest.mark.gpu
-GUARD = 4096          # bytes each side
-
-
-class Guarded:
-    def __init__(self):
-        self.bufs = []
-
-    def make(self, shape, dtype=torch.float32, fill=None):
-        numel = 1
-        for s in shape:
-            numel *= s
-        nbytes = numel * torch.empty((), dtype=dtype).element_size()
-        pad = (-nbytes) % 16
-        raw = torch.full((GUARD + nbytes + pad + GUARD,), 0x5A, dtype=torch.uint8, device="cuda")
-        view = raw[GUARD:GUARD + nbytes].view(dtype).view(shape)
-        if fill is not None:
-            view.copy_(fill)
-        self.bufs.append((raw, nbytes))
-        return view
-
-    def check(self):
-        torch.cuda.synchronize()
-        for raw, nbytes in self.bufs:
-            assert bool((raw[:GUARD] == 0x5A).all()), "write BEFORE an output buffer"
-            assert bool((raw[GUARD + nbytes:] == 0x5A).all()), "write PAST an output buffer"
 
 
 @pytest.mark.parametrize("T,N,c", [(32, 4099, 54), (5, 37, 18), (33, 130, 1), (7, 3, 54)])

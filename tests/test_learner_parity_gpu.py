@@ -172,7 +172,9 @@ def test_advantage_normalisation(m):
 
 
 # ----------------------------------------------------------------------------------------------- PPO loss
-@pytest.mark.parametrize("m", [1, 127, 128, 4099, 32768])
+# 75777: CTAs of the 592-CTA persistent grid take a second tile (mbarrier phase flip, grad_mu store drained first);
+# 700001: CTA 140 takes 10 tiles -- a mid-loop fp32 -> fp64 flush after PPO_FLUSH = 8 and a ragged last tile
+@pytest.mark.parametrize("m", [1, 127, 128, 4099, 32768, 75777, 700001])
 @pytest.mark.parametrize("bound_form", ["v1.1.3", "outside"])
 def test_ppo_loss_forward_backward(m, bound_form):
     from oracle import rl_games_oracle as rg
