@@ -96,24 +96,30 @@ class Guarded:
     def __init__(self):
         self.bufs = []
 
-    def make(self, shape, dtype=torch.float32, fill=None):
+    def make(self, shape, dtype=torch.float32, fill=None, offset=0):
+        """``offset``: the view starts that many bytes past a 16-byte boundary (``data_ptr() % 16 == offset``), so that a
+        launcher which picks its memory path from pointer alignment takes its unaligned one; a multiple of the element size."""
+        esz = torch.empty((), dtype=dtype).element_size()
+        assert 0 <= offset < 16 and offset % esz == 0, f"offset {offset} is not a multiple of the {esz}-byte element"
         numel = 1
         for s in shape:
             numel *= s
-        nbytes = numel * torch.empty((), dtype=dtype).element_size()
-        pad = (-nbytes) % 16
-        raw = torch.full((GUARD + nbytes + pad + GUARD,), 0x5A, dtype=torch.uint8, device="cuda")
-        view = raw[GUARD:GUARD + nbytes].view(dtype).view(shape)
+        nbytes = numel * esz
+        pad = (-(offset + nbytes)) % 16
+        raw = torch.full((GUARD + offset + nbytes + pad + GUARD,), 0x5A, dtype=torch.uint8, device="cuda")
+        start = GUARD + offset
+        view = raw[start:start + nbytes].view(dtype).view(shape)
+        assert view.data_ptr() % 16 == offset
         if fill is not None:
             view.copy_(fill)
-        self.bufs.append((raw, nbytes))
+        self.bufs.append((raw, start, nbytes))
         return view
 
     def check(self):
         torch.cuda.synchronize()
-        for raw, nbytes in self.bufs:
-            assert bool((raw[:GUARD] == 0x5A).all()), "write BEFORE an output buffer"
-            assert bool((raw[GUARD + nbytes:] == 0x5A).all()), "write PAST an output buffer"
+        for raw, start, nbytes in self.bufs:
+            assert bool((raw[:start] == 0x5A).all()), "write BEFORE an output buffer"
+            assert bool((raw[start + nbytes:] == 0x5A).all()), "write PAST an output buffer"
 
 
 def ulp(x):
