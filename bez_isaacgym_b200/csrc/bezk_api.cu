@@ -83,7 +83,7 @@ static bezk::TaskArgs step_args(float* dof_state, const float* rigid_body, float
 
 static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* stream, const char* where, int task = BEZK_TASK_KICK,
                     bezk::EpArgs* ep = nullptr, const bezk::NormArgs* nm = nullptr, bezk::OutArgs* oa = nullptr,
-                    bezk::TermArgs* ta = nullptr) {
+                    bezk::TermArgs* ta = nullptr, bezk::GameTermArgs* ga = nullptr) {
     if (int rc = check_cfg(cfg)) return rc;
     REQUIRE(a.n >= 0, "n < 0");
     if (a.n == 0) return 0;
@@ -104,11 +104,12 @@ static int run_task(int parts, bezk::TaskArgs& a, const BezkTaskCfg* cfg, void* 
         if (cfg->flags & BEZK_F_RESET_ROOT_STATES) REQUIRE(a.initial_root, "initial_root_states NULL");
     }
     bezk::fill_alignment(a, *cfg);
-    bezk::set_l2_policy(task, cfg->flags, a, ep);
+    bezk::set_l2_policy(task, cfg->flags, a, ep, ga);
     if (ep) ep->w = (a.n + 31) / 32;
     if (oa) oa->w = (a.n + 31) / 32;
     if (ta) ta->w = (a.n + 31) / 32;
-    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm, oa, ta), where);
+    if (ga) ga->w = (a.n + 31) / 32;
+    return cuda_rc(bezk::launch_task(task, parts, a, *cfg, ep, (cudaStream_t)stream, nm, oa, ta, ga), where);
 }
 
 int bezk_compute_observations(const float* dof_state, const float* rigid_body, const float* root_states, float* net_contact,
@@ -301,9 +302,10 @@ int bezk_post_physics_task(int task, float* dof_state, const float* rigid_body, 
 
 }  // extern "C"
 
-// the whole step with the optional episode accumulators, observation normaliser, outcome counts and reward terms: the body of
-// bezk_post_physics_rollout_ep_norm (outcome_partials and term_partials NULL), bezk_post_physics_rollout_ep_outcome (term_partials
-// NULL) and bezk_post_physics_rollout_ep_terms
+// the whole step with the optional episode accumulators, observation normaliser, outcome counts, reward terms and game term
+// returns: the body of bezk_post_physics_rollout_ep_norm (outcome_partials, term_partials and the game term arguments NULL),
+// bezk_post_physics_rollout_ep_outcome (term_partials and the game term arguments NULL), bezk_post_physics_rollout_ep_terms (the
+// game term arguments NULL) and bezk_post_physics_rollout_ep_game_terms
 static int rollout_step(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact, float* prev_lin_vel,
                         float* goal, const float* goal_angle, const float* ball_init, const float* initial_root_states,
                         const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step, int64_t* reset_buf,
@@ -311,7 +313,7 @@ static int rollout_step(int task, float* dof_state, const float* rigid_body, flo
                         float* obs_clipped, float* rew, const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards,
                         uint8_t* dones_u8, int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
                         const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm, int32_t* outcome_partials,
-                        double* term_partials, void* stream) {
+                        double* term_partials, float* game_term_returns, double* game_term_partials, void* stream) {
     REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
     REQUIRE(env_base >= 0, "env_base < 0");
     REQUIRE(!shaped_rewards || rollout, "shaped_rewards requested without a BezkRolloutCfg");
@@ -336,12 +338,15 @@ static int rollout_step(int task, float* dof_state, const float* rigid_body, flo
     const bezk::NormArgs nm = {obs_mean, obs_var, obs_norm, obs_eps};
     bezk::OutArgs oa = {outcome_partials, 0};
     bezk::TermArgs ta = {term_partials, 0};
+    bezk::GameTermArgs ga = {game_term_returns, game_term_partials, 0};
     return run_task(BEZK_PART_BOOKKEEP | BEZK_PART_OBS | BEZK_PART_REWARD, a, cfg, stream,
-                    term_partials ? "bezk_post_physics_rollout_ep_terms"
-                                  : (outcome_partials ? "bezk_post_physics_rollout_ep_outcome"
-                                                      : (norm ? "bezk_post_physics_rollout_ep_norm"
-                                                              : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout"))),
-                    task, armed ? &ep : nullptr, norm ? &nm : nullptr, outcome_partials ? &oa : nullptr, term_partials ? &ta : nullptr);
+                    game_term_returns ? "bezk_post_physics_rollout_ep_game_terms"
+                    : term_partials   ? "bezk_post_physics_rollout_ep_terms"
+                                      : (outcome_partials ? "bezk_post_physics_rollout_ep_outcome"
+                                                          : (norm ? "bezk_post_physics_rollout_ep_norm"
+                                                                  : (armed ? "bezk_post_physics_rollout_ep" : "bezk_post_physics_rollout"))),
+                    task, armed ? &ep : nullptr, norm ? &nm : nullptr, outcome_partials ? &oa : nullptr, term_partials ? &ta : nullptr,
+                    game_term_returns ? &ga : nullptr);
 }
 
 extern "C" {
@@ -357,7 +362,7 @@ int bezk_post_physics_rollout_ep_norm(int task, float* dof_state, const float* r
     return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
                         initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
                         obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
-                        obs_mean, obs_var, obs_eps, obs_norm, nullptr, nullptr, stream);
+                        obs_mean, obs_var, obs_eps, obs_norm, nullptr, nullptr, nullptr, nullptr, stream);
 }
 
 int bezk_post_physics_rollout_ep_outcome(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -376,7 +381,7 @@ int bezk_post_physics_rollout_ep_outcome(int task, float* dof_state, const float
     return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
                         initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
                         obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
-                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, nullptr, stream);
+                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, nullptr, nullptr, nullptr, stream);
 }
 
 int bezk_post_physics_rollout_ep_terms(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -397,7 +402,32 @@ int bezk_post_physics_rollout_ep_terms(int task, float* dof_state, const float* 
     return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
                         initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
                         obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
-                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, term_partials, stream);
+                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, term_partials, nullptr, nullptr, stream);
+}
+
+int bezk_post_physics_rollout_ep_game_terms(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
+                                            float* prev_lin_vel, float* goal, const float* goal_angle, const float* ball_init,
+                                            const float* initial_root_states, const float* uniforms, const float* goal_uniforms,
+                                            uint64_t seed, uint64_t step, int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                            int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped, float* rew,
+                                            const BezkRolloutCfg* rollout, const float* values, float* shaped_rewards, uint8_t* dones_u8,
+                                            int64_t env_base, int64_t n, float* ep_return, float* ep_length, double* ep_partials,
+                                            const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm,
+                                            int32_t* outcome_partials, double* term_partials, float* game_term_returns,
+                                            double* game_term_partials, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(game_term_returns && game_term_partials, "game_term_returns / game_term_partials NULL");
+    REQUIRE(ep_return && ep_length && ep_partials, "the game term returns need the episode accumulators: ep_return, ep_length and ep_partials must be non-NULL");
+    REQUIRE(!(term_partials && (obs_mean || obs_var || obs_norm)), "the reward terms do not ride with the observation normaliser: obs_mean, obs_var and obs_norm must be NULL with term_partials");
+    if (!ALIGNED(game_term_returns, 4) || !ALIGNED(game_term_partials, 8))
+        return fail(BEZK_E_ALIGN, "game_term_returns must be 4-byte and game_term_partials 8-byte aligned");
+    if (!ALIGNED(term_partials, 8)) return fail(BEZK_E_ALIGN, "term_partials must be 8-byte aligned");
+    if (!ALIGNED(outcome_partials, 4)) return fail(BEZK_E_ALIGN, "outcome_partials must be 4-byte aligned");
+    return rollout_step(task, dof_state, rigid_body, root_states, net_contact, prev_lin_vel, goal, goal_angle, ball_init,
+                        initial_root_states, uniforms, goal_uniforms, seed, step, reset_buf, progress_buf, timeout_buf, randomize_buf, cfg,
+                        obs, obs_clipped, rew, rollout, values, shaped_rewards, dones_u8, env_base, n, ep_return, ep_length, ep_partials,
+                        obs_mean, obs_var, obs_eps, obs_norm, outcome_partials, term_partials, game_term_returns, game_term_partials,
+                        stream);
 }
 
 int bezk_post_physics_rollout_ep(int task, float* dof_state, const float* rigid_body, float* root_states, float* net_contact,
@@ -495,6 +525,32 @@ int bezk_reward_terms_update(const double* partials, int steps, int64_t n, int t
     if (!ALIGNED(partials, 8) || !ALIGNED(mean_k, 8)) return fail(BEZK_E_ALIGN, "partials / mean_k must be 8-byte aligned");
     return cuda_rc(bezk::launch_reward_terms_update(partials, steps, n, bezk::reward_terms(task), mean_k, (cudaStream_t)stream),
                    "bezk_reward_terms_update");
+}
+
+int bezk_game_terms_meter_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int task,
+                                 int64_t games_to_track, float* mean_k, int64_t* size, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    REQUIRE(games_to_track > 0, "games_to_track must be positive");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(ep_partials && term_partials && mean_k && size, "ep_partials / term_partials / mean_k / size NULL");
+    if (!ALIGNED(ep_partials, 8) || !ALIGNED(term_partials, 8) || !ALIGNED(mean_k, 4) || !ALIGNED(size, 8))
+        return fail(BEZK_E_ALIGN, "ep_partials / term_partials / size must be 8-byte and mean_k 4-byte aligned");
+    return cuda_rc(bezk::launch_game_terms_meter_update(ep_partials, term_partials, steps, n, bezk::reward_terms(task), games_to_track,
+                                                        mean_k, size, (cudaStream_t)stream), "bezk_game_terms_meter_update");
+}
+
+int bezk_player_game_terms_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int task,
+                                  int64_t games_num, double* sums, double* per_step, void* stream) {
+    REQUIRE(task == BEZK_TASK_KICK || task == BEZK_TASK_WALK || task == BEZK_TASK_ORIENT, "unknown task");
+    REQUIRE(steps >= 0 && n >= 0, "steps / n < 0");
+    REQUIRE(games_num > 0, "games_num must be positive");
+    if (steps == 0 || n == 0) return 0;
+    REQUIRE(ep_partials && term_partials && sums, "ep_partials / term_partials / sums NULL");
+    if (!ALIGNED(ep_partials, 8) || !ALIGNED(term_partials, 8) || !ALIGNED(sums, 8) || !ALIGNED(per_step, 8))
+        return fail(BEZK_E_ALIGN, "ep_partials / term_partials / sums / per_step must be 8-byte aligned");
+    return cuda_rc(bezk::launch_player_game_terms_update(ep_partials, term_partials, steps, n, bezk::reward_terms(task), games_num, sums,
+                                                         per_step, (cudaStream_t)stream), "bezk_player_game_terms_update");
 }
 
 int bezk_goal_uniforms(uint64_t seed, uint64_t step, float* out2, void* stream) {

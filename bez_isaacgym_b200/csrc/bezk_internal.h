@@ -96,8 +96,17 @@ struct TermArgs {
     double* partials;            // (K, W): per warp of 32 envs the fp64 sum of term k over its envs
     int64_t w;                   // W
 };
-// fills l2_resident (bezk_task.cu): after fill_alignment, before the launch; ep: the armed episode accumulators or nullptr
-void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a, const EpArgs* ep = nullptr);
+// Game term returns of the fused step (bezk_post_physics_rollout_ep_game_terms): per env one carried accumulator per reward term,
+// with episode_step's recurrence, and per warp the fp64 sum of the done envs' per-term episode returns.  A separate kernel parameter
+// of task_tile_game_kernel / task_tile_game_l2_kernel, appended after every other pack element, for the reason EpArgs is one.
+struct GameTermArgs {
+    float* acc;                  // (K, n), term-major: acc + term, times (1 - done)
+    double* partials;            // (K, W): per warp of 32 envs the fp64 sum of (acc + term) over its done envs
+    int64_t w;                   // W
+};
+// fills l2_resident (bezk_task.cu): after fill_alignment, before the launch; ep: the armed episode accumulators or nullptr; ga: the
+// armed game term accumulators or nullptr (they join the carried set)
+void set_l2_policy(int task, uint32_t cfg_flags, TaskArgs& a, const EpArgs* ep = nullptr, const GameTermArgs* ga = nullptr);
 // demote [ptr, ptr + bytes) to the normal L2 eviction priority (the 128-byte lines entirely inside the range)
 cudaError_t launch_l2_release(const void* ptr, uint64_t bytes, cudaStream_t st);
 struct PpoArgs {
@@ -116,9 +125,11 @@ struct PpoArgs {
 // task_tile_ep_kernel / task_tile_ep_l2_kernel) only with parts = 7; nm (the observation normaliser, task_tile_obsnorm_kernel /
 // task_tile_obsnorm_l2_kernel) and oa (the outcome counts, task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel) only
 // together with ep; ta (the reward terms, task_tile_terms_kernel / task_tile_outcome_terms_kernel) only together with ep and
-// without nm.  cudaErrorInvalidValue for any other combination.
+// without nm; ga (the game term returns, task_tile_game_kernel) with any of those packs.  cudaErrorInvalidValue for any other
+// combination.
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
-                        const NormArgs* nm = nullptr, const OutArgs* oa = nullptr, const TermArgs* ta = nullptr);
+                        const NormArgs* nm = nullptr, const OutArgs* oa = nullptr, const TermArgs* ta = nullptr,
+                        const GameTermArgs* ga = nullptr);
 // folds `steps` x (3, ceil(n / 32)) partials of launch_task's episode accumulators into the two AverageMeters (bezk_rollout.cu)
 cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                                         int64_t* size2, cudaStream_t st);
@@ -135,6 +146,13 @@ cudaError_t launch_player_outcome_update(const int32_t* partials, int steps, int
                                          double* per_step, cudaStream_t st);
 // folds `steps` x (K, ceil(n / 32)) reward term partials into the (K,) means per env-step over steps x n (bezk_rollout.cu)
 cudaError_t launch_reward_terms_update(const double* partials, int steps, int64_t n, int k, double* mean_k, cudaStream_t st);
+// rl_games AverageMeter(K, games_to_track) fed with one K-row of game term returns per done env, from `steps` x (3, ceil(n / 32))
+// episode partials (the done counts) and `steps` x (K, ceil(n / 32)) game term partials (bezk_rollout.cu)
+cudaError_t launch_game_terms_meter_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int k,
+                                           int64_t games_to_track, float* mean_k, int64_t* size, cudaStream_t st);
+// folds the same partials into [games_counted, sum_0 .. sum_{K-1}] with player_tally_kernel's cutoff (bezk_rollout.cu)
+cudaError_t launch_player_game_terms_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int k,
+                                            int64_t games_num, double* sums, double* per_step, cudaStream_t st);
 cudaError_t launch_goal_uniforms(uint64_t seed, uint64_t step, float* out2, cudaStream_t st);
 void fill_alignment(TaskArgs& a, const BezkTaskCfg& cfg);
 cudaError_t stage_feet_gather(const float*, const BezkTaskCfg&, float*, int64_t, int64_t, cudaStream_t);

@@ -531,6 +531,58 @@ struct EpmScratch {
     unsigned* tickets;     // (steps + 1,) zeroed: per step (its warps), then the steps
 };
 
+// Step blockIdx.x's sums of `rows` (<= R) rows of W slots each, row r at row(r), in episode_meter_kernel's order: thread i adds
+// slots i, i + EPM_THREADS, ... in order, a shuffle-down tree (16, 8, 4, 2, 1) per warp, and the last warp of the CTA to finish
+// (ticket) adds the EPM_WARPS warp sums in order into step_sums[step * rows + r].  True in every lane of the last warp of the
+// launch to finish (the steps' ticket).  episode_meter_kernel keeps its own copy of this code (R = rows = 3), compiled as before.
+template <int R, typename Row>
+__device__ __forceinline__ bool epm_step_sums(Row row, int rows, int steps, int64_t w, EpmScratch sc) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int step = blockIdx.x;
+    double acc[R];
+#pragma unroll
+    for (int k = 0; k < R; ++k) acc[k] = 0.0;
+    for (int64_t i = threadIdx.x; i < w; i += EPM_THREADS) {
+#pragma unroll
+        for (int k = 0; k < R; ++k)
+            if (k < rows) acc[k] += row(k)[i];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int k = 0; k < R; ++k) acc[k] += __shfl_down_sync(0xffffffffu, acc[k], o);
+    }
+    const unsigned full = 0xffffffffu;
+    int last = 0;
+    if (lane == 0) {
+        double* ws = sc.warp_sums + ((int64_t)step * EPM_WARPS + warp) * rows;
+#pragma unroll
+        for (int k = 0; k < R; ++k)
+            if (k < rows) ws[k] = acc[k];
+        __threadfence();
+        last = atomicAdd(&sc.tickets[step], 1u) == EPM_WARPS - 1;
+    }
+    if (!__shfl_sync(full, last, 0)) return false;
+    // the last warp of this CTA: the step's sums, warp by warp in order
+    __threadfence();
+    if (lane == 0) {
+        const double* wsum = sc.warp_sums + (int64_t)step * EPM_WARPS * rows;
+#pragma unroll
+        for (int k = 0; k < R; ++k) {
+            if (k >= rows) continue;
+            double v = 0.0;
+#pragma unroll
+            for (int j = 0; j < EPM_WARPS; ++j) v += __ldcg(wsum + j * rows + k);
+            sc.step_sums[step * rows + k] = v;
+        }
+        __threadfence();
+        last = atomicAdd(&sc.tickets[steps], 1u) == (unsigned)steps - 1;
+    }
+    if (!__shfl_sync(full, last, 0)) return false;
+    __threadfence();
+    return true;
+}
+
 __global__ void __launch_bounds__(EPM_THREADS) episode_meter_kernel(const double* __restrict__ partials, int steps, int64_t w,
                                                                     int64_t max_size, EpmScratch sc, float* mean2, int64_t* size2) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -607,19 +659,25 @@ __global__ void __launch_bounds__(EPM_THREADS) episode_meter_kernel(const double
     }
 }
 
+// the sums and tickets of epm_step_sums over `rows` rows live for one launch only: stream-ordered scratch (capturable in a CUDA graph,
+// no host synchronisation), tickets zeroed on the stream
+static cudaError_t epm_scratch(int steps, int rows, cudaStream_t st, void** buf, EpmScratch& sc) {
+    const size_t nd = (size_t)steps * (EPM_WARPS + 1) * rows, bytes = nd * sizeof(double) + (size_t)(steps + 1) * sizeof(unsigned);
+    cudaError_t e = cudaMallocAsync(buf, bytes, st);
+    if (e != cudaSuccess) return e;
+    sc.warp_sums = static_cast<double*>(*buf);
+    sc.step_sums = sc.warp_sums + (size_t)steps * EPM_WARPS * rows;
+    sc.tickets = reinterpret_cast<unsigned*>(sc.warp_sums + nd);
+    return cudaMemsetAsync(sc.tickets, 0, (size_t)(steps + 1) * sizeof(unsigned), st);
+}
+
 cudaError_t launch_episode_meter_update(const double* partials, int steps, int64_t n, int64_t games_to_track, float* mean2,
                                         int64_t* size2, cudaStream_t st) {
     if (steps == 0 || n == 0) return cudaSuccess;
-    // the sums and tickets live for this launch only: stream-ordered scratch (capturable in a CUDA graph, no host synchronisation)
-    const size_t nd = (size_t)steps * (EPM_WARPS + 1) * 3, bytes = nd * sizeof(double) + (size_t)(steps + 1) * sizeof(unsigned);
     void* buf = nullptr;
-    cudaError_t e = cudaMallocAsync(&buf, bytes, st);
-    if (e != cudaSuccess) return e;
     EpmScratch sc;
-    sc.warp_sums = static_cast<double*>(buf);
-    sc.step_sums = sc.warp_sums + (size_t)steps * EPM_WARPS * 3;
-    sc.tickets = reinterpret_cast<unsigned*>(sc.warp_sums + nd);
-    e = cudaMemsetAsync(sc.tickets, 0, (size_t)(steps + 1) * sizeof(unsigned), st);
+    cudaError_t e = epm_scratch(steps, 3, st, &buf, sc);
+    if (buf == nullptr) return e;
     if (e == cudaSuccess)
         e = launch_ex(episode_meter_kernel, dim3((unsigned)steps), dim3(EPM_THREADS), 0, st, partials, steps, (n + 31) / 32,
                       games_to_track, sc, mean2, size2);
@@ -953,6 +1011,161 @@ cudaError_t launch_reward_terms_update(const double* partials, int steps, int64_
     if (e == cudaSuccess)
         e = launch_ex(reward_terms_kernel, dim3((unsigned)steps, (unsigned)k), dim3(RT_THREADS), 0, st, partials, steps, (n + 31) / 32,
                       n, sc, mean_k);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Game term returns: the per-step (K, W) fp64 game term partials of the fused step (per warp of 32 envs the sum of each term's
+// episode return over its done envs) with row 0 of the step's ep_partials (per warp its done count), folded into
+//   * game_terms_meter_kernel: rl_games' AverageMeter(K, games_to_track) fed with one K-row per done env -- episode_meter_kernel's
+//     recurrence, step by step in order, with new_mean[k] = (float)(sum_k / count) in fp64 and size = count, so this meter's size
+//     always equals the game meters' size;
+//   * player_game_terms_kernel: [games_counted, sum_0 .. sum_{K-1}] with player_tally_kernel's cutoff -- a step that starts with
+//     games_counted >= games_num adds nothing, the step that reaches it is added whole -- and optionally each folded step's K sums.
+// Each step's 1 + K sums come from epm_step_sums (fixed order: the same bits every run, restated in tests/game_terms_oracle.py).
+// No barrier, no local memory, scratch from stream-ordered allocation: capturable in a CUDA graph.
+// ------------------------------------------------------------------------------------------------
+constexpr int GT_MAX = 6;
+
+// step blockIdx.x's [done count, sum_0 .. sum_{K-1}] into sc.step_sums (rows of 1 + k); true in the last warp of the launch
+__device__ __forceinline__ bool game_terms_step_sums(const double* __restrict__ ep_partials, const double* __restrict__ term_partials,
+                                                     int steps, int64_t w, int k, EpmScratch sc) {
+    const double* ep = ep_partials + (int64_t)blockIdx.x * 3 * w;
+    const double* tp = term_partials + (int64_t)blockIdx.x * k * w;
+    return epm_step_sums<1 + GT_MAX>([&](int r) { return r == 0 ? ep : tp + (r - 1) * w; }, 1 + k, steps, w, sc);
+}
+
+__global__ void __launch_bounds__(EPM_THREADS) game_terms_meter_kernel(const double* __restrict__ ep_partials,
+                                                                       const double* __restrict__ term_partials, int steps, int64_t w,
+                                                                       int k, int64_t max_size, EpmScratch sc, float* mean_k,
+                                                                       int64_t* size) {
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    pdl_launch_dependents();
+    pdl_wait();
+    if (!game_terms_step_sums(ep_partials, term_partials, steps, w, k, sc)) return;
+    // the recurrence, step by step in order: lane j loads step t0 + j's sums, every lane runs the same arithmetic
+    float mean[GT_MAX];
+#pragma unroll
+    for (int c = 0; c < GT_MAX; ++c) mean[c] = c < k ? mean_k[c] : 0.0f;
+    int64_t cur = *size;
+    for (int t0 = 0; t0 < steps; t0 += 32) {
+        double cnt = 0.0, sum[GT_MAX];
+#pragma unroll
+        for (int c = 0; c < GT_MAX; ++c) sum[c] = 0.0;
+        if (t0 + lane < steps) {
+            const double* q = sc.step_sums + (int64_t)(t0 + lane) * (1 + k);
+            cnt = __ldcg(q);
+#pragma unroll
+            for (int c = 0; c < GT_MAX; ++c)
+                if (c < k) sum[c] = __ldcg(q + 1 + c);
+        }
+        const int m = steps - t0 < 32 ? steps - t0 : 32;
+        for (int j = 0; j < m; ++j) {
+            const double cj = __shfl_sync(full, cnt, j);
+            double sj[GT_MAX];
+#pragma unroll
+            for (int c = 0; c < GT_MAX; ++c) sj[c] = __shfl_sync(full, sum[c], j);
+            if (!(cj > 0.0)) continue;          // AverageMeter.update: size == 0 -> no-op
+            const int64_t sz = (int64_t)cj < max_size ? (int64_t)cj : max_size;
+            const int64_t old_size = (max_size - sz) < cur ? (max_size - sz) : cur;
+            const int64_t size_sum = old_size + sz;
+            cur = size_sum;
+#pragma unroll
+            for (int c = 0; c < GT_MAX; ++c) {
+                const float new_mean = (float)(sj[c] / cj);
+                mean[c] = (mean[c] * (float)old_size + new_mean * (float)sz) / (float)size_sum;
+            }
+        }
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int c = 0; c < GT_MAX; ++c)
+            if (c < k) mean_k[c] = mean[c];
+        *size = cur;
+    }
+}
+
+__global__ void __launch_bounds__(EPM_THREADS) player_game_terms_kernel(const double* __restrict__ ep_partials,
+                                                                        const double* __restrict__ term_partials, int steps, int64_t w,
+                                                                        int k, double games_num, EpmScratch sc, double* sums,
+                                                                        double* per_step) {
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    pdl_launch_dependents();
+    pdl_wait();
+    if (!game_terms_step_sums(ep_partials, term_partials, steps, w, k, sc)) return;
+    double games = __ldcg(sums), tot[GT_MAX];
+#pragma unroll
+    for (int c = 0; c < GT_MAX; ++c) tot[c] = c < k ? __ldcg(sums + 1 + c) : 0.0;
+    for (int t0 = 0; t0 < steps; t0 += 32) {
+        double cnt = 0.0, sum[GT_MAX];
+#pragma unroll
+        for (int c = 0; c < GT_MAX; ++c) sum[c] = 0.0;
+        if (t0 + lane < steps) {
+            const double* q = sc.step_sums + (int64_t)(t0 + lane) * (1 + k);
+            cnt = __ldcg(q);
+#pragma unroll
+            for (int c = 0; c < GT_MAX; ++c)
+                if (c < k) sum[c] = __ldcg(q + 1 + c);
+        }
+        bool mine = false;                      // this lane's step was folded
+        const int m = steps - t0 < 32 ? steps - t0 : 32;
+        for (int j = 0; j < m; ++j) {
+            const double cj = __shfl_sync(full, cnt, j);
+            double sj[GT_MAX];
+#pragma unroll
+            for (int c = 0; c < GT_MAX; ++c) sj[c] = __shfl_sync(full, sum[c], j);
+            if (games >= games_num) continue;   // the cutoff was reached by an earlier step
+            if (lane == j) mine = true;
+            if (cj > 0.0) {
+                games += cj;
+#pragma unroll
+                for (int c = 0; c < GT_MAX; ++c) tot[c] += sj[c];
+            }
+        }
+        if (per_step && t0 + lane < steps) {
+            double* q = per_step + (int64_t)k * (t0 + lane);
+#pragma unroll
+            for (int c = 0; c < GT_MAX; ++c)
+                if (c < k) q[c] = mine ? sum[c] : 0.0;
+        }
+    }
+    if (lane == 0) {
+        sums[0] = games;
+#pragma unroll
+        for (int c = 0; c < GT_MAX; ++c)
+            if (c < k) sums[1 + c] = tot[c];
+    }
+}
+
+cudaError_t launch_game_terms_meter_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int k,
+                                           int64_t games_to_track, float* mean_k, int64_t* size, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    if (k < 1 || k > GT_MAX) return cudaErrorInvalidValue;
+    void* buf = nullptr;
+    EpmScratch sc;
+    cudaError_t e = epm_scratch(steps, 1 + k, st, &buf, sc);
+    if (buf == nullptr) return e;
+    if (e == cudaSuccess)
+        e = launch_ex(game_terms_meter_kernel, dim3((unsigned)steps), dim3(EPM_THREADS), 0, st, ep_partials, term_partials, steps,
+                      (n + 31) / 32, k, games_to_track, sc, mean_k, size);
+    const cudaError_t f = cudaFreeAsync(buf, st);
+    return e != cudaSuccess ? e : f;
+}
+
+cudaError_t launch_player_game_terms_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int k,
+                                            int64_t games_num, double* sums, double* per_step, cudaStream_t st) {
+    if (steps == 0 || n == 0) return cudaSuccess;
+    if (k < 1 || k > GT_MAX) return cudaErrorInvalidValue;
+    void* buf = nullptr;
+    EpmScratch sc;
+    cudaError_t e = epm_scratch(steps, 1 + k, st, &buf, sc);
+    if (buf == nullptr) return e;
+    if (e == cudaSuccess)
+        e = launch_ex(player_game_terms_kernel, dim3((unsigned)steps), dim3(EPM_THREADS), 0, st, ep_partials, term_partials, steps,
+                      (n + 31) / 32, k, (double)games_num, sc, sums, per_step);
     const cudaError_t f = cudaFreeAsync(buf, st);
     return e != cudaSuccess ? e : f;
 }

@@ -263,19 +263,26 @@ __device__ __forceinline__ void episode_epilogue(const EpArgs& ep, int64_t e, fl
     done = reset != 0;
 }
 
-__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep) { return ep; }
-__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const NormArgs&) { return ep; }
-__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const OutArgs&) { return ep; }
-__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const NormArgs&, const OutArgs&) { return ep; }
-__device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs& nm) { return nm; }
-__device__ __forceinline__ const NormArgs& norm_of(const EpArgs&, const NormArgs& nm, const OutArgs&) { return nm; }
-__device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const OutArgs& oa) { return oa; }
-__device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const NormArgs&, const OutArgs& oa) { return oa; }
-__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const TermArgs&) { return ep; }
-__device__ __forceinline__ const EpArgs& ep_of(const EpArgs& ep, const OutArgs&, const TermArgs&) { return ep; }
-__device__ __forceinline__ const OutArgs& out_of(const EpArgs&, const OutArgs& oa, const TermArgs&) { return oa; }
-__device__ __forceinline__ const TermArgs& terms_of(const EpArgs&, const TermArgs& ta) { return ta; }
-__device__ __forceinline__ const TermArgs& terms_of(const EpArgs&, const OutArgs&, const TermArgs& ta) { return ta; }
+// the game term returns of one env in the reward epilogue: episode_step's recurrence on each term's accumulator.  acc holds the
+// carried values on entry and r_k = acc_k + term_k on return; the carried values are stored as multiplies by (1 - done)
+template <bool L2H, int K>
+__device__ __forceinline__ void game_terms_epilogue(const GameTermArgs& ga, int64_t n, int64_t e, int64_t reset, const float (&tm)[K],
+                                                    float (&acc)[K]) {
+    const float not_done = 1.0f - (reset != 0 ? 1.0f : 0.0f);
+    const uint64_t pk = L2H ? policy_evict_last() : 0;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        acc[k] = acc[k] + tm[k];
+        L2HINT(st_f32, pk, ga.acc + k * n + e, acc[k] * not_done);
+    }
+}
+
+// the pack element of type T
+template <typename T, typename P0, typename... P>
+__device__ __forceinline__ const T& arg_of(const P0& p0, const P&... p) {
+    if constexpr (std::is_same<T, P0>::value) return p0;
+    else return arg_of<T>(p...);
+}
 template <typename T, typename... P>
 constexpr bool has_arg = (std::is_same<T, P>::value || ...);
 
@@ -283,7 +290,8 @@ constexpr bool has_arg = (std::is_same<T, P>::value || ...);
 // whole step only) -- or EpArgs and NormArgs: the eval-mode observation normaliser too (task_tile_obsnorm_kernel /
 // task_tile_obsnorm_l2_kernel).  Either EP pack may end in OutArgs: the per-warp episode outcome counts too
 // (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms).  EpArgs (and OutArgs) may be followed by
-// TermArgs: the per-warp reward term sums too (task_tile_terms_kernel / task_tile_outcome_terms_kernel and their _l2 forms).  A
+// TermArgs: the per-warp reward term sums too (task_tile_terms_kernel / task_tile_outcome_terms_kernel and their _l2 forms).  Any of
+// these packs may end in GameTermArgs: the carried game term returns too (task_tile_game_kernel / task_tile_game_l2_kernel).  A
 // parameter pack rather than always-present arguments: the kernels without accumulators make exactly the call they made before the
 // accumulators existed (an unused EpArgs argument alone changes their register allocation).
 template <int PARTS, bool CLEATS, int TILE, int TASK, bool L2H, typename... Ep>
@@ -292,6 +300,8 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     constexpr bool NORM = has_arg<NormArgs, Ep...>;
     constexpr bool OUT = has_arg<OutArgs, Ep...>;
     constexpr bool TERMS = has_arg<TermArgs, Ep...>;
+    constexpr bool GAME = has_arg<GameTermArgs, Ep...>;
+    constexpr int K_TERMS = reward_terms(TASK);
     static_assert(!EP || PARTS == 7, "the episode accumulators ride in the whole step");
     constexpr int ROOT_ROW = root_row(TASK);
     constexpr int OBS_ROW = obs_row(TASK);
@@ -341,17 +351,27 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
     gather_env<OBS, (BOOK || REW), CLEATS, TASK, L2H>(a, cfg, e, valid, rb, cf_l, cf_r, g);
     float ep_ret = 0.0f, ep_len = 0.0f;    // carried like the bookkeeping: the same addresses every step
     if constexpr (EP) {
-        const EpArgs& ep = ep_of(eps...);
+        const EpArgs& ep = arg_of<EpArgs>(eps...);
         if (valid) {
             const uint64_t pk = L2H ? policy_evict_last() : 0;
             ep_ret = L2HINT(ld_f32, pk, ep.ret + e);
             ep_len = L2HINT(ld_f32, pk, ep.len + e);
         }
     }
+    float gacc[K_TERMS] = {};              // GAME: the carried game term returns, then this step's r_k (0 in lanes past the last env)
+    if constexpr (GAME) {
+        const GameTermArgs& ga = arg_of<GameTermArgs>(eps...);
+        if (valid) {
+            const uint64_t pk = L2H ? policy_evict_last() : 0;
+#pragma unroll
+            for (int k = 0; k < K_TERMS; ++k) gacc[k] = L2HINT(ld_f32, pk, ga.acc + k * a.n + e);
+        }
+    }
     bool ep_done = false;                  // this env's episode ended in this step, with return ep_r and length ep_l
     float ep_r = 0.0f, ep_l = 0.0f;
     int ep_oc = OUTCOME_NONE;              // OUT: the rule that ended it (the outcome class), from the reward call whose rew is stored
-    float tm[reward_terms(TASK)] = {};     // TERMS: this env's reward terms, from the same call (0 in lanes past the last env)
+    float tm[K_TERMS] = {};                // TERMS / GAME: this env's reward terms, from the same call (0 in lanes past the last env)
+    constexpr bool TM = TERMS || GAME;
 
 
     // ---- 2. dense tiles: TMA bulk copies (full sub-tiles) or cooperative coalesced loads (tail) ----
@@ -601,34 +621,35 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
             for (int k = 0; k < 3; ++k) { s.v[k] = v[k]; s.w[k] = w[k]; }
             s.pos_sq = pos_sq;
             Mth<true> mr;
-            reward_term<true, OUT, TERMS>(s, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
+            reward_term<true, OUT, TM>(s, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
             if (mr.bad()) {
                 Mth<false> mp;
-                reward_term<false, OUT, TERMS>(s, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
+                reward_term<false, OUT, TM>(s, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
             }
         } else {
             Mth<true> mr;
             if (TASK == BEZK_TASK_WALK)
-                reward_walk<true, OUT, TERMS>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
-            else reward_orient<true, OUT, TERMS>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
+                reward_walk<true, OUT, TM>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
+            else reward_orient<true, OUT, TM>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mr, &ep_oc, tm);
             if (mr.bad()) {
                 Mth<false> mp;
                 if (TASK == BEZK_TASK_WALK)
-                    reward_walk<false, OUT, TERMS>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
-                else reward_orient<false, OUT, TERMS>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
+                    reward_walk<false, OUT, TM>(bez, q, v, w, pos_sq, goal, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
+                else reward_orient<false, OUT, TM>(bez, q, v, w, pos_sq, g.gang, cfg, progress, reset_cur, &rew, &reset, mp, &ep_oc, tm);
             }
         }
         L2HINT(st_f32, L2H ? policy_evict_last() : 0, a.rew + e, rew);
         L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.reset_out + e, reset);
         if (BOOK) { L2HINT(st_i64, L2H ? policy_evict_last() : 0, a.progress_out + e, progress); rollout_epilogue(a, e, rew, reset, timeout, g.value); }
-        if constexpr (EP) episode_epilogue<L2H>(ep_of(eps...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
+        if constexpr (EP) episode_epilogue<L2H>(arg_of<EpArgs>(eps...), e, rew, reset, ep_ret, ep_len, ep_done, ep_r, ep_l);
+        if constexpr (GAME) game_terms_epilogue<L2H>(arg_of<GameTermArgs>(eps...), a.n, e, reset, tm, gacc);
     }
 
     // ---- 9. this warp's slot of the per-step episode statistics: [count of done envs, sum of their returns, sum of their
     // lengths] at (k, env / 32).  Fixed-order shuffle tree, one store per value, every step (zeros included): nothing needs
     // zeroing, no atomics, and the sums are the same bits from run to run ----
     if constexpr (EP) if (nv > 0) {
-        const EpArgs& ep = ep_of(eps...);
+        const EpArgs& ep = arg_of<EpArgs>(eps...);
         const unsigned done_mask = __ballot_sync(0xffffffffu, ep_done);
         double sr = ep_done ? (double)ep_r : 0.0, sl = ep_done ? (double)ep_l : 0.0;
 #pragma unroll
@@ -646,7 +667,7 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
             // ... and the count of its done envs per outcome class at (k, env / 32): one ballot per class, lane k stores class k.
             // In the whole step an env is done exactly when a rule fired (reset_cur is 0 on entry), so the K counts sum to the
             // done count above
-            const OutArgs& oa = out_of(eps...);
+            const OutArgs& oa = arg_of<OutArgs>(eps...);
             constexpr int K = outcome_classes(TASK);
             unsigned mine = 0;
 #pragma unroll
@@ -658,13 +679,24 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
         }
         if constexpr (TERMS) {
             // ... and the fp64 sum of each reward term over its envs at (k, env / 32), with the same fixed-order tree
-            const TermArgs& ta = terms_of(eps...);
+            const TermArgs& ta = arg_of<TermArgs>(eps...);
 #pragma unroll
             for (int k = 0; k < reward_terms(TASK); ++k) {
                 double s = (double)tm[k];
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
                 if (lane == 0) ta.partials[k * ta.w + e0 / WT] = s;
+            }
+        }
+        if constexpr (GAME) {
+            // ... and the fp64 sum of each term's episode return over its done envs at (k, env / 32), with the same tree
+            const GameTermArgs& ga = arg_of<GameTermArgs>(eps...);
+#pragma unroll
+            for (int k = 0; k < K_TERMS; ++k) {
+                double s = ep_done ? (double)gacc[k] : 0.0;
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+                if (lane == 0) ga.partials[k * ga.w + e0 / WT] = s;
             }
         }
     }
@@ -675,7 +707,7 @@ __device__ __forceinline__ void task_tile(const TaskArgs& a, const BezkTaskCfg& 
         // plain operator for a chunk with an operand outside its range), clamp to +-5 with NaN propagating.  Lane j holds the
         // statistics of columns j and 32 + j, read from the device every launch.  The tile is normalised in place once the
         // stores above have read it, then leaves as one more bulk store (normal L2 priority: not part of the carried set) ----
-        const NormArgs& nm = norm_of(eps...);
+        const NormArgs& nm = arg_of<NormArgs>(eps...);
         if (nv == 0) return;                             // warp-uniform: a warp past the last env
         const float m_lo = (float)nm.mean[lane], d_lo = sqrtf((float)nm.var[lane] + nm.eps);
         float m_hi = 0.0f, d_hi = 1.0f;
@@ -811,6 +843,20 @@ __global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_o
     const TaskArgs a, const __grid_constant__ BezkTaskCfg cfg, const EpArgs ep, const OutArgs oa, const TermArgs ta) {
     task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, ep, oa, ta);
 }
+// every EP step above that also carries the game term returns (bezk_post_physics_rollout_ep_game_terms): Ep is that step's pack
+// followed by GameTermArgs
+template <bool CLEATS, int TILE, int TASK, typename... Ep>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_game_kernel(const TaskArgs a,
+                                                                                           const __grid_constant__ BezkTaskCfg cfg,
+                                                                                           const Ep... eps) {
+    task_tile<7, CLEATS, TILE, TASK, false>(a, cfg, eps...);
+}
+template <bool CLEATS, int TILE, int TASK, typename... Ep>
+__global__ void __launch_bounds__(TILE, BEZK_TILE_CTAS * 128 / TILE) task_tile_game_l2_kernel(const TaskArgs a,
+                                                                                              const __grid_constant__ BezkTaskCfg cfg,
+                                                                                              const Ep... eps) {
+    task_tile<7, CLEATS, TILE, TASK, true>(a, cfg, eps...);
+}
 
 // ------------------------------------------------------------------------------------------------
 // K3 (function level): reset_idx over an explicit id list; one thread per (id, dof) pair + root rows.
@@ -866,8 +912,9 @@ static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>
 // Ep: empty (task_tile_kernel / task_tile_l2_kernel), the episode accumulators (task_tile_ep_kernel / task_tile_ep_l2_kernel) or
 // those and the observation normaliser (task_tile_obsnorm_kernel / task_tile_obsnorm_l2_kernel), either EP pack followed by the
 // outcome counts (task_tile_outcome_kernel / task_tile_obsnorm_outcome_kernel and their _l2 forms), the EP or EP + outcome pack
-// followed by the reward terms (task_tile_terms_kernel / task_tile_outcome_terms_kernel and their _l2 forms); a.l2_resident picks the L2
-// variant.  Every variant has the same shared memory: the normaliser works in the observation tile.
+// followed by the reward terms (task_tile_terms_kernel / task_tile_outcome_terms_kernel and their _l2 forms), any of those packs
+// followed by the game term returns (task_tile_game_kernel / task_tile_game_l2_kernel); a.l2_resident picks the L2 variant.  Every
+// variant has the same shared memory: the normaliser works in the observation tile.
 template <int PARTS, bool CLEATS, int TILE, int TASK, typename... Ep>
 static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaStream_t st, const Ep&... eps) {
     static_assert(sizeof...(Ep) == 0 || PARTS == 7, "the episode accumulators ride in the whole step");
@@ -875,6 +922,8 @@ static cudaError_t launch_tile(const TaskArgs& a, const BezkTaskCfg& cfg, cudaSt
         constexpr bool NORM = has_arg<NormArgs, Ep...>, OUT = has_arg<OutArgs, Ep...>, TERMS = has_arg<TermArgs, Ep...>;
         if constexpr (sizeof...(Ep) == 0)
             return a.l2_resident ? task_tile_l2_kernel<PARTS, CLEATS, TILE, TASK> : task_tile_kernel<PARTS, CLEATS, TILE, TASK>;
+        else if constexpr (has_arg<GameTermArgs, Ep...>)
+            return a.l2_resident ? task_tile_game_l2_kernel<CLEATS, TILE, TASK, Ep...> : task_tile_game_kernel<CLEATS, TILE, TASK, Ep...>;
         else if constexpr (TERMS && OUT)
             return a.l2_resident ? task_tile_outcome_terms_l2_kernel<CLEATS, TILE, TASK> : task_tile_outcome_terms_kernel<CLEATS, TILE, TASK>;
         else if constexpr (TERMS)
@@ -900,31 +949,28 @@ template <int V>
 using Int = std::integral_constant<int, V>;
 
 cudaError_t launch_task(int task, int parts, const TaskArgs& a, const BezkTaskCfg& cfg, const EpArgs* ep, cudaStream_t st,
-                        const NormArgs* nm, const OutArgs* oa, const TermArgs* ta) {
+                        const NormArgs* nm, const OutArgs* oa, const TermArgs* ta, const GameTermArgs* ga) {
     const bool cleats = (cfg.flags & BEZK_F_CLEATS) != 0;
-    if ((nm || oa || ta) && !ep) return cudaErrorInvalidValue;
+    if ((nm || oa || ta || ga) && !ep) return cudaErrorInvalidValue;
     if (ta && nm) return cudaErrorInvalidValue;
-    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators (and the normaliser / outcome counts) only with the
-    // whole step
+    // one (TASK, PARTS) pair, with or without cleats; the episode accumulators (and the normaliser / outcome counts / reward terms /
+    // game term returns) only with the whole step
     const auto tile = [&](auto task_c, auto parts_c) -> cudaError_t {
         constexpr int TASK = decltype(task_c)::value, PARTS = decltype(parts_c)::value;
         if constexpr (PARTS == 7) {
-            if (ta && oa)
-                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa, *ta)
-                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa, *ta);
-            if (ta)
-                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *ta)
-                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *ta);
-            if (nm && oa)
-                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm, *oa)
-                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm, *oa);
-            if (oa)
-                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa)
-                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *oa);
-            if (nm)
-                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm)
-                              : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep, *nm);
-            if (ep) return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, *ep) : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, *ep);
+            // the EP pack, followed by the game term returns when they are armed
+            const auto whole = [&](const auto&... pk) -> cudaError_t {
+                if (ga)
+                    return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, pk..., *ga)
+                                  : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, pk..., *ga);
+                return cleats ? launch_tile<7, true, BEZK_TILE, TASK>(a, cfg, st, pk...) : launch_tile<7, false, BEZK_TILE, TASK>(a, cfg, st, pk...);
+            };
+            if (ta && oa) return whole(*ep, *oa, *ta);
+            if (ta) return whole(*ep, *ta);
+            if (nm && oa) return whole(*ep, *nm, *oa);
+            if (oa) return whole(*ep, *oa);
+            if (nm) return whole(*ep, *nm);
+            if (ep) return whole(*ep);
         }
         if (ep) return cudaErrorInvalidValue;
         return cleats ? launch_tile<PARTS, true, BEZK_TILE, TASK>(a, cfg, st) : launch_tile<PARTS, false, BEZK_TILE, TASK>(a, cfg, st);
@@ -1019,12 +1065,13 @@ static bool on_device(const void* p) {
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { (void)cudaGetLastError(); return false; }
     return at.type == cudaMemoryTypeDevice;
 }
-void set_l2_policy(int task, uint32_t flags, TaskArgs& a, const EpArgs* ep) {
+void set_l2_policy(int task, uint32_t flags, TaskArgs& a, const EpArgs* ep, const GameTermArgs* ga) {
     a.l2_resident = 0;
     if (!l2_resident_enabled()) return;
     const void* carried[] = {a.obs, a.obs_clipped, a.reset_out, a.progress_out, a.timeout_buf, a.rew, a.prev_lin_vel, a.goal,
-                             a.ball_init, a.goal_angle, ep ? ep->ret : nullptr, ep ? ep->len : nullptr};
+                             a.ball_init, a.goal_angle, ep ? ep->ret : nullptr, ep ? ep->len : nullptr, ga ? ga->acc : nullptr};
     int64_t per_env = ep ? 8 : 0;          // the two episode accumulators, when armed
+    if (ga) per_env += 4 * reward_terms(task);   // and the K game term accumulators
     for (const void* p : carried)
         if (!on_device(p)) return;
     const bool obs_kept = !(flags & BEZK_F_OBS_STREAMED);

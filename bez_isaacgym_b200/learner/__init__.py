@@ -7,9 +7,9 @@ from .losses import ppo_loss, PPOLossConfig
 from .experience import ExperienceBuffer, PPODataset, SlabDataset
 from .policy_head import policy_head
 from .agent import A2CAgent, A2CNetwork, AdaptiveScheduler
-from .episode_meter import EpisodeMeter, OutcomeMeter, RewardTerms
+from .episode_meter import EpisodeMeter, GameTermMeter, OutcomeMeter, RewardTerms
 from .player import PpoPlayerContinuous
 
 __all__ = ["RunningMeanStd", "discount_values", "normalize_advantages", "swap_and_flatten01",
            "ppo_loss", "PPOLossConfig", "ExperienceBuffer", "PPODataset", "SlabDataset", "policy_head", "A2CAgent", "A2CNetwork",
-           "AdaptiveScheduler", "EpisodeMeter", "OutcomeMeter", "RewardTerms", "PpoPlayerContinuous"]
+           "AdaptiveScheduler", "EpisodeMeter", "GameTermMeter", "OutcomeMeter", "RewardTerms", "PpoPlayerContinuous"]

@@ -22,7 +22,7 @@ from torch import nn
 
 from .. import dist as bdist
 from . import a2c_common, experience, losses
-from .episode_meter import EpisodeMeter, OutcomeMeter, RewardTerms
+from .episode_meter import EpisodeMeter, GameTermMeter, OutcomeMeter, RewardTerms
 from .policy_head import policy_head as _policy_head
 from .running_mean_std import RunningMeanStd
 
@@ -78,6 +78,10 @@ OUTCOME_DEFAULTS = dict(track_outcomes=False)
 #: this project's own option: ``track_reward_terms`` -- sum each of the env's ``REWARD_TERMS`` in the step kernel and add a
 #: ``reward_terms`` entry (term name -> mean per env-step of the epoch's rollout) to each ``train()`` history row
 REWARD_TERM_DEFAULTS = dict(track_reward_terms=False)
+#: this project's own option: ``track_game_reward_terms`` -- carry each episode's return per term of the env's ``REWARD_TERMS`` in
+#: the step kernel, into the ``game_reward_terms`` meter and a ``game_reward_terms`` entry (term name -> mean return per game) of
+#: each ``train()`` history row
+GAME_TERM_DEFAULTS = dict(track_game_reward_terms=False)
 
 
 class A2CAgent:
@@ -88,7 +92,7 @@ class A2CAgent:
         ``global_advantage_stats``) the advantage moments all use the same group, so a rank-0 checkpoint carries the
         statistics of every shard.  Pass ``env.env_base`` = the rank's shard offset (``cfg['env']['envBase']``) so that the
         reset / exploration noise is keyed by global env ids."""
-        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS, **OUTCOME_DEFAULTS, **REWARD_TERM_DEFAULTS)
+        cfg = dict(DEFAULT_CONFIG, **TRAIN_DEFAULTS, **OUTCOME_DEFAULTS, **REWARD_TERM_DEFAULTS, **GAME_TERM_DEFAULTS)
         cfg.update(config or {})
         process_group = bdist.resolve_group(process_group)
         self.config, self.env, self.group = cfg, env, process_group
@@ -150,6 +154,14 @@ class A2CAgent:
         if self.track_reward_terms:
             self._rt_partials = torch.zeros(T, len(env.REWARD_TERMS), (N + 31) // 32, dtype=torch.float64, device=self.device)
             self.reward_terms = RewardTerms(env.REWARD_TERMS, self.device)
+        # track_game_reward_terms: each env's per-term episode return (carried across epochs like current_rewards), the per-step
+        # sums of the done envs' per-term returns (per 32 envs) and their meter
+        self.track_game_reward_terms = bool(cfg["track_game_reward_terms"])
+        if self.track_game_reward_terms:
+            k = len(env.REWARD_TERMS)
+            self.current_term_rewards = torch.zeros(k, N, **f32)
+            self._gt_partials = torch.zeros(T, k, (N + 31) // 32, dtype=torch.float64, device=self.device)
+            self.game_reward_terms = GameTermMeter(env.REWARD_TERMS, int(cfg["games_to_track"]), self.device)
         self.obs = env.reset()["obs"].clone()
         self.dones = torch.zeros(N, dtype=torch.uint8, device=self.device)
         self.dataset = None
@@ -196,7 +208,9 @@ class A2CAgent:
                                         value_bootstrap=self.config["value_bootstrap"], episode_returns=self.current_rewards,
                                         episode_lengths=self.current_lengths, episode_partials=self._ep_partials[t],
                                         episode_outcomes=self._oc_partials[t] if self.track_outcomes else None,
-                                        reward_terms=self._rt_partials[t] if self.track_reward_terms else None)
+                                        reward_terms=self._rt_partials[t] if self.track_reward_terms else None,
+                                        game_term_returns=self.current_term_rewards if self.track_game_reward_terms else None,
+                                        game_term_partials=self._gt_partials[t] if self.track_game_reward_terms else None)
                 if head_targets:
                     env.step_precomputed_targets(res["env_actions"])
                 else:
@@ -207,6 +221,8 @@ class A2CAgent:
                 self.game_outcomes.update(self._oc_partials, self.num_actors)
             if self.track_reward_terms:
                 self.reward_terms.update(self._rt_partials, self.num_actors)
+            if self.track_game_reward_terms:
+                self.game_reward_terms.update(self._ep_partials, self._gt_partials, self.num_actors)
             _, last_v = self._forward(self._norm_obs(self.obs))
             last_values = self.value_mean_std(last_v, unnorm=True) if self.config["normalize_value"] else last_v
             a2c_common.discount_values(self.dones, last_values, buf.tensor_dict["dones"], buf.tensor_dict["values"], self.mb_rewards,
@@ -344,7 +360,9 @@ class A2CAgent:
         same epoch (in rl_games the other ranks would wait in the next epoch's collectives).  Returns ``(last_mean_rewards,
         epoch)`` and a per-epoch history (mean return / length or None before the first finished game, losses, lr; with
         ``track_outcomes`` also ``outcomes``: outcome name -> share of the tracked games, None before the first finished game; with
-        ``track_reward_terms`` also ``reward_terms``: term name -> mean per env-step of the epoch's rollout, on this rank's envs)."""
+        ``track_reward_terms`` also ``reward_terms``: term name -> mean per env-step of the epoch's rollout, on this rank's envs;
+        with ``track_game_reward_terms`` also ``game_reward_terms``: term name -> mean return per tracked game, None before the first
+        finished game -- the terms sum to ``mean_reward`` up to fp32 rounding)."""
         cfg = self.config
         rank0 = not bdist.is_distributed(self.group) or torch.distributed.get_rank() == 0
         if rank0:
@@ -359,6 +377,8 @@ class A2CAgent:
                 row["outcomes"] = None
             if self.track_reward_terms:
                 row["reward_terms"] = self.reward_terms.as_dict()
+            if self.track_game_reward_terms:
+                row["game_reward_terms"] = None
             should_exit = False
             if rank0:
                 if self.game_rewards.current_size > 0:
@@ -366,6 +386,8 @@ class A2CAgent:
                     row["mean_reward"], row["mean_length"] = mean_rewards, float(self.game_lengths.get_mean()[0])
                     if self.track_outcomes:
                         row["outcomes"] = self.game_outcomes.as_dict()
+                    if self.track_game_reward_terms:
+                        row["game_reward_terms"] = self.game_reward_terms.as_dict()
                     if cfg["save_frequency"] > 0 and epoch % cfg["save_frequency"] == 0 and mean_rewards <= self.last_mean_rewards:
                         self.save(os.path.join(directory, f"last_{cfg['name']}_ep_{epoch}"))
                     if mean_rewards > self.last_mean_rewards and epoch >= cfg["save_best_after"]:

@@ -120,3 +120,50 @@ class RewardTerms:
     def as_dict(self):
         """name -> mean per env-step, one device-to-host read."""
         return dict(zip(self.names, self._mean.tolist()))
+
+
+class GameTermMeter:
+    """``AverageMeter(K, games_to_track)`` fed with one K-row per finished episode: that episode's return in each reward term
+    ``names`` (the env's ``REWARD_TERMS``), so the means say what the last ``games_to_track`` games' mean return is made of.  Kept
+    on the device and fed by the fused step's game term partials (``KickEnv.set_rollout_targets(game_term_returns=...,
+    game_term_partials=...)``) together with the episode partials (their done counts), with ``EpisodeMeter``'s recurrence and step
+    order, so after the same updates ``current_size`` equals the game meters'.  Summed over the terms the means are the mean game
+    return up to fp32 rounding."""
+
+    def __init__(self, names, games_to_track=100, device="cuda"):
+        from ..tasks import KickEnv, OrientEnv, WalkEnv
+        if int(games_to_track) <= 0:
+            raise ValueError("games_to_track must be positive")
+        self.names = tuple(names)
+        # the fold takes the task whose terms these are
+        tasks = {env.REWARD_TERMS: env.TASK for env in (KickEnv, WalkEnv, OrientEnv)}
+        if self.names not in tasks:
+            raise ValueError(f"names must be the REWARD_TERMS of an env: {', '.join(map(str, tasks))}")
+        self.task = tasks[self.names]
+        self.max_size = int(games_to_track)
+        self.device = torch.device(device)
+        self._mean = torch.zeros(len(self.names), dtype=torch.float32, device=self.device)
+        self._size = torch.zeros(1, dtype=torch.int64, device=self.device)
+
+    def update(self, ep_partials, term_partials, num_envs):
+        """Fold (T, 3, W) float64 episode partials and (T, K, W) float64 game term partials, W = ceil(num_envs/32) -- T consecutive
+        steps -- step by step in order, one launch."""
+        k, w = len(self.names), (int(num_envs) + 31) // 32
+        ops.game_terms_meter_update(ep_partials, term_partials, num_envs, self.task, self.max_size, self._mean, self._size,
+                                    steps=term_partials.numel() // (k * w))
+
+    @property
+    def current_size(self):
+        return int(self._size[0])
+
+    def get_mean(self):
+        """numpy (K,): each term's mean return per tracked game."""
+        return self._mean.cpu().numpy()
+
+    def as_dict(self):
+        """name -> mean per game, one device-to-host read."""
+        return dict(zip(self.names, (float(x) for x in self.get_mean())))
+
+    def clear(self):
+        self._mean.zero_()
+        self._size.zero_()

@@ -12,7 +12,9 @@ rl_games' per-step tally (``done.nonzero()``, ``cr[done].sum().item()``, ``steps
 (``bezk_player_tally_update``) and one host read every ``sync_every`` steps; the fold stops adding at the step that reaches
 ``games_num * n_game_life`` games, so the result does not depend on ``sync_every``.  With ``track_outcomes`` the step also counts
 how each episode ended (the env's ``OUTCOMES``), and a second fold with the same cutoff (``bezk_player_outcome_update``) joins the
-same host read.  With observation domain randomisation the
+same host read.  With ``track_reward_terms`` the step also carries each episode's return per reward term (the env's
+``REWARD_TERMS``), and a third fold with the same cutoff (``bezk_player_game_terms_update``) joins that read too.  With observation
+domain randomisation the
 noise lands after the step kernel, so the player then normalises the noisy rows with ``RunningMeanStd`` (eval mode) instead.
 """
 import math
@@ -29,11 +31,12 @@ MAX_STEPS = 108000 // 4
 
 
 class PpoPlayerContinuous:
-    def __init__(self, env, config=None, seed=0, sync_every=32, track_outcomes=False):
+    def __init__(self, env, config=None, seed=0, sync_every=32, track_outcomes=False, track_reward_terms=False):
         """``config``: ``PLAYER_DEFAULTS`` keys (``utils.config.player_config``; the older spelling ``determenistic`` is accepted)
         and ``normalize_input`` (default True, as ``learner.A2CAgent``).  ``seed``: Philox key of the sampled actions.
         ``sync_every``: env steps per tally fold and host read.  ``track_outcomes``: also count the games per outcome class
-        (``run()`` then returns ``outcomes`` / ``outcome_rates`` and prints an ``outcomes:`` line)."""
+        (``run()`` then returns ``outcomes`` / ``outcome_rates`` and prints an ``outcomes:`` line).  ``track_reward_terms``: also
+        sum the games' returns per reward term (``run()`` then returns ``reward_terms`` and prints a ``reward terms:`` line)."""
         config = dict(config or {})
         if "determenistic" in config:
             config.setdefault("deterministic", config.pop("determenistic"))
@@ -67,6 +70,13 @@ class PpoPlayerContinuous:
         if self.track_outcomes:
             self._oc_partials = torch.zeros(self.sync_every, len(env.OUTCOMES), w, dtype=torch.int32, device=self.device)
             self._oc_counts = torch.zeros(1 + len(env.OUTCOMES), **f64)
+        # track_reward_terms: each env's per-term episode return, the game term partials of one chunk and [games_counted, sum per term]
+        self.track_reward_terms = bool(track_reward_terms)
+        if self.track_reward_terms:
+            k = len(env.REWARD_TERMS)
+            self.current_term_rewards = torch.zeros(k, n, **f32)
+            self._gt_partials = torch.zeros(self.sync_every, k, w, **f64)
+            self._gt_sums = torch.zeros(1 + k, **f64)
 
     # ------------------------------------------------------------------ checkpoints
     def restore(self, fn):
@@ -121,6 +131,8 @@ class PpoPlayerContinuous:
         extra = dict(obs_norm=self.obs_norm, obs_mean=rms.running_mean, obs_var=rms.running_var, obs_eps=rms.epsilon) if fused else {}
         if self.track_outcomes:
             extra["episode_outcomes"] = self._oc_partials[t]
+        if self.track_reward_terms:
+            extra.update(game_term_returns=self.current_term_rewards, game_term_partials=self._gt_partials[t])
         self.env.set_rollout_targets(episode_returns=self.current_rewards, episode_lengths=self.current_lengths,
                                      episode_partials=self._partials[t], **extra)
 
@@ -138,6 +150,8 @@ class PpoPlayerContinuous:
         obs = self.env.reset()["obs"]
         self.current_rewards.zero_()
         self.current_lengths.zero_()
+        if self.track_reward_terms:
+            self.current_term_rewards.zero_()
         return obs
 
     def run(self):
@@ -145,14 +159,18 @@ class PpoPlayerContinuous:
         restarting from ``env_reset()`` every ``max_steps`` steps.  Prints rl_games' ``reward: ... steps: ...`` line for every
         step with finished games (``print_stats``) and the final ``av reward: ... av steps: ...``.  Returns dict(games_played,
         sum_rewards, sum_steps, av_reward, av_steps); with ``track_outcomes`` also ``outcomes`` (outcome name -> games) and
-        ``outcome_rates`` (outcome name -> share of the games played), printed as one ``outcomes:`` line after ``av reward``."""
+        ``outcome_rates`` (outcome name -> share of the games played), printed as one ``outcomes:`` line after ``av reward``; with
+        ``track_reward_terms`` also ``reward_terms`` (term name -> the term's return per game, scaled like ``av_reward``, so the terms
+        sum to it up to rounding), printed as one ``reward terms:`` line after those."""
         env, n = self.env, self.env.num_envs
         n_games = self.games_num * self.n_game_life
         tally = self._tally.zero_()
         if self.track_outcomes:
             self._oc_counts.zero_()
+        if self.track_reward_terms:
+            self._gt_sums.zero_()
         games_played = sum_rewards = sum_steps = 0.0
-        oc_host = None
+        oc_host = gt_host = None
         try:
             with torch.no_grad():
                 for _ in range(n_games):
@@ -173,8 +191,15 @@ class PpoPlayerContinuous:
                         if self.track_outcomes:
                             ops.player_outcome_update(self._oc_partials[:k], n, env.TASK, n_games, self._oc_counts, steps=k)
                             parts.append(self._oc_counts)
+                        if self.track_reward_terms:
+                            ops.player_game_terms_update(self._partials[:k], self._gt_partials[:k], n, env.TASK, n_games, self._gt_sums,
+                                                         steps=k)
+                            parts.append(self._gt_sums)
                         host = torch.cat(parts).cpu()      # the one host read of the chunk
                         games_played, sum_rewards, sum_steps = float(host[0]), float(host[1]), float(host[2])
+                        if self.track_reward_terms:
+                            gt_host = host[-self._gt_sums.numel():]
+                            host = host[:-self._gt_sums.numel()]
                         if self.track_outcomes:
                             oc_host = host[4 + 3 * k:]
                             host = host[:4 + 3 * k]
@@ -195,4 +220,9 @@ class PpoPlayerContinuous:
             res["outcome_rates"] = {name: (c / games_played if games_played else math.nan) for name, c in res["outcomes"].items()}
             print("outcomes:", " ".join(f"{name} {int(c)} ({100.0 * res['outcome_rates'][name]:.1f} %)"
                                         for name, c in res["outcomes"].items()))
+        if self.track_reward_terms:
+            sums = [0.0] * len(env.REWARD_TERMS) if gt_host is None else [float(x) for x in gt_host[1:]]
+            res["reward_terms"] = {name: (s / games_played * self.n_game_life if games_played else math.nan)
+                                   for name, s in zip(env.REWARD_TERMS, sums)}
+            print("reward terms:", " ".join(f"{name} {v}" for name, v in res["reward_terms"].items()))
         return res

@@ -444,6 +444,86 @@ def reward_terms_update(partials, n, task, mean_k, steps=None):
                                             _cuda(mean_k, F64, "mean_k", k), _stream(partials)), "bezk_reward_terms_update")
 
 
+def post_physics_rollout_ep_game_terms(task, dof_state, rigid_body, root_states, net_contact, goal, initial_root_states, reset_buf,
+                                       progress_buf, timeout_buf, cfg, obs, rew, episode_returns, episode_lengths, episode_partials,
+                                       game_term_returns, game_term_partials, outcome_partials=None, term_partials=None, obs_mean=None,
+                                       obs_var=None, obs_norm=None, obs_eps=1e-5, rollout_cfg=None, values=None, shaped_rewards=None,
+                                       dones_u8=None, goal_angle=None, ball_init=None, prev_lin_vel=None, uniforms=None,
+                                       goal_uniforms=None, seed=0, step=0, randomize_buf=None, obs_clipped=None, env_base=0):
+    """``post_physics_rollout_ep`` (with the optional normaliser, outcome counts and reward terms of ``_ep_norm`` / ``_ep_outcome``
+    / ``_ep_terms``) that also carries each env's per-term episode returns (``game_term_returns``, (K, N) float32, CUDA) and writes
+    the per-warp sums of the done envs' per-term returns (``game_term_partials``, (K, ceil(N/32)) float64, CUDA;
+    ``bezk_post_physics_rollout_ep_game_terms``)."""
+    n = progress_buf.shape[0]
+    nb = cfg.num_bodies
+    actors, _, width = bm.task_dims(task)
+    w = (n + 31) // 32
+    k = reward_terms(task)
+    ret = _cuda(episode_returns, F32, "episode_returns", n)
+    length = _cuda(episode_lengths, F32, "episode_lengths", n)
+    part = _cuda(episode_partials, F64, "episode_partials", 3 * w)
+    gacc = _cuda(game_term_returns, F32, "game_term_returns", k * n)
+    gpart = _cuda(game_term_partials, F64, "game_term_partials", k * w)
+    oc = None if outcome_partials is None else _cuda(outcome_partials, I32, "outcome_partials", outcome_classes(task) * w)
+    tm = None if term_partials is None else _cuda(term_partials, F64, "term_partials", k * w)
+    if any(t is not None for t in (obs_mean, obs_var, obs_norm)):
+        mean, var = _cuda(obs_mean, F64, "obs_mean", width), _cuda(obs_var, F64, "obs_var", width)
+        out = _cuda(obs_norm, F32, "obs_norm", n * width)
+    else:
+        mean = var = out = None
+    lib = _lib.load()
+    _lib.check(lib.bezk_post_physics_rollout_ep_game_terms(
+        _TASK_ID[task], _p(dof_state, F32, "dof_state", n * 36), _p(rigid_body, F32, "rigid_body", n * nb * 13),
+        _p(root_states, F32, "root_states", n * actors * 13), _p(net_contact, F32, "net_contact", n * nb * 3),
+        _p(prev_lin_vel, F32, "prev_lin_vel", n * 3, True), _p(goal, F32, "goal", n * 2),
+        _p(goal_angle, F32, "goal_angle", n, True), _p(ball_init, F32, "ball_init", n * 2, True),
+        _p(initial_root_states, F32, "initial_root_states", n * actors * 13, True),
+        _p(uniforms, F32, "uniforms", n * 36, True), _p(goal_uniforms, F32, "goal_uniforms", 2, True), seed, step,
+        _p(reset_buf, I64, "reset_buf", n), _p(progress_buf, I64, "progress_buf", n),
+        _p(timeout_buf, I64, "timeout_buf", n), _p(randomize_buf, I64, "randomize_buf", n, True), C.byref(cfg),
+        _p(obs, F32, "obs", n * width), _p(obs_clipped, F32, "obs_clipped", n * width, True), _p(rew, F32, "rew", n),
+        C.byref(rollout_cfg) if rollout_cfg is not None else None, _p(values, F32, "values", n, True),
+        _p(shaped_rewards, F32, "shaped_rewards", n, True), _p(dones_u8, U8, "dones_u8", n, True), int(env_base), n,
+        ret, length, part, mean, var, float(obs_eps), out, oc, tm, gacc, gpart, _stream(dof_state)),
+        "bezk_post_physics_rollout_ep_game_terms")
+
+
+def _game_term_steps(ep_partials, term_partials, n, k, steps):
+    w = (int(n) + 31) // 32
+    if steps is None:
+        steps = term_partials.numel() // (k * w) if isinstance(term_partials, torch.Tensor) and w else 0
+    if not isinstance(term_partials, torch.Tensor) or term_partials.numel() != int(steps) * k * w:
+        raise BezkError(f"term_partials must hold steps x {k} x {w} float64 values")
+    if not isinstance(ep_partials, torch.Tensor) or ep_partials.numel() != int(steps) * 3 * w:
+        raise BezkError(f"ep_partials must hold steps x 3 x {w} float64 values")
+    return int(steps)
+
+
+def game_terms_meter_update(ep_partials, term_partials, n, task, games_to_track, mean_k, size, steps=None):
+    """Fold ``steps`` consecutive (3, ceil(n/32)) episode partials and (K, ceil(n/32)) float64 game term partials (each (steps, ., W)
+    or (., W)) into rl_games' ``AverageMeter(K, games_to_track)`` ``mean_k`` ((K,) float32) / ``size`` ((1,) int64), fed one K-row
+    of per-term returns per finished game, on the device (``bezk_game_terms_meter_update``)."""
+    k = reward_terms(task)
+    steps = _game_term_steps(ep_partials, term_partials, n, k, steps)
+    lib = _lib.load()
+    _lib.check(lib.bezk_game_terms_meter_update(_cuda(ep_partials, F64, "ep_partials", None), _cuda(term_partials, F64, "term_partials", None),
+                                                steps, int(n), _TASK_ID[task], int(games_to_track), _cuda(mean_k, F32, "mean_k", k),
+                                                _cuda(size, I64, "size", 1), _stream(term_partials)), "bezk_game_terms_meter_update")
+
+
+def player_game_terms_update(ep_partials, term_partials, n, task, games_num, sums, per_step=None, steps=None):
+    """Fold the same partials into ``sums`` ((1 + K,) float64: games_counted, then each term's sum of per-game returns) up to
+    ``games_num`` games, with ``player_tally_update``'s cutoff; ``per_step`` ((steps, K) float64, optional) gets each folded step's
+    sums (``bezk_player_game_terms_update``)."""
+    k = reward_terms(task)
+    steps = _game_term_steps(ep_partials, term_partials, n, k, steps)
+    ps = None if per_step is None else _cuda(per_step, F64, "per_step", steps * k)
+    lib = _lib.load()
+    _lib.check(lib.bezk_player_game_terms_update(_cuda(ep_partials, F64, "ep_partials", None), _cuda(term_partials, F64, "term_partials", None),
+                                                 steps, int(n), _TASK_ID[task], int(games_num), _cuda(sums, F64, "sums", 1 + k), ps,
+                                                 _stream(term_partials)), "bezk_player_game_terms_update")
+
+
 def reset_idx_task(task, env_ids, dof_state, root_states, initial_root_states, goal, progress, reset, cfg, uniforms=None,
                    goal_uniforms=None, seed=0, step=0, env_base=0):
     k = int(env_ids.numel())

@@ -223,6 +223,7 @@ class KickEnv(VecTask):
         self._obs_norm = None               # (obs_mean, obs_var, obs_eps, obs_norm) set by set_rollout_targets
         self._outcomes = None               # (K, ceil(N/32)) int32 outcome partials set by set_rollout_targets
         self._reward_terms = None           # (K, ceil(N/32)) float64 reward term partials set by set_rollout_targets
+        self._game_terms = None             # ((K, N) float32 game term returns, (K, ceil(N/32)) float64 partials) likewise
         self._d_values = None               # staged_ce host pipeline: device image of host-resident critic values
         self._lib = _lib.load()
         # the step keeps these in L2 with evict_last (bezk.h, bezk_l2_release): demoted again when the env goes away
@@ -525,6 +526,15 @@ class KickEnv(VecTask):
             if self._episode is not None:     # + rl_games' episode return / length bookkeeping (set_rollout_targets)
                 # + the eval-mode observation normaliser when armed (all NULL: exactly bezk_post_physics_rollout_ep)
                 mean, var, eps, out = self._obs_norm or (None, None, 0.0, None)
+                if self._game_terms is not None:      # + the per-term episode returns (and whatever else is armed)
+                    rc = self._lib.bezk_post_physics_rollout_ep_game_terms(
+                        ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed, self._rng_step, t[0], t[1], t[2], t[3],
+                        t[4], t[5], t[6], t[7], *tail, self.env_base, self.num_envs, *[_ptr(x) for x in self._episode], _ptr(mean),
+                        _ptr(var), eps, _ptr(out), _ptr(self._outcomes), _ptr(self._reward_terms), *[_ptr(x) for x in self._game_terms],
+                        self._stream())
+                    if rc:
+                        _lib.check(rc, "bezk_post_physics_rollout_ep_game_terms")
+                    return
                 if self._reward_terms is not None:    # + the per-warp reward term sums (and the outcome counts when armed)
                     rc = self._lib.bezk_post_physics_rollout_ep_terms(
                         ops._TASK_ID[self.TASK], *f["head"], prev, *f["mid_task"], self._seed, self._rng_step, t[0], t[1], t[2], t[3],
@@ -834,7 +844,8 @@ class KickEnv(VecTask):
 
     def set_rollout_targets(self, values=None, shaped_rewards=None, dones_u8=None, gamma=0.99, scale_value=0.01, shift_value=0.0,
                             value_bootstrap=True, episode_returns=None, episode_lengths=None, episode_partials=None, obs_norm=None,
-                            obs_mean=None, obs_var=None, obs_eps=1e-5, episode_outcomes=None, reward_terms=None):
+                            obs_mean=None, obs_var=None, obs_eps=1e-5, episode_outcomes=None, reward_terms=None,
+                            game_term_returns=None, game_term_partials=None):
         """Arm the reward epilogue of the fused step (SURVEY 8 a16; rl_games ``play_steps``): the NEXT steps also write
         ``shaped_rewards = (rew + shift) * scale + gamma * values * time_outs`` (e.g. ``mb_rewards[t]``) and the uint8 reset
         mask ``dones_u8`` (e.g. the experience buffer's ``dones`` slot ``t + 1``).  ``values``: the (N,)/(N,1) un-normalised
@@ -852,7 +863,13 @@ class KickEnv(VecTask):
         ``learner.OutcomeMeter`` and of the player's outcome counts.
         ``reward_terms`` ((K, ceil(N/32)) float64, K = ``len(REWARD_TERMS)``), with the episode tensors armed and without
         ``obs_norm``, GPU pipeline only: the step also writes, per group of 32 envs, the sum of each of ``REWARD_TERMS`` over its envs
-        -- the input of ``learner.RewardTerms``.  Call with no arguments to disarm everything."""
+        -- the input of ``learner.RewardTerms``.
+        ``game_term_returns`` ((K, N) float32, zeroed by the caller once, like ``episode_returns``) and ``game_term_partials``
+        ((K, ceil(N/32)) float64), K = ``len(REWARD_TERMS)``, both or none, with the episode tensors armed, GPU pipeline only: the
+        step also carries each env's episode return per term of ``REWARD_TERMS`` (zeroed by a multiply when the env is done) and
+        writes, per group of 32 envs, the sum of its done envs' per-term returns -- the input of ``learner.GameTermMeter`` and of
+        the player's per-term returns.  They combine with ``obs_norm``, ``episode_outcomes`` and ``reward_terms``.  Call with no
+        arguments to disarm everything."""
         if self.fusion != "fused":
             raise NotImplementedError("the reward epilogue rides in the fused step (fusion='fused')")
         n, dev = self.num_envs, self.compute_device
@@ -895,6 +912,21 @@ class KickEnv(VecTask):
             t = reward_terms
             if t.dtype != torch.float64 or t.numel() != numel or not t.is_contiguous() or t.device != dev:
                 raise ValueError(f"reward_terms must be a contiguous torch.float64 tensor with {numel} elements on {dev}")
+        game = (game_term_returns, game_term_partials)
+        if any(t is not None for t in game):
+            if self.host_staged:
+                raise NotImplementedError("game term returns need the GPU pipeline")
+            if any(t is None for t in game):
+                raise ValueError("game_term_returns and game_term_partials are armed together")
+            if episode_returns is None:
+                raise ValueError("game_term_returns needs the episode tensors (episode_returns, episode_lengths, episode_partials)")
+            k = len(self.REWARD_TERMS)
+            for t, dtype, numel, name in zip(game, (torch.float32, torch.float64), (k * n, k * ((n + 31) // 32)),
+                                             ("game_term_returns", "game_term_partials")):
+                if t.dtype != dtype or t.numel() != numel or not t.is_contiguous() or t.device != dev:
+                    raise ValueError(f"{name} must be a contiguous {dtype} tensor with {numel} elements on {dev}")
+        else:
+            game = None
         eps = (episode_returns, episode_lengths, episode_partials)
         if any(t is not None for t in eps):
             if self.host_staged:
@@ -911,6 +943,7 @@ class KickEnv(VecTask):
         self._obs_norm = norm
         self._outcomes = episode_outcomes
         self._reward_terms = reward_terms
+        self._game_terms = game
         if shaped_rewards is None and dones_u8 is None:
             self._rollout = None
             return

@@ -134,9 +134,9 @@ TRAIN_LOOP_KEYS = ("games_to_track", "save_best_after", "save_frequency", "score
 
 def train_loop_config(train_cfg):
     """``params.config`` of a resolved train yaml -> the training-loop keys of ``learner.A2CAgent``'s ``config``.  The agent's
-    ``track_outcomes`` (``learner.agent.OUTCOME_DEFAULTS``) and ``track_reward_terms`` (``learner.agent.REWARD_TERM_DEFAULTS``) are
-    not read from the yaml: they are this project's own options, not rl_games settings, so callers pass them in the ``config`` dict
-    themselves."""
+    ``track_outcomes`` (``learner.agent.OUTCOME_DEFAULTS``), ``track_reward_terms`` (``learner.agent.REWARD_TERM_DEFAULTS``) and
+    ``track_game_reward_terms`` (``learner.agent.GAME_TERM_DEFAULTS``) are not read from the yaml: they are this project's own
+    options, not rl_games settings, so callers pass them in the ``config`` dict themselves."""
     c = train_cfg["params"]["config"]
     return {k: c[k] for k in TRAIN_LOOP_KEYS if k in c}
 

@@ -493,6 +493,52 @@ int bezk_post_physics_rollout_ep_terms(int task, float* dof_state, const float* 
  * mean_k[k] = (sum of term k over the steps x n env-steps) / (steps * n), written to mean_k (K,) f64, DEVICE memory.  Fixed
  * summation order (the same bits every run); no host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op. */
 int bezk_reward_terms_update(const double* partials, int steps, int64_t n, int task, double* mean_k, void* stream);
+/* Game term returns: what each finished episode's return is made of, one return per reward term of bezk_reward_terms.  The step
+ * carries K accumulators per env next to ep_return, with ep_return's recurrence:
+ *   r_k = acc_k + term_k;   acc_k <- r_k * (1 - done)          (a multiply: NaN / inf stays, as in rl_games)
+ * where term_k is the value the step computes for term k in the reward call whose rew it stores.  When an env is done, r_k is its
+ * episode's return in term k, and:
+ *   1. termination is exact: the termination term is 0 except in the step where a rule fires, so a finished game's termination
+ *      return equals the reward of its last step bit for bit, and a live env's termination accumulator is exactly 0;
+ *   2. the terms sum to the return: sum_k r_k equals the return the step adds to ep_partials, up to fp32 re-association;
+ *   3. the counts agree: the folds below take their game counts from ep_partials.
+ * bezk_post_physics_rollout_ep_terms that also carries the game term returns:
+ *   game_term_returns  (K, n) f32 in/out, DEVICE memory, term-major, 4-byte aligned: the accumulators acc_k (zero them once, like
+ *                      ep_return).
+ *   game_term_partials (K, W) f64 out, DEVICE memory, W = ceil(n / 32), 8-byte aligned: at [k * W + env / 32] the sum of r_k over
+ *                      the done envs of that group of 32 (a fixed-order shuffle tree: the same bits every run).  Every slot is
+ *                      written each step (zeros included), so the buffer needs no zeroing.
+ * Both and the episode accumulators are required (BEZK_E_BADARG).  The normaliser arguments (all NULL or all non-NULL),
+ * outcome_partials and term_partials are optional, but the normaliser does not combine with term_partials (BEZK_E_BADARG).
+ * Every check runs before any device access.  Every other output is the same bytes as without the game term arguments. */
+int bezk_post_physics_rollout_ep_game_terms(int task, float* dof_state, const float* rigid_body, float* root_states,
+                                            float* net_contact, float* prev_lin_vel, float* goal, const float* goal_angle,
+                                            const float* ball_init, const float* initial_root_states,
+                                            const float* uniforms, const float* goal_uniforms, uint64_t seed, uint64_t step,
+                                            int64_t* reset_buf, int64_t* progress_buf, int64_t* timeout_buf,
+                                            int64_t* randomize_buf, const BezkTaskCfg* cfg, float* obs, float* obs_clipped,
+                                            float* rew, const BezkRolloutCfg* rollout, const float* values,
+                                            float* shaped_rewards, uint8_t* dones_u8, int64_t env_base, int64_t n,
+                                            float* ep_return, float* ep_length, double* ep_partials,
+                                            const double* obs_mean, const double* obs_var, float obs_eps, float* obs_norm,
+                                            int32_t* outcome_partials, double* term_partials, float* game_term_returns,
+                                            double* game_term_partials, void* stream);
+/* rl_games' AverageMeter(K, games_to_track) fed with one K-row of game term returns per finished game, from `steps` consecutive
+ * ep_partials ((steps, 3, ceil(n / 32)) f64; row 0 gives the done counts) and game_term_partials ((steps, K, ceil(n / 32)) f64),
+ * step by step in order, with bezk_episode_meter_update's recurrence: size = the step's done count, new_mean[k] =
+ * (float)(sum_k / count) in fp64.  A step with no done env changes nothing, so *size always equals the game meters' size.
+ * mean_k (K,) f32 and size (1,) i64, DEVICE memory, in/out.  Fixed summation order (the same bits every run); no host
+ * synchronisation (graph capturable); steps == 0 or n == 0 is a no-op. */
+int bezk_game_terms_meter_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int task,
+                                 int64_t games_to_track, float* mean_k, int64_t* size, void* stream);
+/* BasePlayer.run's game tally per reward term: `steps` consecutive ep_partials and game_term_partials folded into sums (1 + K,)
+ * f64 in/out, DEVICE memory: [games_counted, sum_0 .. sum_{K-1}], with bezk_player_tally_update's cutoff (a step that starts with
+ * games_counted >= games_num adds nothing, the step that reaches it is added whole), so over the same steps games_counted equals
+ * that tally's games_played.  per_step (steps, K) f64 out or NULL: each folded step's K sums, zeros for the steps not folded.
+ * Fixed summation order; no host synchronisation (graph capturable); steps == 0 or n == 0 is a no-op; games_num <= 0 is
+ * BEZK_E_BADARG. */
+int bezk_player_game_terms_update(const double* ep_partials, const double* term_partials, int steps, int64_t n, int task,
+                                  int64_t games_num, double* sums, double* per_step, void* stream);
 /* bezk_reset_idx for any task: root rows are 13 floats for walk / orient, and their goal (n,2) rows are redrawn.
  * env_base: global id of local env 0 (Philox key = env_base + env id), as in bezk_post_physics_rollout. */
 int bezk_reset_idx_task(int task, const int64_t* env_ids, int64_t k, const float* uniforms, const float* goal_uniforms,
